@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- masked-coalition Wav2Vec2 forwards/sec on N B200s (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C2] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C2] [--impl reference] [--dump-outputs DIR]
 
 A "step" = one pass of the hot path over one batch of synthetic input: every coalition of the workload
 (C2: 2048 coalitions of one 5 s clip, 100 segments) through mask -> Wav2Vec2 -> per-character CTC
@@ -119,6 +119,30 @@ def make_hf_model(cfg):
     return build_random_init_model(cfg, seed=0)
 
 
+def clip_targets(model, clip):
+    """Per-character (frame, token) targets of the unmasked clip, from the fp32 forward of `model` on the host.  Random-init
+    logits are nearly flat (on C2 about one frame in ten has its top-2 margin inside the bf16 error of the device path), so
+    targets taken from the build under test would differ between builds; these do not.  -> (logits, frames, tokens)"""
+    from shap_transformer_asr_b200 import char_targets
+    with torch.no_grad():
+        lg = model(torch.from_numpy(clip)[None]).logits[0].numpy()
+    frames, tokens = char_targets(lg)
+    return lg, frames, tokens
+
+
+DUMP_LIMIT = 60 << 20          # data bytes of a --dump-outputs file: with its header, under 64 MB
+
+
+def dump_outputs(path, name, a):
+    """Write `a` as <path>/<name>.npy in float32; above DUMP_LIMIT bytes, a fixed seeded sample of its rows."""
+    a = np.ascontiguousarray(a, dtype=np.float32)
+    if a.nbytes > DUMP_LIMIT:
+        rows = DUMP_LIMIT // a[:1].nbytes
+        a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], rows, replace=False))]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, name + ".npy"), a)
+
+
 def cpu_reference_rate(model, cfg, clip, Z, bounds, frames, tokens, n_rows, batch=32, threads=None):
     """forwards/s of the reference's CPU path: transformers fp32 forward on masked waveforms -> log_softmax -> gather."""
     from oracle import callback as CB
@@ -151,12 +175,9 @@ def run_reference(args):
         return
     wl, cfg, clip, Z, kw = build_problem(args.workload)
     from oracle import callback as CB
-    from shap_transformer_asr_b200 import char_targets
     model = make_hf_model(cfg)
     bounds = CB.segment_bounds(wl.num_samples, wl.num_segments)
-    with torch.no_grad():
-        lg = model(torch.from_numpy(clip)[None]).logits[0].numpy()
-    frames, tokens = char_targets(lg)
+    _, frames, tokens = clip_targets(model, clip)
     threads = os.cpu_count() or 1
     # bounded sample per step: calibrate on 8 rows so that warmup+steps finish within a few minutes
     r0, _, dt0, _ = cpu_reference_rate(model, cfg, clip, Z, bounds, frames, tokens, 8, batch=8, threads=threads)
@@ -167,6 +188,8 @@ def run_reference(args):
         r, done, dt, _ = cpu_reference_rate(model, cfg, clip, Z, bounds, frames, tokens, n_rows, batch=32, threads=threads)
         if i >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, "logprobs", cpu_reference_rate.last_outputs)
     total = sum(times)
     value = n_rows * args.steps / total
     line = {
@@ -184,7 +207,7 @@ def run_reference(args):
 
 def run_b200(args):
     import torch.distributed as td
-    from shap_transformer_asr_b200 import CoalitionCallback, Engine, char_targets, dist as wdist
+    from shap_transformer_asr_b200 import CoalitionCallback, Engine, dist as wdist
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank, world = wdist.init_from_env("cuda") if world > 1 else (0, 1)
@@ -203,10 +226,7 @@ def run_b200(args):
                  graphs=not args.no_graph)
     eng.set_clip(clip, num_segments=wl.num_segments)
     # targets: per-character frames of the unmasked clip (all frames if the random-init transcript is empty)
-    eng.set_targets("logits")
-    ones = eng.bits_to_device(np.ones((1, wl.num_segments), np.uint8))
-    lg = eng.eval_bits(ones).view(-1, cfg.vocab_size).cpu().numpy()
-    frames, tokens = char_targets(lg)
+    lg, frames, tokens = clip_targets(model, clip)
     eng.set_targets("logprob", frames, tokens)
     D = len(frames)
     K = Z.shape[0]
@@ -238,6 +258,8 @@ def run_b200(args):
     e1.record()
     torch.cuda.synchronize()
     launches = eng.launch_count() - launches0                            # counted inside the library at launch time
+    if args.dump_outputs and rank == 0:                                  # the rows the last timed step handed back
+        dump_outputs(args.dump_outputs, "logprobs", (gathered if world > 1 else out).cpu().numpy())
     if world > 1:
         td.barrier()
     ms = e0.elapsed_time(e1)
@@ -430,7 +452,11 @@ def main():
     ap.add_argument("--coalitions", type=int, default=0, help="profiling aid: evaluate only the first N coalitions per step")
     ap.add_argument("--preln-fp32", action="store_true", help="A/B: fp32 pre-LayerNorm tensors (W2S_FLAG_FP32_PRELN)")
     ap.add_argument("--no-graph", action="store_true", help="A/B: launch every kernel of a tile instead of replaying a graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.impl == "reference":
         run_reference(args)
         return
