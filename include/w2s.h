@@ -177,6 +177,20 @@ int64_t w2s_sample_rows(int M, int n_full, int n_paired, const int64_t* ind_set,
 int w2s_debug_gemm(int use_tcgen05, const void* a_bf16, const void* w_bf16, const float* bias,
                    const void* residual, int res_fp32, float alpha, void* out, int M, int N, int K, int act,
                    int out_fp32, void* stream);
+/* Self-attention of one layer on caller-owned device buffers, with the operand layout of the model paths: qkv[B*T, 3H] =
+ * q | k | v, or with pos_proj [2T-1, H] (row r <-> relative position T-1-r) the relative-position conformer's
+ * qkv[B*T, 4H] = q+u | q+v | k | v; H = 64 * heads.  use_tcgen05 = 1: the tensor-core kernel (attention_fa without
+ * pos_proj, which also writes lse[B, heads, T], the log2-domain log-sum-exp of the scaled scores, when lse != NULL;
+ * attention_rel with it); 0: the CUDA-core validation kernel (T <= 1024, lse must be NULL).  ctx[B*T, H] bf16.
+ * Errors via w2s_last_error(NULL). */
+int w2s_debug_attention(int use_tcgen05, const void* qkv, const void* pos_proj, int B, int T, int heads, float scale,
+                        void* ctx, float* lse, void* stream);
+/* Its backward (no relative positions): d ctx[B*T, H] -> dqkv[B*T, 3H] bf16.  use_tcgen05 = 1: the gradient path's fused
+ * kernel with its delta pre-pass and dQ cast, fed the forward's ctx and lse (from w2s_debug_attention); 0: the CUDA-core
+ * cross-check kernels (T <= 1024; ctx / lse unused).  The workspace is allocated and freed inside: the call synchronises
+ * the stream. */
+int w2s_debug_attention_bwd(int use_tcgen05, const void* qkv, const void* ctx, const void* dctx, const float* lse, int B,
+                            int T, int heads, float scale, void* dqkv, void* stream);
 /* Per-launch CUDA-event profile on the launching stream (bench.py roofline leg): enable, run evaluations,
  * then read per launch class (newline-separated names) total milliseconds, algorithmic FLOPs / bytes and
  * launch counts.  Returns the number of classes, or -1 if `names_cap` is too small. */

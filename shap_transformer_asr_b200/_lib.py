@@ -75,6 +75,10 @@ SIGNATURES = {
                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "w2s_debug_gemm": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_float,
                                  C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "w2s_debug_attention": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p,
+                                      C.c_void_p, C.c_void_p]),
+    "w2s_debug_attention_bwd": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                          C.c_float, C.c_void_p, C.c_void_p]),
     "w2s_profile_enable": (C.c_int, [C.c_void_p, C.c_int]),
     "w2s_profile_read": (C.c_int64, [C.c_void_p, C.c_char_p, C.c_int64, C.POINTER(C.c_double), C.POINTER(C.c_double),
                                      C.POINTER(C.c_double), C.POINTER(C.c_int64), C.c_int64]),

@@ -967,6 +967,29 @@ int fail(w2s_handle* h, const std::string& e) {
   return 1;
 }
 
+// SM count of the current device (the debug entry points have no handle)
+int debug_num_sms() {
+  static int sms = 0;
+  if (sms == 0) {
+    int dev = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  }
+  return sms;
+}
+
+// The operand layout of the model paths (PlanBuilder): q | k | v at 0 / H / 2H of a 3H row, or the relative-position
+// conformer's q+u | q+v | k | v at 0 / H / 2H / 3H of a 4H row.
+AttnParams debug_attn_params(const void* qkv, const void* pos_proj, int B, int T, int heads, float scale) {
+  AttnParams ap{};
+  const int H = heads * 64, nq = pos_proj ? 2 : 1;
+  ap.qkv = (const bf16*)qkv; ap.B = B; ap.T = T; ap.Tp = (T + 63) / 64 * 64; ap.H = H; ap.heads = heads; ap.hd = 64;
+  ap.ld = (nq + 2) * H; ap.q_off = 0; ap.qv_off = pos_proj ? H : 0; ap.k_off = nq * H; ap.v_off = (nq + 1) * H;
+  ap.scale = scale;
+  ap.pos_proj = (const bf16*)pos_proj;
+  return ap;
+}
+
 }  // namespace
 
 // =================================================================================================
@@ -1219,15 +1242,84 @@ int w2s_debug_gemm(int use_tcgen05, const void* a_bf16, const void* w_bf16, cons
     p.epi.bias = bias; p.epi.act = act; p.epi.out = out; p.epi.out_fp32 = out_fp32;
     p.epi.residual = residual; p.epi.res_fp32 = res_fp32; p.epi.alpha = alpha;
     GemmLaunch gl;
-    static int sms = 0;
-    if (sms == 0) {
-      int dev = 0;
-      cudaGetDevice(&dev);
-      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    }
-    e = gemm_prepare(p, sms, &gl);
+    e = gemm_prepare(p, debug_num_sms(), &gl);
     if (e.empty()) e = use_tcgen05 ? gemm_launch_tc(gl, (cudaStream_t)stream) : gemm_launch_simt(gl, (cudaStream_t)stream);
   }
+  if (!e.empty()) {
+    g_create_error = e;
+    return 1;
+  }
+  return 0;
+}
+
+int w2s_debug_attention(int use_tcgen05, const void* qkv, const void* pos_proj, int B, int T, int heads, float scale,
+                        void* ctx, float* lse, void* stream) {
+  g_create_error.clear();
+  const cudaStream_t s = (cudaStream_t)stream;
+  AttnParams ap = debug_attn_params(qkv, pos_proj, B, T, heads, scale);
+  ap.ctx = (bf16*)ctx;
+  ap.lse = lse;
+  std::string e;
+  if (B <= 0 || T <= 0 || heads <= 0 || !qkv || !ctx) {
+    e = "debug_attention: need B, T', heads >= 1 and qkv / ctx buffers";
+  } else if (lse && (pos_proj || !use_tcgen05)) {
+    e = "debug_attention: only the tcgen05 kernel without relative positions writes the log-sum-exp";
+  } else if (!(e = gemm_init()).empty()) {
+    // the tensor-map encoder the tcgen05 plans need is not available
+  } else if (!use_tcgen05) {
+    e = launch_attention_simt(ap, s);
+  } else if (pos_proj) {
+    AttnRelPlan* rp = nullptr;
+    e = attention_rel_init();
+    if (e.empty()) e = attention_rel_prepare(ap, &rp);
+    if (e.empty()) e = attention_rel_launch(rp, s);
+    if (rp) attention_rel_free(rp);   // the tensor maps travel in the kernel parameters: the plan may go after the launch
+  } else {
+    AttnFaPlan* fp = nullptr;
+    e = attention_fa_init();
+    if (e.empty()) e = attention_fa_prepare(ap, debug_num_sms(), &fp);
+    if (e.empty()) e = attention_fa_launch(fp, s);
+    if (fp) attention_fa_free(fp);
+  }
+  if (!e.empty()) {
+    g_create_error = e;
+    return 1;
+  }
+  return 0;
+}
+
+int w2s_debug_attention_bwd(int use_tcgen05, const void* qkv, const void* ctx, const void* dctx, const float* lse, int B,
+                            int T, int heads, float scale, void* dqkv, void* stream) {
+  g_create_error.clear();
+  const cudaStream_t s = (cudaStream_t)stream;
+  const AttnParams ap = debug_attn_params(qkv, nullptr, B, T, heads, scale);
+  const long long rows = (long long)B * T;
+  std::string e;
+  float *delta = nullptr, *dq = nullptr, *stats = nullptr;
+  auto dalloc = [&](float** p, size_t n) {
+    if (e.empty() && cudaMalloc((void**)p, sizeof(float) * n) != cudaSuccess) e = "debug_attention_bwd: out of device memory";
+  };
+  if (B <= 0 || T <= 0 || heads <= 0 || !qkv || !dctx || !dqkv) {
+    e = "debug_attention_bwd: need B, T', heads >= 1 and qkv / dctx / dqkv buffers";
+  } else if (use_tcgen05) {
+    if (!ctx || !lse) e = "debug_attention_bwd: the fused kernel needs the forward's ctx and log-sum-exp";
+    if (e.empty()) e = gemm_init();   // the tensor-map encoder of the plan
+    dalloc(&delta, (size_t)rows * heads);
+    dalloc(&dq, (size_t)rows * ap.H);
+    AttnBwdPlan* bp = nullptr;
+    if (e.empty()) e = attention_bwd_init();
+    if (e.empty()) e = attention_bwd_prepare(ap, (const bf16*)dctx, lse, delta, dq, (bf16*)dqkv, debug_num_sms(), &bp);
+    if (e.empty()) e = attention_bwd_launch(bp, (const bf16*)dctx, (const bf16*)ctx, ap.q_off, s);
+    if (bp) attention_bwd_free(bp);
+  } else {
+    dalloc(&stats, (size_t)rows * heads * 3);
+    if (e.empty()) e = launch_attn_bwd(ap.qkv, (const bf16*)dctx, B, T, ap.H, heads, scale, (bf16*)dqkv, stats, s);
+  }
+  // the workspace lives for this call only
+  const cudaError_t se = cudaStreamSynchronize(s);
+  if (se != cudaSuccess && e.empty()) e = std::string("debug_attention_bwd: ") + cudaGetErrorString(se);
+  for (float* p : {delta, dq, stats})
+    if (p) cudaFree(p);
   if (!e.empty()) {
     g_create_error = e;
     return 1;

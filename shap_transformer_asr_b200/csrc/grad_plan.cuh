@@ -245,6 +245,10 @@ struct GradBuilder {
     // attention backward: one fused tcgen05 kernel (attention_bwd.cu) unless the relative-position term is present or a
     // cross-check form was asked for (w2s_grad_debug bits 1 / 2)
     const bool attn_fused = !rel && !h->grad_attn_simt && !h->grad_attn_unfused;
+    // the other forms hold a whole score row per warp (attn_rows_t_kernel, attn_bwd_q_kernel): refuse before launching anything
+    if (!attn_fused && T > 1024)
+      return std::string("gradient path: ") + (rel ? "the relative-position attention backward" : "the cross-check attention backward") +
+             " takes at most 1024 frames (this clip has " + std::to_string(T) + ")";
     const size_t nlse = (size_t)n * c.num_attention_heads * T;
     std::vector<GradLayerBuf> lb(conf ? 0 : NL);
     for (int l = 0; l < NL && !conf; ++l) {

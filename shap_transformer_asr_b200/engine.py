@@ -319,3 +319,65 @@ def debug_gemm(a: torch.Tensor, w: torch.Tensor, bias=None, act: int = 0, out_fp
     if rc != 0:
         raise RuntimeError("w2s_debug_gemm: " + lib.w2s_last_error(None).decode())
     return out
+
+
+def _check_buffer(name: str, t: torch.Tensor, dtype: torch.dtype, numel: int):
+    if t.dtype != dtype or not t.is_cuda or not t.is_contiguous() or t.numel() < numel:
+        raise ValueError(f"{name}: need a contiguous {dtype} CUDA tensor of at least {numel} elements")
+
+
+def debug_attention(qkv: torch.Tensor, B: int, heads: int, pos_proj=None, scale: float = 0.125, tcgen05: bool = True,
+                    with_lse: bool = False, ctx=None, lse=None):
+    """Self-attention of one layer through the library's kernels (tests only): qkv [B*T, 3H] (q | k | v) or, with pos_proj
+    [2T-1, H], [B*T, 4H] (q+u | q+v | k | v), bf16, H = 64 * heads.  tcgen05: the tensor-core kernel (attention_fa, or
+    attention_rel with pos_proj), else the CUDA-core validation kernel.  Returns (ctx [B*T, H] bf16, lse [B, heads, T] fp32
+    log2-domain log-sum-exp or None); ``ctx`` / ``lse`` may be caller buffers (at least that many elements)."""
+    lib = _lib.load()
+    H = 64 * heads
+    T = qkv.shape[0] // B
+    _check_buffer("qkv", qkv, torch.bfloat16, B * T * (4 if pos_proj is not None else 3) * H)
+    if qkv.shape != (B * T, (4 if pos_proj is not None else 3) * H):
+        raise ValueError(f"qkv: shape {tuple(qkv.shape)} does not fit B={B}, heads={heads}")
+    if pos_proj is not None:
+        _check_buffer("pos_proj", pos_proj, torch.bfloat16, (2 * T - 1) * H)
+    if ctx is None:
+        ctx = torch.empty((B * T, H), dtype=torch.bfloat16, device=qkv.device)
+    _check_buffer("ctx", ctx, torch.bfloat16, B * T * H)
+    if lse is None and with_lse:
+        lse = torch.empty((B, heads, T), dtype=torch.float32, device=qkv.device)
+    if lse is not None:
+        _check_buffer("lse", lse, torch.float32, B * heads * T)
+    rc = lib.w2s_debug_attention(int(tcgen05), qkv.data_ptr(), pos_proj.data_ptr() if pos_proj is not None else None,
+                                 B, T, heads, float(scale), ctx.data_ptr(), lse.data_ptr() if lse is not None else None,
+                                 torch.cuda.current_stream().cuda_stream)
+    if rc != 0:
+        raise RuntimeError("w2s_debug_attention: " + lib.w2s_last_error(None).decode())
+    return ctx, lse
+
+
+def debug_attention_bwd(qkv: torch.Tensor, dctx: torch.Tensor, B: int, heads: int, ctx=None, lse=None, scale: float = 0.125,
+                        tcgen05: bool = True, dqkv=None):
+    """Backward of `debug_attention` without relative positions (tests only): d ctx [B*T, H] -> dqkv [B*T, 3H] bf16.
+    tcgen05: the gradient path's fused kernel, which needs the forward's ``ctx`` and ``lse``; else the CUDA-core
+    cross-check kernels.  ``dqkv`` may be a caller buffer."""
+    lib = _lib.load()
+    H = 64 * heads
+    T = qkv.shape[0] // B
+    _check_buffer("qkv", qkv, torch.bfloat16, B * T * 3 * H)
+    if qkv.shape != (B * T, 3 * H):
+        raise ValueError(f"qkv: shape {tuple(qkv.shape)} does not fit B={B}, heads={heads}")
+    _check_buffer("dctx", dctx, torch.bfloat16, B * T * H)
+    if tcgen05:
+        if ctx is None or lse is None:
+            raise ValueError("the fused backward needs the forward's ctx and lse")
+        _check_buffer("ctx", ctx, torch.bfloat16, B * T * H)
+        _check_buffer("lse", lse, torch.float32, B * heads * T)
+    if dqkv is None:
+        dqkv = torch.empty((B * T, 3 * H), dtype=torch.bfloat16, device=qkv.device)
+    _check_buffer("dqkv", dqkv, torch.bfloat16, B * T * 3 * H)
+    rc = lib.w2s_debug_attention_bwd(int(tcgen05), qkv.data_ptr(), ctx.data_ptr() if ctx is not None else None,
+                                     dctx.data_ptr(), lse.data_ptr() if lse is not None else None, B, T, heads, float(scale),
+                                     dqkv.data_ptr(), torch.cuda.current_stream().cuda_stream)
+    if rc != 0:
+        raise RuntimeError("w2s_debug_attention_bwd: " + lib.w2s_last_error(None).decode())
+    return dqkv

@@ -145,7 +145,11 @@ def test_gradient_stages_match_autograd_tiny(P, variant, attn):
                                       ("wav2vec2-large", 4, 16000), ("tiny_layer_stable", 34, 9000),
                                       ("wav2vec2-large-lv60", 3, 16000), ("tiny_conformer_rel", 34, 9000),
                                       ("tiny_conformer_rotary", 33, 9000), ("wav2vec2-conformer-large", 3, 16000),
-                                      ("tiny_group", 2, 330000)])      # T' = 1031: nine key blocks in the fused attention backward
+                                      ("tiny_group", 2, 330000),       # T' = 1031: nine key blocks in the fused attention backward
+                                      # T' = 312 and 573 (the reference's clip): the relative-position conformer's unfused
+                                      # attention backward with the rel-shift in the softmax row kernel; rotary on the fused one
+                                      ("tiny_conformer_rel", 4, 100000), ("tiny_conformer_rotary", 4, 100000),
+                                      ("tiny_conformer_rel", 3, 183600), ("tiny_conformer_rotary", 3, 183600)])
 def test_input_gradients_match_autograd_at_batch_32(P, name, n, L):
     """d (max logit of frame j) / d waveform for >= 32 rows with different target frames (one ragged tile for the tiny
     model: 32 + 3) against torch autograd on the transformers model."""
@@ -217,8 +221,9 @@ def test_expected_gradients_explainer_properties(P):
 
 
 def test_gradient_path_rejects_unbuilt_configurations(P):
-    """What the gradient path does not cover fails loudly: the conformer's CUDA-core attention cross-check, and a target
-    frame outside the clip."""
+    """What the gradient path does not cover fails loudly: the conformer's CUDA-core attention cross-check, a target
+    frame outside the clip, and the relative-position conformer on clips past the 1024 frames its attention backward
+    takes (T' = 1031), before anything is launched."""
     cfg = VARIANTS["tiny_conformer_rel"]
     eng = P.Engine(build_model(cfg), cfg, max_batch=2)
     eng.grad_debug(False, simt_attention=True)
@@ -227,6 +232,12 @@ def test_gradient_path_rejects_unbuilt_configurations(P):
     eng.grad_debug(False, simt_attention=False)
     with pytest.raises(RuntimeError, match="target frame"):
         eng.grad_waveforms(torch.zeros((1, 4000), device="cuda"), [10 ** 6])
+    assert cfg.num_frames(330000) == 1031
+    with pytest.raises(RuntimeError, match="at most 1024 frames"):
+        eng.grad_waveforms(torch.zeros((1, 330000), device="cuda"), [0])
+    # the handle stays usable
+    g, _ = eng.grad_waveforms(torch.randn((1, 4000), device="cuda"), [0])
+    assert torch.isfinite(g).all()
     eng.close()
 
 
