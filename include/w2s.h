@@ -45,9 +45,9 @@ enum {
 };
 
 /* Mirrors transformers.Wav2Vec2Config / Wav2Vec2ConformerConfig (the objects the reference
- * obtains from from_pretrained at shap_calculation.py:218-219, w2v2conformer.py:58-59). */
+ * obtains from from_pretrained at shap_calculation.py:218-219, w2v2conformer.py:58-59) / WavLMConfig. */
 typedef struct {
-  int32_t kind;                 /* 0 = Wav2Vec2ForCTC, 1 = Wav2Vec2ConformerForCTC */
+  int32_t kind;                 /* 0 = Wav2Vec2ForCTC, 1 = Wav2Vec2ConformerForCTC, 2 = WavLMForCTC */
   int32_t num_conv_layers;
   int32_t conv_dim[W2S_MAX_CONV_LAYERS];
   int32_t conv_kernel[W2S_MAX_CONV_LAYERS];
@@ -69,11 +69,14 @@ typedef struct {
   int32_t rotary_embedding_base;
   int32_t max_batch;            /* coalitions evaluated per internal batch tile (0 = choose) */
   int32_t flags;                /* W2S_FLAG_* */
+  int32_t num_buckets;          /* WavLM: relative-position buckets (320) */
+  int32_t max_bucket_distance;  /* WavLM: distance where the log buckets saturate (800) */
 } w2s_config;
 
 /* Replaces model construction + .to(device) (shap_calculation.py:218-219,258).
  * `names[i]` are HF state_dict keys ("wav2vec2.feature_extractor.conv_layers.0.conv.weight", ...,
- * "lm_head.bias"; the weight-normed pos-conv must be passed folded as
+ * "lm_head.bias"; prefix "wav2vec2_conformer." for kind 1, "wavlm." for kind 2; the weight-normed pos-conv must be
+ * passed folded as
  * "<prefix>encoder.pos_conv_embed.conv.weight"), `ptrs[i]` fp32 DEVICE pointers in the HF layout with
  * `numels[i]` elements.  Weights are converted/re-laid-out into handle-owned storage; the caller may
  * free its copies after the call returns (the call synchronises the device once). */
@@ -119,7 +122,8 @@ int w2s_eval_waveforms(w2s_handle* h, const float* x_dev, int64_t n, int64_t L, 
  * x[n, L] (fp32, device, row stride `ld`) and one output frame per row (host array): out[r] = max_v logits[r,
  * frames[r], v] (shap_calculation.py:50) and grad[r, :] = d out[r] / d x[r, :] (fp32 [n, L], device).  Input
  * gradients only -- no weight gradients.  First slice: Wav2Vec2ForCTC with the group-norm front end and a post-LN
- * encoder (wav2vec2-base / -large); other configurations return an error. */
+ * encoder (wav2vec2-base / -large); other configurations return an error.  WavLMForCTC is refused: the backward of its
+ * gated relative-position bias is not built. */
 int w2s_grad_waveforms(w2s_handle* h, const float* x_dev, int64_t n, int64_t L, int64_t ld,
                        const int32_t* frames_host, float* grad_dev, float* out_dev, void* stream);
 /* The same backward pass seeded with an upstream gradient over ALL output frames -- the vector-Jacobian product autograd
@@ -171,6 +175,11 @@ int64_t w2s_sample_rows(int M, int n_full, int n_paired, const int64_t* ind_set,
                         int64_t samples_left, int64_t added, uint32_t* mt_key, int32_t* mt_pos,
                         uint32_t* z_words, double* weights, int64_t cap_rows, int64_t* ind_used);
 
+/* WavLM's relative-position buckets (HF wavlm/modeling_wavlm.py:253-271, _relative_positions_bucket) for a clip of T
+ * frames: out[r] = bucket(r - (T - 1)), r = 0 .. 2T-2, computed on the HOST in double precision.  Returns 0, or 1 on a bad
+ * argument (T < 1, num_buckets < 4, max_distance <= num_buckets / 4).  No device is touched. */
+int w2s_relative_buckets(int T, int num_buckets, int max_distance, int32_t* out);
+
 /* Test / profiling hooks for the individual kernels (used by tests/ and bench.py only). */
 /* out[M, N] = act(a[M, K] w[N, K]^T + bias) * alpha + residual (residual == out with fp32 data: in-place
  * accumulation, which the CTA-pair kernel performs with TMA reduce-add). */
@@ -185,6 +194,11 @@ int w2s_debug_gemm(int use_tcgen05, const void* a_bf16, const void* w_bf16, cons
  * Errors via w2s_last_error(NULL). */
 int w2s_debug_attention(int use_tcgen05, const void* qkv, const void* pos_proj, int B, int T, int heads, float scale,
                         void* ctx, float* lse, void* stream);
+/* w2s_debug_attention (no pos_proj) with WavLM's gated relative-position bias: score[b, h, i, j] += gate[b, h, i] *
+ * rel_bias[h, T - 1 + j - i], rel_bias [heads, 2T-1] and gate [B, heads, T] fp32 in natural units, device.  The bias
+ * variant writes no log-sum-exp: lse != NULL is an error.  Errors via w2s_last_error(NULL). */
+int w2s_debug_attention_bias(int use_tcgen05, const void* qkv, const float* rel_bias, const float* gate, int B, int T,
+                             int heads, float scale, void* ctx, float* lse, void* stream);
 /* Its backward (no relative positions): d ctx[B*T, H] -> dqkv[B*T, 3H] bf16.  use_tcgen05 = 1: the gradient path's fused
  * kernel with its delta pre-pass and dQ cast, fed the forward's ctx and lse (from w2s_debug_attention); 0: the CUDA-core
  * cross-check kernels (T <= 1024; ctx / lse unused).  The workspace is allocated and freed inside: the call synchronises

@@ -43,6 +43,8 @@ class W2SConfig(C.Structure):
         ("rotary_embedding_base", C.c_int32),
         ("max_batch", C.c_int32),
         ("flags", C.c_int32),
+        ("num_buckets", C.c_int32),
+        ("max_bucket_distance", C.c_int32),
     ]
 
 
@@ -73,10 +75,13 @@ SIGNATURES = {
                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "w2s_sample_rows": (C.c_int64, [C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "w2s_relative_buckets": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "w2s_debug_gemm": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_float,
                                  C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "w2s_debug_attention": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p,
                                       C.c_void_p, C.c_void_p]),
+    "w2s_debug_attention_bias": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float,
+                                           C.c_void_p, C.c_void_p, C.c_void_p]),
     "w2s_debug_attention_bwd": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                           C.c_float, C.c_void_p, C.c_void_p]),
     "w2s_profile_enable": (C.c_int, [C.c_void_p, C.c_int]),

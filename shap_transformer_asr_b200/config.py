@@ -6,8 +6,8 @@ The reference never stores an architecture itself: it pulls
 (feasability_tests/w2v2conformer.py:57) from the hub.  The hub is unreachable
 here, so the hyper-parameters below ARE the definition of the named
 architectures for this repo (SURVEY.md section 8c).  Field names follow
-``transformers.Wav2Vec2Config`` / ``Wav2Vec2ConformerConfig`` so a config object
-from either library can be converted with :func:`ModelConfig.from_hf`.
+``transformers.Wav2Vec2Config`` / ``Wav2Vec2ConformerConfig`` / ``WavLMConfig`` so a
+config object of any of them can be converted with :func:`ModelConfig.from_hf`.
 """
 from __future__ import annotations
 
@@ -17,7 +17,7 @@ from typing import Tuple
 
 @dataclass(frozen=True)
 class ModelConfig:
-    kind: str = "wav2vec2"                      # "wav2vec2" | "conformer"
+    kind: str = "wav2vec2"                      # "wav2vec2" | "conformer" | "wavlm"
     conv_dim: Tuple[int, ...] = (512,) * 7
     conv_kernel: Tuple[int, ...] = (10, 3, 3, 3, 3, 2, 2)
     conv_stride: Tuple[int, ...] = (5, 2, 2, 2, 2, 2, 2)
@@ -38,6 +38,9 @@ class ModelConfig:
     hidden_act: str = "gelu"                    # conformer hub checkpoints use "swish"
     rotary_embedding_base: int = 10000
     max_source_positions: int = 5000
+    # WavLM only: gated relative-position bias buckets
+    num_buckets: int = 320
+    max_bucket_distance: int = 800
 
     @property
     def head_dim(self) -> int:
@@ -63,8 +66,9 @@ class ModelConfig:
 
     @staticmethod
     def from_hf(cfg) -> "ModelConfig":
-        """Build from a transformers Wav2Vec2Config / Wav2Vec2ConformerConfig (duck-typed)."""
-        kind = "conformer" if "Conformer" in type(cfg).__name__ else "wav2vec2"
+        """Build from a transformers Wav2Vec2Config / Wav2Vec2ConformerConfig / WavLMConfig (duck-typed)."""
+        name = type(cfg).__name__
+        kind = "conformer" if "Conformer" in name else "wavlm" if "WavLM" in name else "wav2vec2"
         kw = dict(
             kind=kind,
             conv_dim=tuple(cfg.conv_dim), conv_kernel=tuple(cfg.conv_kernel),
@@ -84,6 +88,8 @@ class ModelConfig:
                       conv_depthwise_kernel_size=cfg.conv_depthwise_kernel_size,
                       rotary_embedding_base=cfg.rotary_embedding_base,
                       max_source_positions=cfg.max_source_positions)
+        if kind == "wavlm":
+            kw.update(num_buckets=cfg.num_buckets, max_bucket_distance=cfg.max_bucket_distance)
         return ModelConfig(**kw)
 
 
@@ -98,6 +104,12 @@ MODELS = {
         kind="conformer", hidden_size=1024, num_hidden_layers=24, num_attention_heads=16,
         intermediate_size=4096, conv_bias=True, feat_extract_norm="layer",
         position_embeddings_type="relative", hidden_act="swish"),
+    # transformers.WavLMConfig() defaults == microsoft/wavlm-base-plus (group-norm front end, post-LN encoder)
+    "wavlm-base-plus": ModelConfig(kind="wavlm"),
+    # microsoft/wavlm-large (layer-norm front end with conv bias, stable-LN encoder)
+    "wavlm-large": ModelConfig(kind="wavlm", hidden_size=1024, num_hidden_layers=24, num_attention_heads=16,
+                               intermediate_size=4096, feat_extract_norm="layer", conv_bias=True,
+                               do_stable_layer_norm=True),
     # tiny variants used by the CPU/GPU parity tests (same code paths, seconds on CPU)
     "wav2vec2-tiny": ModelConfig(hidden_size=128, num_hidden_layers=2, num_attention_heads=2,
                                  intermediate_size=256, conv_dim=(64,) * 7,
@@ -125,4 +137,7 @@ WORKLOADS = {
                    "wav2vec2-large 10 s clip, 200 segments, 8192 coalitions"),
     "C4": Workload("C4", "wav2vec2-conformer-large", 80000, 100, 4096,
                    "wav2vec2-conformer-large 5 s clip, 100 segments, 4096 coalitions"),
+    # C2's shape on WavLM: the attention cost of the gated relative-position bias compares directly with C2
+    "C6": Workload("C6", "wavlm-base-plus", 80000, 100, 2048,
+                   "wavlm-base-plus 5 s clip, 100 segments, 2048 coalitions"),
 }

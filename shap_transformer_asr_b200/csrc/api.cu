@@ -33,6 +33,8 @@ struct LayerW {
   float *lnc_g = nullptr, *lnc_b = nullptr, *lnfin_g = nullptr, *lnfin_b = nullptr;
   float *dw_w = nullptr, *dw_scale = nullptr, *dw_shift = nullptr;  // depthwise taps [H][k], folded BatchNorm
   bf16* pos_proj = nullptr;  // [2T-1, H], built per clip length
+  // WavLM: gru_rel_pos_linear [8, 64] / [8] and gru_rel_pos_const [heads] of this layer
+  float *gate_w = nullptr, *gate_b = nullptr, *gate_c = nullptr;
 };
 
 struct Step {
@@ -105,6 +107,7 @@ struct w2s_handle {
   bf16* pos_w = nullptr;
   float* pos_b = nullptr;
   float *enc_ln_g = nullptr, *enc_ln_b = nullptr;
+  float* rel_embed = nullptr;   // WavLM: layer 0's rel_attn_embed [num_buckets, heads], shared by every layer
   std::vector<LayerW> layers;
   bf16* head_w = nullptr;
   float* head_b = nullptr;
@@ -135,6 +138,8 @@ struct w2s_handle {
   float* pre = nullptr;
   float* logits = nullptr;
   bf16* hrot = nullptr;
+  float* rel_bias = nullptr;    // WavLM: bias table of the current clip length (AttnParams::rel_bias)
+  float* gate = nullptr;        // WavLM: [max_batch, heads, T'] gate of the current layer
   double* wls_work = nullptr;
   long long wls_cap = 0;
   std::map<int, std::unique_ptr<Plan>> plans;
@@ -290,7 +295,7 @@ std::string load_weights(w2s_handle* h, const WeightTable& wt) {
   W2S_TRY(copy_f32(h, wt, P + "encoder.layer_norm.weight", H, &h->enc_ln_g));
   W2S_TRY(copy_f32(h, wt, P + "encoder.layer_norm.bias", H, &h->enc_ln_b));
   h->layers.resize(c.num_hidden_layers);
-  if (c.kind == 0) {
+  if (c.kind != 1) {   // wav2vec2 and WavLM
     const int G = c.num_conv_pos_embedding_groups, kp = c.num_conv_pos_embeddings, cpg = H / G;
     const float* src = nullptr;
     W2S_TRY(wt.get(P + "encoder.pos_conv_embed.conv.weight", (int64_t)H * cpg * kp, &src));
@@ -326,7 +331,15 @@ std::string load_weights(w2s_handle* h, const WeightTable& wt) {
       W2S_TRY(copy_f32(h, wt, lp + "feed_forward.output_dense.bias", H, &w.b2));
       W2S_TRY(copy_f32(h, wt, lp + "final_layer_norm.weight", H, &w.ln2_g));
       W2S_TRY(copy_f32(h, wt, lp + "final_layer_norm.bias", H, &w.ln2_b));
+      if (c.kind == 2) {   // HF wavlm/modeling_wavlm.py:141-146
+        W2S_TRY(copy_f32(h, wt, lp + "attention.gru_rel_pos_linear.weight", 8 * 64, &w.gate_w));
+        W2S_TRY(copy_f32(h, wt, lp + "attention.gru_rel_pos_linear.bias", 8, &w.gate_b));
+        W2S_TRY(copy_f32(h, wt, lp + "attention.gru_rel_pos_const", c.num_attention_heads, &w.gate_c));
+      }
     }
+    if (c.kind == 2)   // only layer 0 has the embedding; HF passes its ungated bias down the stack (:410-430)
+      W2S_TRY(copy_f32(h, wt, P + "encoder.layers.0.attention.rel_attn_embed.weight",
+                       (int64_t)c.num_buckets * c.num_attention_heads, &h->rel_embed));
   } else {
     const int kd = c.conv_depthwise_kernel_size;
     for (int l = 0; l < c.num_hidden_layers; ++l) {
@@ -493,9 +506,24 @@ std::string ensure_workspace(w2s_handle* h, long long L) {
   W2S_TRY(dalloc(pool, &h->ctx, rows * H));
   W2S_TRY(dalloc(pool, &h->ffn, rows * I));
   W2S_TRY(dalloc(pool, &h->logits, rows * (size_t)h->head_ldl));
-  if (c.kind == 0) {
+  if (c.kind != 1) {
     W2S_TRY(dalloc(pool, &h->hp,
                    nb * (size_t)(T + c.num_conv_pos_embeddings) * c.num_conv_pos_embedding_groups * 64));
+    if (c.kind == 2) {
+      // WavLM: the relative-position bias table, input independent, built once per clip length from host-computed
+      // buckets (HF modeling_wavlm.py:234-243, :253-271)
+      const int heads = c.num_attention_heads;
+      std::vector<int32_t> bk((size_t)(2 * T - 1));
+      if (w2s_relative_buckets((int)T, c.num_buckets, c.max_bucket_distance, bk.data()) != 0)
+        return "WavLM: num_buckets / max_bucket_distance out of range";
+      int32_t* bk_dev = nullptr;
+      W2S_TRY(dalloc(pool, &bk_dev, bk.size()));
+      W2S_CUDA_OK(cudaMemcpy(bk_dev, bk.data(), sizeof(int32_t) * bk.size(), cudaMemcpyHostToDevice));
+      W2S_TRY(dalloc(pool, &h->rel_bias, (size_t)heads * rel_bias_ld((int)T)));
+      W2S_TRY(launch_rel_bias_table(h->rel_embed, bk_dev, (int)T, heads, h->rel_bias, 0));
+      W2S_TRY(dalloc(pool, &h->gate, rows * heads));
+      W2S_CUDA_OK(cudaDeviceSynchronize());
+    }
   } else {
     if (c.position_embeddings_type == 2) W2S_TRY(dalloc(pool, &h->hrot, rows * H));
     if (c.position_embeddings_type == 1) {
@@ -636,7 +664,7 @@ struct PlanBuilder {
     {
       GemmProblem p = plain(h->fpn, rows, Cl, h->fp_w, H);
       p.epi.bias = h->fp_b;
-      if (c.kind == 0) {
+      if (c.kind != 1) {
         p.epi.out = h->h0;
       } else {  // conformer: the un-normalised residual stream lives in fp32
         p.epi.out = h->pre;
@@ -644,7 +672,8 @@ struct PlanBuilder {
       }
       W2S_TRY(add_gemm("featproj", p));
     }
-    if (c.kind != 0) return build_conformer();
+    if (c.kind == 1) return build_conformer();
+    const bool wavlm = c.kind == 2;
     const bool stable = c.do_stable_layer_norm != 0;
     // ---- K4: positional conv (grouped, k=128) + GELU + residual (+ LayerNorm) ----------------------------
     {
@@ -677,6 +706,10 @@ struct PlanBuilder {
     ap.heads = c.num_attention_heads; ap.hd = H / c.num_attention_heads;
     ap.ld = 3 * H; ap.q_off = 0; ap.qv_off = 0; ap.k_off = H; ap.v_off = 2 * H;
     ap.scale = 1.0f / sqrtf((float)ap.hd);
+    if (wavlm) {
+      ap.rel_bias = h->rel_bias;
+      ap.gate = h->gate;
+    }
     // attention: the persistent tcgen05 kernel, or -- W2S_FLAG_VALIDATE_ATTN only -- the CUDA-core cross-check.
     // A shape the tensor-core kernel cannot take is an error, never a silent change of code path.
     AttnFaPlan* afl = nullptr;
@@ -703,6 +736,12 @@ struct PlanBuilder {
         p.epi.bias = w.bqkv;
         p.epi.out = h->qkv;
         W2S_TRY(add_gemm(ls + "qkv", p));
+      }
+      if (wavlm) {   // the gate reads the attention input hb (HF modeling_wavlm.py:160-176)
+        const float *gw = w.gate_w, *gb = w.gate_b, *gc = w.gate_c;
+        const int heads = ap.heads;
+        add(ls + "wavlm_gate", [=](cudaStream_t s) { return launch_wavlm_gate(hh->hb, nn, T, heads, gw, gb, gc, hh->gate, s); },
+            2.0 * rows * 8 * H, (double)rows * H * 2.0 + (double)rows * heads * 4.0);
       }
       if (afl) add(ls + "attention", [=](cudaStream_t s) { return attention_fa_launch(afl, s); }, attn_flops);
       else add(ls + "attention", [=](cudaStream_t s) { return launch_attention_simt(ap, s); }, attn_flops);
@@ -1037,6 +1076,15 @@ int w2s_create(const w2s_config* cfg, const char* const* names, const float* con
     g_create_error = "num_conv_layers out of range";
     return 1;
   }
+  if (cfg->kind < 0 || cfg->kind > 2) {
+    g_create_error = "unknown model kind " + std::to_string(cfg->kind) +
+                     " (0 = Wav2Vec2ForCTC, 1 = Wav2Vec2ConformerForCTC, 2 = WavLMForCTC)";
+    return 1;
+  }
+  if (cfg->kind == 2 && cfg->hidden_size != 64 * cfg->num_attention_heads) {
+    g_create_error = "WavLMForCTC: head_dim must be 64";
+    return 1;
+  }
   if (cfg->hidden_size % cfg->num_attention_heads) {
     g_create_error = "hidden_size must be divisible by num_attention_heads";
     return 1;
@@ -1048,7 +1096,7 @@ int w2s_create(const w2s_config* cfg, const char* const* names, const float* con
   if (e.empty()) e = attention_bwd_init();
   if (e.empty()) {
     WeightTable wt;
-    wt.prefix = cfg->kind == 1 ? "wav2vec2_conformer." : "wav2vec2.";
+    wt.prefix = cfg->kind == 1 ? "wav2vec2_conformer." : cfg->kind == 2 ? "wavlm." : "wav2vec2.";
     for (int i = 0; i < n_weights; ++i) wt.t[names[i]] = {ptrs[i], numels[i]};
     e = load_weights(h.get(), wt);
   }
@@ -1288,6 +1336,46 @@ int w2s_debug_attention(int use_tcgen05, const void* qkv, const void* pos_proj, 
   return 0;
 }
 
+int w2s_debug_attention_bias(int use_tcgen05, const void* qkv, const float* rel_bias, const float* gate, int B, int T,
+                             int heads, float scale, void* ctx, float* lse, void* stream) {
+  g_create_error.clear();
+  const cudaStream_t s = (cudaStream_t)stream;
+  AttnParams ap = debug_attn_params(qkv, nullptr, B, T, heads, scale);
+  ap.ctx = (bf16*)ctx;
+  ap.gate = gate;
+  std::string e;
+  float* table = nullptr;
+  if (B <= 0 || T <= 0 || heads <= 0 || !qkv || !ctx || !rel_bias || !gate) {
+    e = "debug_attention_bias: need B, T', heads >= 1 and qkv / rel_bias / gate / ctx buffers";
+  } else if (lse) {
+    e = "debug_attention_bias: the relative-position bias variant writes no log-sum-exp (lse must be NULL)";
+  } else if (cudaMalloc((void**)&table, sizeof(float) * heads * rel_bias_ld(T)) != cudaSuccess) {
+    e = "debug_attention_bias: out of device memory";
+  } else if (!(e = launch_rel_bias_table(rel_bias, nullptr, T, heads, table, s)).empty()) {
+  } else if (!(e = gemm_init()).empty()) {
+  } else {
+    ap.rel_bias = table;
+    if (!use_tcgen05) {
+      e = launch_attention_simt(ap, s);
+    } else {
+      AttnFaPlan* fp = nullptr;
+      e = attention_fa_init();
+      if (e.empty()) e = attention_fa_prepare(ap, debug_num_sms(), &fp);
+      if (e.empty()) e = attention_fa_launch(fp, s);
+      if (fp) attention_fa_free(fp);
+    }
+  }
+  // the table lives for this call only
+  const cudaError_t se = cudaStreamSynchronize(s);
+  if (se != cudaSuccess && e.empty()) e = std::string("debug_attention_bias: ") + cudaGetErrorString(se);
+  if (table) cudaFree(table);
+  if (!e.empty()) {
+    g_create_error = e;
+    return 1;
+  }
+  return 0;
+}
+
 int w2s_debug_attention_bwd(int use_tcgen05, const void* qkv, const void* ctx, const void* dctx, const float* lse, int B,
                             int T, int heads, float scale, void* dqkv, void* stream) {
   g_create_error.clear();
@@ -1397,8 +1485,9 @@ double w2s_flops_per_forward(const w2s_handle* h, int64_t L) {
     f += 2.0 * Tl[l] * c.conv_dim[l] * (l == 0 ? 1 : c.conv_dim[l - 1]) * c.conv_kernel[l];
   const double H = c.hidden_size, I = c.intermediate_size;
   f += 2.0 * T * c.conv_dim[c.num_conv_layers - 1] * H;
-  if (c.kind == 0) f += 2.0 * T * H * (H / c.num_conv_pos_embedding_groups) * c.num_conv_pos_embeddings;
+  if (c.kind != 1) f += 2.0 * T * H * (H / c.num_conv_pos_embedding_groups) * c.num_conv_pos_embeddings;
   double per_layer = 2.0 * T * H * 3 * H + 4.0 * T * T * H + 2.0 * T * H * H + 4.0 * T * H * I;
+  if (c.kind == 2) per_layer += 2.0 * T * 8 * H;                    // WavLM gate
   if (c.kind == 1) {
     per_layer += 4.0 * T * H * I;                                   // second macaron FFN
     per_layer += 2.0 * T * H * 2 * H + 2.0 * T * H * c.conv_depthwise_kernel_size + 2.0 * T * H * H;  // conv module

@@ -4,8 +4,8 @@
 //  * attention_fa.cu       : the tcgen05 kernel of the plain / rotary models (persistent, warp-specialised, key blocks
 //                            streamed through independent accumulators; any clip length).
 //  * attention_rel_kernel  : conformer relative-position attention on tcgen05 (any clip length).
-//  * attention_simt_kernel : CUDA-core cross-check (one warp per query row), reachable through W2S_FLAG_VALIDATE_ATTN
-//                            only -- never a fallback of the product path.
+//  * attention_simt_kernel : CUDA-core cross-check (one warp per query row, with the WavLM bias when given), reachable
+//                            through W2S_FLAG_VALIDATE_ATTN only -- never a fallback of the product path.
 #include "kernels.cuh"
 #include "gemm.cuh"
 
@@ -32,6 +32,9 @@ __global__ void __launch_bounds__(128) attention_simt_kernel(const AttnParams p)
     qs[warp][1][d] = p.pos_proj ? __bfloat162float(qrow[p.qv_off + d]) : 0.f;
   }
   __syncwarp();
+  // WavLM: gate * table entry (log2 units) * ln 2 = the natural-units bias
+  const float gb = p.rel_bias ? p.gate[((long long)b * p.heads + h) * p.T + i] * 0.6931471805599453f : 0.f;
+  const float* brow = p.rel_bias ? p.rel_bias + (long long)h * rel_bias_ld(p.T) + REL_BIAS_PAD + p.T - 1 - i : nullptr;
   float s[SIMT_MAXC];
   float mx = -INFINITY;
 #pragma unroll
@@ -56,6 +59,7 @@ __global__ void __launch_bounds__(128) attention_simt_kernel(const AttnParams p)
         }
       }
       acc *= p.scale;
+      if (brow) acc = fmaf(gb, brow[j], acc);
     }
     s[c] = acc;
     mx = fmaxf(mx, acc);

@@ -17,8 +17,14 @@
 // O accumulators stay double-buffered (the first version held all blocks of an item in TMEM: T' <= 512, single-buffered
 // beyond 256).
 // HF wav2vec2/modeling_wav2vec2.py:438-463 (softmax(Q K^T / sqrt d) V, no mask, eval mode).
+// BIAS (WavLM, HF wavlm/modeling_wavlm.py:147-186): every score gains the gated relative-position bias
+// g[b, h, i] * E[bucket(j - i), h].  The softmax thread of query row i adds it to each score read from TMEM, in both
+// passes, before the padding mask; the Toeplitz table is read through L1 (lanes are consecutive query rows, so a warp's
+// read of one key column covers 32 consecutive floats), shared memory being full.
 #include "kernels.cuh"
 #include "gemm.cuh"
+
+#include <type_traits>
 
 namespace w2s {
 
@@ -28,9 +34,15 @@ struct AttnFaDev {
   int B, T, H, heads, qtiles, num_items, nb;
   float scale_log2e;
 };
+// the bias variant's parameters extend the plain ones (which stay as they are: a larger parameter block alone changes
+// how the plain variants are scheduled)
+struct AttnFaBiasDev : AttnFaDev {
+  const float* rel_bias;   // [heads, rel_bias_ld(T)], see AttnParams
+  const float* gate;       // [B, heads, T]
+};
 struct AttnFaPlan {
   CUtensorMap mapQ, mapK, mapV;
-  AttnFaDev dev;
+  AttnFaBiasDev dev;   // rel_bias == null: the plain variant
   int nb, grid;
 };
 
@@ -45,10 +57,10 @@ constexpr size_t FA_SMEM = FA_BAR + 512 + 1024;
 
 __device__ __forceinline__ uint64_t fa_desc_mn(uint32_t a) { return umma_desc_sw128(a); }
 
-template <int NBT>
+template <int NBT, bool BIAS>
 __global__ void __launch_bounds__(384, 1)
 attention_fa_kernel(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensorMap mapK,
-                    const __grid_constant__ CUtensorMap mapV, const AttnFaDev p) {
+                    const __grid_constant__ CUtensorMap mapV, const std::conditional_t<BIAS, AttnFaBiasDev, AttnFaDev> p) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw = smem_u32(smem_raw);
   const uint32_t base = (raw + 1023u) & ~1023u;
@@ -215,6 +227,16 @@ attention_fa_kernel(const __grid_constant__ CUtensorMap mapQ, const __grid_const
     const uint32_t sp_row = base + FA_SP + grp * 32768 + row * 128;
     const uint32_t sw = (uint32_t)row & 7u;
     const float2 sc2 = make_float2(p.scale_log2e, p.scale_log2e);
+    // BIAS: this thread's query row i of the current item reads table entry 128 + T - 1 - i + key, scaled by its gate
+    // (divided by scale_log2e: the scores stay unscaled until the exponentials)
+    const float* brow = nullptr;
+    float gsc = 0.f;
+    auto add_bias = [&](float (&v)[32], int key0) {
+      if constexpr (BIAS) {
+#pragma unroll
+        for (int t = 0; t < 32; ++t) v[t] = fmaf(gsc, __ldg(brow + key0 + t), v[t]);
+      }
+    };
 
     auto mask_tail = [&](float (&v)[32], int col0, int nvalid) {
 #pragma unroll
@@ -288,7 +310,7 @@ attention_fa_kernel(const __grid_constant__ CUtensorMap mapQ, const __grid_const
       const float inv = rcp_approx(L);
       const int qt = item % p.qtiles, h = (item / p.qtiles) % p.heads, b = item / (p.qtiles * p.heads);
       const int i = qt * 128 + row;
-      if (p.lse && grp == 0 && i < p.T) p.lse[((long long)b * p.heads + h) * p.T + i] = fmaf(m, p.scale_log2e, __log2f(L));
+      if (!BIAS && p.lse && grp == 0 && i < p.T) p.lse[((long long)b * p.heads + h) * p.T + i] = fmaf(m, p.scale_log2e, __log2f(L));
       if (i < p.T) {
         __nv_bfloat16* orow = p.ctx + ((long long)b * p.T + i) * p.H + h * 64 + grp * 32;
 #pragma unroll
@@ -314,6 +336,8 @@ attention_fa_kernel(const __grid_constant__ CUtensorMap mapQ, const __grid_const
       tmem_ld_32x32_issue(s_addr, s0);
       tmem_ld_32x32_issue(s_addr + 32, s1);
       tmem_ld_wait();
+      add_bias(s0, j * 128);
+      add_bias(s1, j * 128 + 32);
       if (nvalid < 64) {
         mask_tail(s0, 0, nvalid);
         mask_tail(s1, 32, nvalid);
@@ -322,6 +346,8 @@ attention_fa_kernel(const __grid_constant__ CUtensorMap mapQ, const __grid_const
       tmem_ld_32x32_issue(s_addr + 64, s0);
       tmem_ld_32x32_issue(s_addr + 96, s1);
       tmem_ld_wait();
+      add_bias(s0, j * 128 + 64);
+      add_bias(s1, j * 128 + 96);
       if (nvalid < 128) {
         mask_tail(s0, 64, nvalid);
         mask_tail(s1, 96, nvalid);
@@ -353,6 +379,8 @@ attention_fa_kernel(const __grid_constant__ CUtensorMap mapQ, const __grid_const
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(s_empty(grp));   // the MMA warp may overwrite this S buffer
+      add_bias(s0, j * 128);
+      add_bias(s1, j * 128 + 32);
       if (nvalid < 64) {
         mask_tail(s0, 0, nvalid);
         mask_tail(s1, 32, nvalid);
@@ -373,6 +401,12 @@ attention_fa_kernel(const __grid_constant__ CUtensorMap mapQ, const __grid_const
     int pend_item = 0, pend_nbc = 0;
     uint32_t pend_gcx = 0;
     for (int item = blockIdx.x; item < p.num_items; item += gridDim.x, ++it) {
+      if constexpr (BIAS) {
+        const int qt = item % p.qtiles, h = (item / p.qtiles) % p.heads, b = item / (p.qtiles * p.heads);
+        const int i = qt * 128 + row;   // padding rows (i >= T') stay inside the table's zero margins, with gate 0
+        brow = p.rel_bias + (long long)h * rel_bias_ld(p.T) + REL_BIAS_PAD + (p.T - 1 - i);
+        gsc = i < p.T ? p.gate[((long long)b * p.heads + h) * p.T + i] / p.scale_log2e : 0.f;
+      }
 #pragma unroll 1
       for (int c = 0; c < CPI; ++c) {
         const uint32_t gcx = (uint32_t)it * (uint32_t)CPI + (uint32_t)c;
@@ -413,19 +447,30 @@ bool attention_fa_supported(const AttnParams& p) {
   return p.hd == 64 && p.pos_proj == nullptr && (p.H % 8 == 0);
 }
 
+template <bool BIAS>
+static cudaError_t attention_fa_set_smem() {
+  cudaError_t e = cudaFuncSetAttribute(attention_fa_kernel<1, BIAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FA_SMEM);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(attention_fa_kernel<2, BIAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FA_SMEM);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(attention_fa_kernel<0, BIAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FA_SMEM);
+  return e;
+}
+
 std::string attention_fa_init() {
-  cudaError_t e = cudaFuncSetAttribute(attention_fa_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FA_SMEM);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(attention_fa_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FA_SMEM);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(attention_fa_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FA_SMEM);
+  cudaError_t e = attention_fa_set_smem<false>();
+  if (e == cudaSuccess) e = attention_fa_set_smem<true>();
   if (e != cudaSuccess) return std::string("cudaFuncSetAttribute(attention_fa_kernel): ") + cudaGetErrorString(e);
   return "";
 }
 
 std::string attention_fa_prepare(const AttnParams& p, int num_sms, AttnFaPlan** out) {
   if (!attention_fa_supported(p)) return "attention (tcgen05): unsupported shape";
+  if ((p.rel_bias == nullptr) != (p.gate == nullptr)) return "attention (tcgen05): the bias table and the gate go together";
+  if (p.rel_bias && p.lse) return "attention (tcgen05): the log-sum-exp is not written with a relative-position bias";
   AttnFaPlan* pl = new AttnFaPlan();
   pl->dev.ctx = p.ctx;
   pl->dev.lse = p.lse;
+  pl->dev.rel_bias = p.rel_bias;
+  pl->dev.gate = p.gate;
   pl->dev.B = p.B; pl->dev.T = p.T; pl->dev.H = p.H; pl->dev.heads = p.heads;
   pl->dev.qtiles = (p.T + 127) / 128;
   pl->dev.num_items = pl->dev.qtiles * p.heads * p.B;
@@ -448,12 +493,18 @@ std::string attention_fa_prepare(const AttnParams& p, int num_sms, AttnFaPlan** 
   return "";
 }
 
-std::string attention_fa_launch(const AttnFaPlan* pl, cudaStream_t s) {
+template <bool BIAS>
+static cudaError_t attention_fa_launch_as(const AttnFaPlan* pl, cudaStream_t s) {
+  const std::conditional_t<BIAS, AttnFaBiasDev, AttnFaDev>& dev = pl->dev;
   switch (pl->nb) {
-    case 1: W2S_CUDA_OK(launch_pdl(attention_fa_kernel<1>, dim3(pl->grid), dim3(384), FA_SMEM, s, 1, pl->mapQ, pl->mapK, pl->mapV, pl->dev)); break;
-    case 2: W2S_CUDA_OK(launch_pdl(attention_fa_kernel<2>, dim3(pl->grid), dim3(384), FA_SMEM, s, 1, pl->mapQ, pl->mapK, pl->mapV, pl->dev)); break;
-    default: W2S_CUDA_OK(launch_pdl(attention_fa_kernel<0>, dim3(pl->grid), dim3(384), FA_SMEM, s, 1, pl->mapQ, pl->mapK, pl->mapV, pl->dev)); break;
+    case 1: return launch_pdl(attention_fa_kernel<1, BIAS>, dim3(pl->grid), dim3(384), FA_SMEM, s, 1, pl->mapQ, pl->mapK, pl->mapV, dev);
+    case 2: return launch_pdl(attention_fa_kernel<2, BIAS>, dim3(pl->grid), dim3(384), FA_SMEM, s, 1, pl->mapQ, pl->mapK, pl->mapV, dev);
+    default: return launch_pdl(attention_fa_kernel<0, BIAS>, dim3(pl->grid), dim3(384), FA_SMEM, s, 1, pl->mapQ, pl->mapK, pl->mapV, dev);
   }
+}
+
+std::string attention_fa_launch(const AttnFaPlan* pl, cudaStream_t s) {
+  W2S_CUDA_OK(pl->dev.rel_bias ? attention_fa_launch_as<true>(pl, s) : attention_fa_launch_as<false>(pl, s));
   W2S_CUDA_OK(cudaGetLastError());
   return "";
 }

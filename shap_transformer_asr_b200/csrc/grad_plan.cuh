@@ -61,6 +61,7 @@ struct GradPlan {
 
 std::string grad_supported(const w2s_handle* h) {
   const w2s_config& c = h->cfg;
+  if (c.kind == 2) return "gradient path: WavLMForCTC is not supported (no backward of its gated relative-position bias)";
   if (c.kind == 0) {
     if (c.hidden_act != 0) return "gradient path: Wav2Vec2ForCTC is built for GELU only";
     if (c.num_conv_pos_embeddings % 2) return "gradient path: odd positional-conv kernels are not built";

@@ -95,7 +95,22 @@ struct AttnParams {
   // conformer relative positions (null when unused): the biases u / v are already folded into the q+u / q+v columns
   const __nv_bfloat16* pos_proj;  // [2T-1, H] linear_pos(rel_pos_emb), row r <-> relative position T-1-r
   float* lse;                     // optional (attention_fa only): [B, heads, T] log2-domain log-sum-exp, saved for the backward
+  // WavLM gated relative-position bias (null when unused; attention_fa and the CUDA-core kernel): score[i, j] +=
+  // gate[b, h, i] * E[bucket(j - i), h].  rel_bias[h][REL_BIAS_PAD + T - 1 + j - i] = E[bucket(j - i), h] * log2(e), fp32,
+  // with REL_BIAS_PAD zeros on both sides (rows rel_bias_ld(T) apart), so the padding queries and keys of a 128-wide
+  // tile index inside the table
+  const float* rel_bias;
+  const float* gate;              // [B, heads, T] fp32
 };
+constexpr int REL_BIAS_PAD = 128;
+__host__ __device__ constexpr int rel_bias_ld(int T) { return 2 * T - 1 + 2 * REL_BIAS_PAD; }
+// rel_bias table of AttnParams, [heads, rel_bias_ld(T)]: from E [num_buckets, heads] and bucket[2T-1] (entry r <->
+// relative position r - (T-1)), or, with bucket == null, from a full natural-units table src [heads, 2T-1]
+std::string launch_rel_bias_table(const float* src, const int32_t* bucket, int T, int heads, float* out, cudaStream_t s);
+// WavLM gate (HF wavlm/modeling_wavlm.py:166-176), head_dim 64: x [B*T, heads*64] bf16 (the attention input), w [8, 64],
+// b [8], c [heads] -> gate[B, heads, T] = a (c_h b' - 1) + 2, (a, b') = sigmoid(sums of 4 of the 8 outputs W x_h + b)
+std::string launch_wavlm_gate(const __nv_bfloat16* x, int B, int T, int heads, const float* w, const float* b,
+                              const float* c, float* gate, cudaStream_t s);
 std::string launch_attention_simt(const AttnParams& p, cudaStream_t s);
 // persistent, warp-specialised tcgen05 kernel with independent key blocks (attention_fa.cu)
 struct AttnFaPlan;

@@ -16,6 +16,11 @@ from .config import ModelConfig
 from .preprocess import pack_coalitions, segment_bounds
 
 
+# ModelConfig.kind -> w2s_config.kind and the HF state_dict prefix of the encoder
+KIND_IDS = {"wav2vec2": 0, "conformer": 1, "wavlm": 2}
+PREFIXES = {"wav2vec2": "wav2vec2.", "conformer": "wav2vec2_conformer.", "wavlm": "wavlm."}
+
+
 def _fold_pos_conv(sd: Dict[str, torch.Tensor], prefix: str) -> None:
     """weight_norm(dim=2) fold (HF wav2vec2/modeling_wav2vec2.py:337-354): w = g * v / ||v||_(0,1)."""
     p = prefix + "encoder.pos_conv_embed.conv."
@@ -32,7 +37,7 @@ def _fold_pos_conv(sd: Dict[str, torch.Tensor], prefix: str) -> None:
 
 class Engine:
     """B200 evaluation engine for one model.  ``model`` may be a ``transformers`` Wav2Vec2ForCTC /
-    Wav2Vec2ConformerForCTC instance (what the reference builds at shap_calculation.py:218-219) or a
+    Wav2Vec2ConformerForCTC / WavLMForCTC instance (what the reference builds at shap_calculation.py:218-219) or a
     plain ``state_dict`` with HF parameter names plus an explicit :class:`ModelConfig`."""
 
     def __init__(self, model, config: Optional[ModelConfig] = None, device: int = 0, max_batch: int = 0,
@@ -52,7 +57,7 @@ class Engine:
                 raise ValueError("a ModelConfig is required when passing a bare state_dict")
             sd = dict(model)
         self.config = config
-        prefix = "wav2vec2_conformer." if config.kind == "conformer" else "wav2vec2."
+        prefix = PREFIXES[config.kind]
         _fold_pos_conv(sd, prefix)
         keep = {}
         for k, v in sd.items():
@@ -64,7 +69,7 @@ class Engine:
                 continue
             keep[k] = v.to(device=self.device, dtype=torch.float32).contiguous()
         cfg = _lib.W2SConfig()
-        cfg.kind = 1 if config.kind == "conformer" else 0
+        cfg.kind = KIND_IDS[config.kind]
         cfg.num_conv_layers = len(config.conv_dim)
         for i in range(len(config.conv_dim)):
             cfg.conv_dim[i] = config.conv_dim[i]
@@ -86,6 +91,8 @@ class Engine:
         cfg.conv_depthwise_kernel_size = config.conv_depthwise_kernel_size
         cfg.hidden_act = {"gelu": 0, "swish": 1, "silu": 1}[config.hidden_act]
         cfg.rotary_embedding_base = config.rotary_embedding_base
+        cfg.num_buckets = config.num_buckets
+        cfg.max_bucket_distance = config.max_bucket_distance
         cfg.max_batch = int(max_batch)
         cfg.flags = ((_lib.FLAG_VALIDATE_GEMM if validate_gemm else 0) | (_lib.FLAG_VALIDATE_ATTN if validate_attn else 0)
                      | (_lib.FLAG_FP32_PRELN if preln_fp32 else 0) | (0 if graphs else _lib.FLAG_NO_GRAPH))
@@ -353,6 +360,40 @@ def debug_attention(qkv: torch.Tensor, B: int, heads: int, pos_proj=None, scale:
     if rc != 0:
         raise RuntimeError("w2s_debug_attention: " + lib.w2s_last_error(None).decode())
     return ctx, lse
+
+
+def debug_attention_bias(qkv: torch.Tensor, B: int, heads: int, rel_bias: torch.Tensor, gate: torch.Tensor,
+                         scale: float = 0.125, tcgen05: bool = True, ctx=None, lse=None):
+    """`debug_attention` with WavLM's gated relative-position bias (tests only): score[b, h, i, j] += gate[b, h, i] *
+    rel_bias[h, T - 1 + j - i], with rel_bias [heads, 2T-1] and gate [B, heads, T] fp32 in natural units.  The bias
+    variant writes no log-sum-exp: passing ``lse`` raises.  Returns ctx [B*T, H] bf16 (``ctx`` may be a caller buffer)."""
+    lib = _lib.load()
+    H = 64 * heads
+    T = qkv.shape[0] // B
+    _check_buffer("qkv", qkv, torch.bfloat16, B * T * 3 * H)
+    if qkv.shape != (B * T, 3 * H):
+        raise ValueError(f"qkv: shape {tuple(qkv.shape)} does not fit B={B}, heads={heads}")
+    _check_buffer("rel_bias", rel_bias, torch.float32, heads * (2 * T - 1))
+    _check_buffer("gate", gate, torch.float32, B * heads * T)
+    if ctx is None:
+        ctx = torch.empty((B * T, H), dtype=torch.bfloat16, device=qkv.device)
+    _check_buffer("ctx", ctx, torch.bfloat16, B * T * H)
+    rc = lib.w2s_debug_attention_bias(int(tcgen05), qkv.data_ptr(), rel_bias.data_ptr(), gate.data_ptr(), B, T, heads,
+                                      float(scale), ctx.data_ptr(), lse.data_ptr() if lse is not None else None,
+                                      torch.cuda.current_stream().cuda_stream)
+    if rc != 0:
+        raise RuntimeError("w2s_debug_attention_bias: " + lib.w2s_last_error(None).decode())
+    return ctx
+
+
+def relative_buckets(T: int, num_buckets: int = 320, max_distance: int = 800) -> np.ndarray:
+    """WavLM's relative-position buckets for a clip of T frames as the library computes them (host, no device):
+    int32 [2T-1], entry r for relative position r - (T - 1)."""
+    lib = _lib.load()
+    out = np.empty(2 * T - 1, dtype=np.int32)
+    if lib.w2s_relative_buckets(int(T), int(num_buckets), int(max_distance), out.ctypes.data) != 0:
+        raise ValueError("w2s_relative_buckets: bad argument")
+    return out
 
 
 def debug_attention_bwd(qkv: torch.Tensor, dctx: torch.Tensor, B: int, heads: int, ctx=None, lse=None, scale: float = 0.125,

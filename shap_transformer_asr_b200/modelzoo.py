@@ -29,6 +29,10 @@ def build_random_init_model(cfg: ModelConfig, seed: int = 0, perturb_affine: boo
             conv_depthwise_kernel_size=cfg.conv_depthwise_kernel_size, rotary_embedding_base=cfg.rotary_embedding_base,
             max_source_positions=cfg.max_source_positions, **common)
         model = transformers.Wav2Vec2ConformerForCTC(hf_cfg)
+    elif cfg.kind == "wavlm":
+        hf_cfg = transformers.WavLMConfig(do_stable_layer_norm=cfg.do_stable_layer_norm, num_buckets=cfg.num_buckets,
+                                          max_bucket_distance=cfg.max_bucket_distance, **common)
+        model = transformers.WavLMForCTC(hf_cfg)
     else:
         hf_cfg = transformers.Wav2Vec2Config(do_stable_layer_norm=cfg.do_stable_layer_norm, **common)
         model = transformers.Wav2Vec2ForCTC(hf_cfg)
@@ -43,6 +47,8 @@ def build_random_init_model(cfg: ModelConfig, seed: int = 0, perturb_affine: boo
                     p.add_(0.05 * torch.randn(p.shape, generator=g))
                 elif name.endswith("pos_bias_u") or name.endswith("pos_bias_v"):
                     p.add_(0.05 * torch.randn(p.shape, generator=g))
+                elif name.endswith("gru_rel_pos_const"):   # WavLM: random init leaves it at 1
+                    p.add_(0.25 * torch.randn(p.shape, generator=g))
             for name, b in model.named_buffers():
                 if name.endswith("running_mean"):
                     b.add_(0.05 * torch.randn(b.shape, generator=g))
