@@ -97,6 +97,19 @@ int64_t w2s_num_frames(const w2s_handle* h, int64_t num_samples);
 int w2s_set_clip(w2s_handle* h, const float* x_dev, int64_t L, const int32_t* seg_bounds_host, int M,
                  float baseline, void* stream);
 
+/* Background dataset of shap.KernelExplainer(f, data): B rows bg[B, L] (fp32, device, row stride `ld` elements, in the
+ * same normalised input space as the clip; copied into the handle, so the caller may free them when this returns) with
+ * weights w[B] (host, fp64: finite, >= 0, positive sum; normalised here in fp64 and stored as fp32).  1 <= B <=
+ * W2S_MAX_BACKGROUND; L must equal the current clip's length (checked again by w2s_eval / w2s_mask when w2s_set_clip has
+ * changed it since).  B = 0 clears the background and restores the baseline fill exactly.
+ * While a background is set, coalition k is evaluated as B rows: row (k, b) takes sample i from the clip where segment
+ * seg(i) is kept and from bg[b][i] where it is dropped; the baseline of w2s_set_clip is ignored.  w2s_eval then reports
+ * out[k, :] = sum_b w_b * f(row (k, b)), accumulated in fp32 in the order b = 0 .. B-1 with one fmaf per term from 0 --
+ * independent of the batch tile and of how the coalitions are spread over GPUs.  The call synchronises `stream`. */
+#define W2S_MAX_BACKGROUND 256
+int w2s_set_background(w2s_handle* h, const float* bg_dev, int64_t B, int64_t L, int64_t ld, const double* weights_host,
+                       void* stream);
+
 /* Replaces timestep_to_explain / token_id_to_explain (w2v2conformer.py:93-110) and the character-frame
  * list of visualization.py:319-327: D (frame, token) pairs (host arrays, copied before the call returns; ignored
  * for MAX/MEAN/LOGITS).  The upload is ordered on `stream` behind evaluations already queued there. */
@@ -107,7 +120,8 @@ int w2s_set_targets(w2s_handle* h, const int32_t* frame_idx_host, const int32_t*
 int64_t w2s_out_width(const w2s_handle* h, int64_t num_samples);
 
 /* The fused masker + model callable: coalition bit matrix z_bits[K, ceil(M/32)] (device; bit m of row k
- * set = segment m KEPT, clear = replaced by the baseline) -> out[K, width] fp32 (device). */
+ * set = segment m KEPT, clear = replaced by the baseline) -> out[K, width] fp32 (device).  With a background
+ * (w2s_set_background) K * B rows are evaluated and out[K, width] holds their weighted means. */
 int w2s_eval(w2s_handle* h, const uint32_t* z_bits_dev, int64_t K, float* out_dev, void* stream);
 
 /* Replaces ModelWrapper.forward (shap_calculation.py:31-50), predict_function
@@ -150,7 +164,8 @@ int w2s_grad_rules(w2s_handle* h, int rules);
 int64_t w2s_grad_peek(w2s_handle* h, const char* name, void* dst_dev, int64_t max_bytes, void* stream);
 
 /* Standalone masker (conformer_test.ipynb:138-141 semantics with keep-bits): materialise
- * out[K, L] = keep ? x : baseline for the clip set by w2s_set_clip. */
+ * out[K, L] = keep ? x : baseline for the clip set by w2s_set_clip; with a background, out[K * B, L] with row k * B + b =
+ * keep ? x : bg[b] -- the rows w2s_eval evaluates, in its order. */
 int w2s_mask(w2s_handle* h, const uint32_t* z_bits_dev, int64_t K, float* out_dev, void* stream);
 
 /* KernelSHAP constrained weighted least squares (shap KernelExplainer.solve with l1_reg=False; SURVEY.md

@@ -17,6 +17,7 @@ MAX_CONV_LAYERS = 8
 OUT_MAX, OUT_LOGIT, OUT_LOGPROB, OUT_MEAN, OUT_LOGITS = 0, 1, 2, 3, 4
 MODE_IDS = {"max": OUT_MAX, "logit": OUT_LOGIT, "logprob": OUT_LOGPROB, "mean": OUT_MEAN, "logits": OUT_LOGITS}
 FLAG_VALIDATE_GEMM, FLAG_VALIDATE_ATTN, FLAG_FP32_PRELN, FLAG_NO_GRAPH = 1, 2, 4, 16
+MAX_BACKGROUND = 256      # W2S_MAX_BACKGROUND: rows of a background set
 
 
 class W2SConfig(C.Structure):
@@ -57,6 +58,8 @@ SIGNATURES = {
     "w2s_num_frames": (C.c_int64, [C.c_void_p, C.c_int64]),
     "w2s_set_clip": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(C.c_int32), C.c_int, C.c_float,
                                C.c_void_p]),
+    "w2s_set_background": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.POINTER(C.c_double),
+                                     C.c_void_p]),
     "w2s_set_targets": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int, C.c_int,
                                   C.c_void_p]),
     "w2s_out_width": (C.c_int64, [C.c_void_p, C.c_int64]),

@@ -6,6 +6,7 @@
 #include "kernels.cuh"
 
 #include <algorithm>
+#include <cmath>
 #include <cstdlib>
 #include <cstring>
 #include <functional>
@@ -120,6 +121,16 @@ struct w2s_handle {
   uint16_t* seg_id = nullptr;
   long long clip_cap = 0;
 
+  // background (w2s_set_background): bg_B rows of bg_L samples replace the baseline; bg_B == 0: none
+  int bg_B = 0;
+  long long bg_L = 0;
+  float* bg = nullptr;              // [bg_B, bg_L]
+  long long bg_cap = 0;             // floats
+  float* bg_w = nullptr;            // [W2S_MAX_BACKGROUND] normalised weights, fp32
+  std::vector<float> bg_w_host;     // staging of the upload
+  float* bg_rows = nullptr;         // [K * bg_B, width] per-row outputs of the last w2s_eval, reduced by bg_mean_kernel
+  long long bg_rows_cap = 0;        // floats; only grows
+
   // targets
   int mode = W2S_OUT_MAX, D = 0, max_frame = 0;
   int *frames = nullptr, *tokens = nullptr;
@@ -142,7 +153,7 @@ struct w2s_handle {
   float* gate = nullptr;        // WavLM: [max_batch, heads, T'] gate of the current layer
   double* wls_work = nullptr;
   long long wls_cap = 0;
-  std::map<int, std::unique_ptr<Plan>> plans;
+  std::map<std::pair<int, bool>, std::unique_ptr<Plan>> plans;   // keyed by (tile rows, background fill)
 
   // optional per-launch CUDA-event profile (bench.py roofline leg)
   bool profiling = false;
@@ -194,6 +205,9 @@ struct w2s_handle {
     if (dyn_dev) cudaFree(dyn_dev);
     if (clip) cudaFree(clip);
     if (seg_id) cudaFree(seg_id);
+    if (bg) cudaFree(bg);
+    if (bg_w) cudaFree(bg_w);
+    if (bg_rows) cudaFree(bg_rows);
     if (frames) cudaFree(frames);
     if (tokens) cudaFree(tokens);
     if (wls_work) cudaFree(wls_work);
@@ -557,6 +571,7 @@ struct PlanBuilder {
   Plan* plan;
   int n;
   bool simt_gemm, simt_attn;
+  bool bg;   // conv0 fills dropped samples from the background (DynArgs::bg)
 
   std::string add_gemm(const std::string& name, const GemmProblem& p) {
     GemmLaunch* gl = new GemmLaunch();
@@ -631,11 +646,14 @@ struct PlanBuilder {
       cp.ln_wbar = h->ln0_wbar; cp.ln_gram = h->ln0_gram; cp.ln_wb = h->ln0_wb;
       cp.ln_bmean = h->ln0_bmean; cp.ln_b2mean = h->ln0_b2mean; cp.ln_wb48 = h->ln0_wb48;
       cp.out = h->bufA;
+      const bool fill = bg;
+      // with a background every row reads its background row besides the clip (both L2-resident across the tile)
+      const double wave_bytes = (fill ? 8.0 : 4.0) * (double)h->ws_L;
       if (!layer)
-        add("conv0_stats", [=](cudaStream_t s) { return launch_conv0_stats(cp, s); }, 0.0,
-            (4.0 * (double)h->ws_L + (double)cp.C * (8.0 + 64.0)) * n);
-      add("conv0", [=](cudaStream_t s) { return launch_conv0(cp, layer, s); },
-          2.0 * cp.T0 * (double)cp.C * cp.kw * n, ((double)cp.T0 * cp.C * 2.0 + 4.0 * (double)h->ws_L) * n);
+        add("conv0_stats", [=](cudaStream_t s) { return launch_conv0_stats(cp, s, fill); }, 0.0,
+            (wave_bytes + (double)cp.C * (8.0 + 64.0)) * n);
+      add("conv0", [=](cudaStream_t s) { return launch_conv0(cp, layer, s, fill); },
+          2.0 * cp.T0 * (double)cp.C * cp.kw * n, ((double)cp.T0 * cp.C * 2.0 + wave_bytes) * n);
     }
     // ---- K2: conv1..6 as implicit GEMM over the stride-row view of the previous layer ---------------------
     bf16* cur = h->bufA;
@@ -892,18 +910,19 @@ std::string PlanBuilder::build_conformer() {
   return "";
 }
 
-std::string get_plan(w2s_handle* h, int n, Plan** out) {
-  auto it = h->plans.find(n);
+std::string get_plan(w2s_handle* h, int n, bool bg, Plan** out) {
+  auto it = h->plans.find({n, bg});
   if (it != h->plans.end()) {
     *out = it->second.get();
     return "";
   }
   std::unique_ptr<Plan> pl(new Plan());
   pl->n = n;
-  PlanBuilder b{h, pl.get(), n, (h->cfg.flags & W2S_FLAG_VALIDATE_GEMM) != 0, (h->cfg.flags & W2S_FLAG_VALIDATE_ATTN) != 0};
+  PlanBuilder b{h, pl.get(), n, (h->cfg.flags & W2S_FLAG_VALIDATE_GEMM) != 0, (h->cfg.flags & W2S_FLAG_VALIDATE_ATTN) != 0,
+                bg};
   W2S_TRY(b.build());
   *out = pl.get();
-  h->plans[n] = std::move(pl);
+  h->plans[{n, bg}] = std::move(pl);
   return "";
 }
 
@@ -942,24 +961,63 @@ void capture_plan(w2s_handle* h, Plan* pl) {
   pl->graph_failed = !ok;
 }
 
+// Profiled launch of one step (w2s_profile_enable): CUDA events around it, accumulated per launch class.
+std::string run_step(w2s_handle* h, const Step& st, cudaStream_t s) {
+  ProfRec rec;
+  if (h->profiling) {
+    rec.name = st.name;
+    rec.flops = st.flops;
+    rec.bytes = st.bytes;
+    cudaEventCreate(&rec.e0);
+    cudaEventCreate(&rec.e1);
+    cudaEventRecord(rec.e0, s);
+  }
+  std::string e = st.run(s);
+  if (h->profiling) {
+    cudaEventRecord(rec.e1, s);
+    h->prof.push_back(rec);
+  }
+  return e.empty() ? "" : st.name + ": " + e;
+}
+
 // One evaluation call: rows in tiles of max_batch (the last tile ragged), each tile = one DynArgs update + the plan.
+// With a background (zbits set and bg_B > 0) the call evaluates K * B rows, row g = (coalition g / B, background row
+// g % B), into the handle's per-row scratch, and bg_mean_kernel reduces each coalition's B rows into out[K, width].
 std::string run_batches(w2s_handle* h, const uint32_t* zbits, const float* x, long long ld, int64_t K, float* out,
                         cudaStream_t s) {
   const int64_t width = out_width(h, h->ws_L);
   if (width <= 0) return "no outputs selected (w2s_set_targets)";
   const bool graphs = h->use_graphs && !h->profiling;
-  for (int64_t k0 = 0; k0 < K; k0 += h->cfg.max_batch) {
-    const int n = (int)((K - k0) < h->cfg.max_batch ? (K - k0) : h->cfg.max_batch);
+  const bool bg = zbits && h->bg_B > 0;
+  const int64_t rows = bg ? K * h->bg_B : K;
+  float* dst = out;
+  if (bg) {
+    const long long need = rows * width;
+    if (h->bg_rows_cap < need) {
+      W2S_CUDA_OK(cudaStreamSynchronize(s));   // evaluations in flight may still write the old scratch
+      if (h->bg_rows) cudaFree(h->bg_rows);
+      h->bg_rows = nullptr;
+      h->bg_rows_cap = 0;
+      W2S_CUDA_OK(cudaMalloc((void**)&h->bg_rows, sizeof(float) * need));
+      h->bg_rows_cap = need;
+    }
+    dst = h->bg_rows;
+  }
+  for (int64_t k0 = 0; k0 < rows; k0 += h->cfg.max_batch) {
+    const int n = (int)((rows - k0) < h->cfg.max_batch ? (rows - k0) : h->cfg.max_batch);
     Plan* pl = nullptr;
-    W2S_TRY(get_plan(h, n, &pl));
+    W2S_TRY(get_plan(h, n, bg, &pl));
     DynArgs d{};
-    if (zbits) {
+    if (bg) {
+      d.clip = h->clip; d.seg_id = h->seg_id; d.zbits = zbits; d.zwords = h->zwords;
+      d.bg = h->bg; d.B = h->bg_B; d.ld = h->bg_L; d.row0 = k0;
+    } else if (zbits) {
       d.clip = h->clip; d.seg_id = h->seg_id; d.zbits = zbits + k0 * h->zwords; d.zwords = h->zwords;
       d.baseline = h->baseline;
     } else {
       d.x = x + k0 * ld; d.ld = ld;
     }
-    d.out = out + k0 * width;
+    d.out = dst + k0 * width;
     d.mode = h->mode; d.D = h->D; d.frames = h->frames; d.tokens = h->tokens;
     set_dyn_kernel<<<1, 1, 0, s>>>(h->dyn_dev, d);
     W2S_CUDA_OK(cudaGetLastError());
@@ -969,23 +1027,15 @@ std::string run_batches(w2s_handle* h, const uint32_t* zbits, const float* x, lo
       W2S_CUDA_OK(cudaGraphLaunch(pl->exec, s));
       continue;
     }
-    for (const Step& st : pl->steps) {
-      ProfRec rec;
-      if (h->profiling) {
-        rec.name = st.name;
-        rec.flops = st.flops;
-        rec.bytes = st.bytes;
-        cudaEventCreate(&rec.e0);
-        cudaEventCreate(&rec.e1);
-        cudaEventRecord(rec.e0, s);
-      }
-      std::string e = st.run(s);
-      if (h->profiling) {
-        cudaEventRecord(rec.e1, s);
-        h->prof.push_back(rec);
-      }
-      if (!e.empty()) return st.name + ": " + e;
-    }
+    for (const Step& st : pl->steps) W2S_TRY(run_step(h, st, s));
+  }
+  if (bg) {
+    const float *rows_in = h->bg_rows, *w = h->bg_w;
+    const int B = h->bg_B;
+    Step st{"bg_mean", [=](cudaStream_t st_s) { return launch_bg_mean(rows_in, w, B, K, width, out, st_s); }};
+    st.bytes = 4.0 * (double)K * width * (B + 1);
+    h->launches += 1;
+    W2S_TRY(run_step(h, st, s));
   }
   return "";
 }
@@ -1150,6 +1200,55 @@ int w2s_set_clip(w2s_handle* h, const float* x_dev, int64_t L, const int32_t* se
   return 0;
 }
 
+int w2s_set_background(w2s_handle* h, const float* bg_dev, int64_t B, int64_t L, int64_t ld, const double* weights_host,
+                       void* stream) {
+  cudaStream_t s = (cudaStream_t)stream;
+  if (B == 0) {
+    h->bg_B = 0;
+    h->bg_L = 0;
+    return 0;
+  }
+  if (B < 0 || B > W2S_MAX_BACKGROUND)
+    return fail(h, "set_background: B = " + std::to_string(B) + " rows; need 1 <= B <= " +
+                       std::to_string(W2S_MAX_BACKGROUND) + " (B = 0 clears the background)");
+  if (h->L <= 0) return fail(h, "set_background: no clip set (w2s_set_clip)");
+  if (L != h->L)
+    return fail(h, "set_background: background rows have " + std::to_string(L) + " samples, the clip has " +
+                       std::to_string(h->L));
+  if (ld < L) return fail(h, "set_background: row stride smaller than the row length");
+  if (!bg_dev || !weights_host) return fail(h, "set_background: null buffer");
+  double sum = 0.0;
+  for (int64_t b = 0; b < B; ++b) {
+    const double w = weights_host[b];
+    if (!std::isfinite(w) || w < 0.0)
+      return fail(h, "set_background: weight " + std::to_string(b) + " is " + std::to_string(w) +
+                         "; weights must be finite and >= 0");
+    sum += w;
+  }
+  if (!(sum > 0.0) || !std::isfinite(sum)) return fail(h, "set_background: the weights sum to zero");
+  // evaluations in flight on the stream still read the old rows and weights
+  if (cudaStreamSynchronize(s) != cudaSuccess) return fail(h, "set_background: stream error");
+  if (h->bg_cap < B * L) {
+    if (h->bg) cudaFree(h->bg);
+    h->bg = nullptr;
+    h->bg_cap = 0;
+    if (cudaMalloc((void**)&h->bg, sizeof(float) * B * L) != cudaSuccess) return fail(h, "set_background: out of device memory");
+    h->bg_cap = B * L;
+  }
+  if (!h->bg_w && cudaMalloc((void**)&h->bg_w, sizeof(float) * W2S_MAX_BACKGROUND) != cudaSuccess)
+    return fail(h, "set_background: out of device memory");
+  h->bg_w_host.resize((size_t)B);
+  for (int64_t b = 0; b < B; ++b) h->bg_w_host[(size_t)b] = (float)(weights_host[b] / sum);
+  if (cudaMemcpy2DAsync(h->bg, sizeof(float) * L, bg_dev, sizeof(float) * ld, sizeof(float) * L, (size_t)B,
+                        cudaMemcpyDeviceToDevice, s) != cudaSuccess ||
+      cudaMemcpyAsync(h->bg_w, h->bg_w_host.data(), sizeof(float) * B, cudaMemcpyHostToDevice, s) != cudaSuccess ||
+      cudaStreamSynchronize(s) != cudaSuccess)
+    return fail(h, std::string("set_background: copy failed: ") + cudaGetErrorString(cudaGetLastError()));
+  h->bg_B = (int)B;
+  h->bg_L = L;
+  return 0;
+}
+
 int w2s_set_targets(w2s_handle* h, const int32_t* frame_idx_host, const int32_t* token_idx_host, int D, int mode,
                     void* stream) {
   cudaStream_t s = (cudaStream_t)stream;
@@ -1195,6 +1294,9 @@ int w2s_eval(w2s_handle* h, const uint32_t* z_bits_dev, int64_t K, float* out_de
   if (h->L <= 0) return fail(h, "eval: no clip set (w2s_set_clip)");
   if (K == 0) return 0;   // empty coalition matrix: nothing to evaluate
   if (K < 0 || !z_bits_dev || !out_dev) return fail(h, "eval: null buffer");
+  if (h->bg_B > 0 && h->bg_L != h->L)
+    return fail(h, "eval: the background rows have " + std::to_string(h->bg_L) + " samples, the clip has " +
+                       std::to_string(h->L) + " (w2s_set_background again, or clear it with B = 0)");
   // the workspace (and with it T') follows the clip of THIS call: w2s_eval_waveforms may have left it at another length
   std::string e = ensure_workspace(h, h->L);
   if (e.empty()) e = check_targets(h);
@@ -1262,8 +1364,13 @@ int64_t w2s_grad_peek(w2s_handle* h, const char* name, void* dst_dev, int64_t ma
 
 int w2s_mask(w2s_handle* h, const uint32_t* z_bits_dev, int64_t K, float* out_dev, void* stream) {
   if (h->L <= 0) return fail(h, "mask: no clip set (w2s_set_clip)");
-  std::string e = launch_mask(h->clip, h->seg_id, z_bits_dev, h->zwords, K, h->L, h->baseline, out_dev, h->L,
-                              (cudaStream_t)stream);
+  if (h->bg_B > 0 && h->bg_L != h->L)
+    return fail(h, "mask: the background rows have " + std::to_string(h->bg_L) + " samples, the clip has " +
+                       std::to_string(h->L) + " (w2s_set_background again, or clear it with B = 0)");
+  std::string e = h->bg_B > 0 ? launch_mask_bg(h->clip, h->seg_id, z_bits_dev, h->zwords, K, h->L, h->bg, h->bg_B, h->bg_L,
+                                               out_dev, h->L, (cudaStream_t)stream)
+                              : launch_mask(h->clip, h->seg_id, z_bits_dev, h->zwords, K, h->L, h->baseline, out_dev, h->L,
+                                            (cudaStream_t)stream);
   return e.empty() ? 0 : fail(h, e);
 }
 

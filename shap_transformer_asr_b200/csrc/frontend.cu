@@ -8,29 +8,37 @@ namespace w2s {
 // K0  mask + baseline fill.  One thread = 4 consecutive samples (float4 store, 128 B per 8 lanes).
 // Follows feasability_tests/conformer_test.ipynb:138-141 (fill value) with keep-bit convention.
 // =================================================================================================
+// BG: global row g = row0 + blockIdx.y is coalition g / B filled from background row g % B (w2s_set_background)
+template <bool BG>
 __global__ void __launch_bounds__(256) mask_kernel(const float* __restrict__ x, const uint16_t* __restrict__ seg_id,
                                                     const uint32_t* __restrict__ zbits, int zwords, long long L,
-                                                    float baseline, float* __restrict__ out, long long ld) {
+                                                    float baseline, float* __restrict__ out, long long ld,
+                                                    const float* __restrict__ bg, int B, long long bg_ld, long long row0) {
   __shared__ uint32_t z[64];
-  const long long k = blockIdx.y;
+  const long long g = BG ? row0 + blockIdx.y : blockIdx.y;
+  const long long k = BG ? g / B : g;
   if (threadIdx.x < zwords) z[threadIdx.x] = zbits[k * zwords + threadIdx.x];
   __syncthreads();
   const long long i0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * 4;
   if (i0 >= L) return;
-  float* o = out + k * ld + i0;
-  if (i0 + 4 <= L && ((ld & 3) == 0)) {
+  float* o = out + g * ld + i0;
+  const float* f = BG ? bg + (g - k * B) * bg_ld : nullptr;
+  if (i0 + 4 <= L && ((ld & 3) == 0) && (!BG || (bg_ld & 3) == 0)) {
     const float4 xv = *reinterpret_cast<const float4*>(x + i0);
     const ushort4 sv = *reinterpret_cast<const ushort4*>(seg_id + i0);
+    float4 fv;
+    if constexpr (BG) fv = *reinterpret_cast<const float4*>(f + i0);
+    else fv = make_float4(baseline, baseline, baseline, baseline);
     float4 r;
-    r.x = (z[sv.x >> 5] >> (sv.x & 31)) & 1u ? xv.x : baseline;
-    r.y = (z[sv.y >> 5] >> (sv.y & 31)) & 1u ? xv.y : baseline;
-    r.z = (z[sv.z >> 5] >> (sv.z & 31)) & 1u ? xv.z : baseline;
-    r.w = (z[sv.w >> 5] >> (sv.w & 31)) & 1u ? xv.w : baseline;
+    r.x = (z[sv.x >> 5] >> (sv.x & 31)) & 1u ? xv.x : fv.x;
+    r.y = (z[sv.y >> 5] >> (sv.y & 31)) & 1u ? xv.y : fv.y;
+    r.z = (z[sv.z >> 5] >> (sv.z & 31)) & 1u ? xv.z : fv.z;
+    r.w = (z[sv.w >> 5] >> (sv.w & 31)) & 1u ? xv.w : fv.w;
     *reinterpret_cast<float4*>(o) = r;
   } else {
     for (int j = 0; j < 4 && i0 + j < L; ++j) {
       const uint32_t sgm = seg_id[i0 + j];
-      o[j] = (z[sgm >> 5] >> (sgm & 31)) & 1u ? x[i0 + j] : baseline;
+      o[j] = (z[sgm >> 5] >> (sgm & 31)) & 1u ? x[i0 + j] : (BG ? f[i0 + j] : baseline);
     }
   }
 }
@@ -40,29 +48,61 @@ std::string launch_mask(const float* x, const uint16_t* seg_id, const uint32_t* 
   if (zwords > 64) return "mask: more than 2048 segments are not supported";
   if (K == 0) return "";
   dim3 grid((unsigned)((L + 1023) / 1024), (unsigned)K);
-  W2S_CUDA_OK(launch_pdl(mask_kernel, grid, dim3(256), 0, s, 1, x, seg_id, zbits, zwords, L, baseline, out, ld));
+  W2S_CUDA_OK(launch_pdl(mask_kernel<false>, grid, dim3(256), 0, s, 1, x, seg_id, zbits, zwords, L, baseline, out, ld,
+                         (const float*)nullptr, 0, 0LL, 0LL));
   W2S_CUDA_OK(cudaGetLastError());
   return "";
 }
 
-// The same selection folded into a consumer's load: `zs` is the coalition's bit row staged in shared memory.
+std::string launch_mask_bg(const float* x, const uint16_t* seg_id, const uint32_t* zbits, int zwords, long long K,
+                           long long L, const float* bg, int B, long long bg_ld, float* out, long long ld, cudaStream_t s) {
+  if (zwords > 64) return "mask: more than 2048 segments are not supported";
+  const long long rows = K * B;
+  for (long long r0 = 0; r0 < rows; r0 += 65535) {   // grid.y limit
+    const long long n = rows - r0 < 65535 ? rows - r0 : 65535;
+    dim3 grid((unsigned)((L + 1023) / 1024), (unsigned)n);
+    W2S_CUDA_OK(launch_pdl(mask_kernel<true>, grid, dim3(256), 0, s, 1, x, seg_id, zbits, zwords, L, 0.f, out, ld, bg, B,
+                           bg_ld, r0));
+    W2S_CUDA_OK(cudaGetLastError());
+  }
+  return "";
+}
+
+// The same selection folded into a consumer's load: `zs` is the coalition's bit row staged in shared memory.  BG: dropped
+// samples come from a background row instead of the constant (a compile-time variant, so that the baseline-fill kernels
+// keep their code).
+template <bool BG = false>
 struct WaveRow {
   const float* x;
   const uint16_t* seg;   // null: plain waveform row
   const uint32_t* zs;
   float baseline;
+  const float* fill;     // BG: background row
   __device__ __forceinline__ float at(long long i) const {
     const float v = __ldg(x + i);
-    if (!seg) return v;
-    const uint32_t sgm = __ldg(seg + i);
-    return (zs[sgm >> 5] >> (sgm & 31)) & 1u ? v : baseline;
+    if constexpr (BG) {
+      const uint32_t sgm = __ldg(seg + i);
+      return (zs[sgm >> 5] >> (sgm & 31)) & 1u ? v : __ldg(fill + i);
+    } else {
+      if (!seg) return v;
+      const uint32_t sgm = __ldg(seg + i);
+      return (zs[sgm >> 5] >> (sgm & 31)) & 1u ? v : baseline;
+    }
   }
 };
-// Row `row` of the tile described by the per-call argument block; ends with a CTA-wide barrier.
-__device__ __forceinline__ WaveRow wave_row(const DynArgs* __restrict__ dyn, int row, uint32_t* zs) {
-  WaveRow w;
+// Row `row` of the tile described by the per-call argument block; ends with a CTA-wide barrier.  BG: tile row r is global
+// row g = row0 + r of the call, coalition g / B with background row g % B.
+template <bool BG = false>
+__device__ __forceinline__ WaveRow<BG> wave_row(const DynArgs* __restrict__ dyn, int row, uint32_t* zs) {
+  WaveRow<BG> w;
   w.zs = zs;
-  if (dyn->clip) {
+  if constexpr (BG) {
+    const long long g = dyn->row0 + row, B = dyn->B, k = g / B;
+    const int zw = dyn->zwords;
+    for (int i = threadIdx.x; i < zw; i += blockDim.x) zs[i] = dyn->zbits[k * zw + i];
+    w.x = dyn->clip; w.seg = dyn->seg_id; w.baseline = 0.f;
+    w.fill = dyn->bg + (g - k * B) * dyn->ld;
+  } else if (dyn->clip) {
     const int zw = dyn->zwords;
     for (int i = threadIdx.x; i < zw; i += blockDim.x) zs[i] = dyn->zbits[(long long)row * zw + i];
     w.x = dyn->clip; w.seg = dyn->seg_id; w.baseline = dyn->baseline;
@@ -89,7 +129,7 @@ __device__ __forceinline__ double warp_sum_f64(double v) {
   return v;
 }
 
-template <int KW>
+template <int KW, bool BG>
 __global__ void __launch_bounds__(256, 1) conv0_stats_kernel(const Conv0Params p) {
   constexpr int NR = KW * (KW + 1) / 2;
   constexpr int NACC = KW + NR;
@@ -97,7 +137,7 @@ __global__ void __launch_bounds__(256, 1) conv0_stats_kernel(const Conv0Params p
   __shared__ double tot[NACC];
   __shared__ uint32_t zs[64];
   const int row = blockIdx.x;
-  const WaveRow x = wave_row(p.dyn, row, zs);
+  const WaveRow<BG> x = wave_row<BG>(p.dyn, row, zs);
   double acc[NACC];
 #pragma unroll
   for (int i = 0; i < NACC; ++i) acc[i] = 0.0;
@@ -176,10 +216,11 @@ __global__ void __launch_bounds__(256, 1) conv0_stats_kernel(const Conv0Params p
   }
 }
 
-std::string launch_conv0_stats(const Conv0Params& p, cudaStream_t s) {
+std::string launch_conv0_stats(const Conv0Params& p, cudaStream_t s, bool bg) {
   if (p.kw != 10) return "conv0: only kernel width 10 is implemented for layer 0";
   if (p.n == 0) return "";
-  W2S_CUDA_OK(launch_pdl(conv0_stats_kernel<10>, dim3(p.n), dim3(256), 0, s, 1, p));
+  if (bg) W2S_CUDA_OK(launch_pdl(conv0_stats_kernel<10, true>, dim3(p.n), dim3(256), 0, s, 1, p));
+  else W2S_CUDA_OK(launch_pdl(conv0_stats_kernel<10, false>, dim3(p.n), dim3(256), 0, s, 1, p));
   W2S_CUDA_OK(cudaGetLastError());
   return "";
 }
@@ -191,7 +232,7 @@ std::string launch_conv0_stats(const Conv0Params& p, cudaStream_t s) {
 // affine constants in registers; all lanes of a warp work on the same frame, so window reads broadcast.
 // HF wav2vec2/modeling_wav2vec2.py:302-323 (group) / :275-299 (layer).
 // =================================================================================================
-template <int KW, bool LAYER>
+template <int KW, bool LAYER, bool BG>
 __global__ void __launch_bounds__(256, 2) conv0_kernel(const Conv0Params p, int FT) {
   extern __shared__ float sm[];
   float* xs = sm;                      // FT*stride + KW window
@@ -202,7 +243,7 @@ __global__ void __launch_bounds__(256, 2) conv0_kernel(const Conv0Params p, int 
   const int row = blockIdx.y;
   const int f0 = blockIdx.x * FT;
   const int nf = min(FT, p.T0 - f0);
-  const WaveRow x = wave_row(p.dyn, row, zs);
+  const WaveRow<BG> x = wave_row<BG>(p.dyn, row, zs);
   const long long x0 = (long long)f0 * p.stride;
   const int nwin = (nf - 1) * p.stride + KW;
   for (int i = threadIdx.x; i < nwin; i += blockDim.x) {
@@ -289,7 +330,7 @@ __global__ void __launch_bounds__(256, 2) conv0_kernel(const Conv0Params p, int 
 // conflict-free ldmatrix), each warp owns 64 channels whose B fragments stay in registers, and the channel
 // permutation inside a warp is chosen so that a thread ends up with 8 consecutive channels per (frame, half):
 // one 16-byte store, 64 contiguous bytes per quad.
-template <int KW, bool PRE>
+template <int KW, bool PRE, bool BG>
 __global__ void __launch_bounds__(256, 2) conv0_mma_kernel(const Conv0Params p, int FT) {
   extern __shared__ __align__(16) uint8_t im2col[];
   constexpr int LDA = 80;
@@ -299,7 +340,7 @@ __global__ void __launch_bounds__(256, 2) conv0_mma_kernel(const Conv0Params p, 
   const int f0 = blockIdx.x * FT;
   const int nf = min(FT, p.T0 - f0);
   const int nfp = (nf + 15) & ~15;
-  const WaveRow x = wave_row(p.dyn, row, zs);
+  const WaveRow<BG> x = wave_row<BG>(p.dyn, row, zs);
   const long long x0 = (long long)f0 * p.stride;
   for (int i = threadIdx.x; i < nfp * KW; i += blockDim.x) {
     const int f = i / KW, j = i - f * KW;
@@ -372,7 +413,7 @@ __global__ void __launch_bounds__(256, 2) conv0_mma_kernel(const Conv0Params p, 
 // window through the Gram matrix of the filter bank, as in the CUDA-core kernel this replaces.
 constexpr int C0L_K = 48, C0L_LDA = 112;   // 112-byte row pitch: 7 x 16 B, conflict-free ldmatrix
 
-template <int KW, bool PRE>
+template <int KW, bool PRE, bool BG>
 __global__ void __launch_bounds__(256, 2) conv0_ln_mma_kernel(const Conv0Params p, int FT) {
   extern __shared__ __align__(16) uint8_t smem_ln[];
   __shared__ uint32_t zs[64];
@@ -382,7 +423,7 @@ __global__ void __launch_bounds__(256, 2) conv0_ln_mma_kernel(const Conv0Params 
   const int f0 = blockIdx.x * FT;
   const int nf = min(FT, p.T0 - f0);
   const int nfp = (nf + 15) & ~15;
-  const WaveRow x = wave_row(p.dyn, row, zs);
+  const WaveRow<BG> x = wave_row<BG>(p.dyn, row, zs);
   const long long x0 = (long long)f0 * p.stride;
   const int nwin = (nf - 1) * p.stride + KW;
   for (int i = threadIdx.x; i < nwin; i += blockDim.x) xs[i] = x.at(x0 + i);
@@ -508,13 +549,13 @@ std::string launch_conv0_ln_b(const float* w, const float* bias, const float* ga
   return "";
 }
 
-std::string launch_conv0(const Conv0Params& p, bool layer_norm, cudaStream_t s) {
-  if (p.kw != 10) return "conv0: only kernel width 10 is implemented for layer 0";
+template <bool BG>
+std::string launch_conv0_t(const Conv0Params& p, bool layer_norm, cudaStream_t s) {
   if (!layer_norm && p.gn_wb && p.C % 64 == 0 && p.C <= 512 && p.n > 0) {
     const int FT = 512;
     dim3 grid((p.T0 + FT - 1) / FT, p.n);
-    if (p.pre_act) W2S_CUDA_OK(launch_pdl(conv0_mma_kernel<10, true>, grid, dim3(p.C / 2), (size_t)FT * 80, s, 1, p, FT));
-    else W2S_CUDA_OK(launch_pdl(conv0_mma_kernel<10, false>, grid, dim3(p.C / 2), (size_t)FT * 80, s, 1, p, FT));
+    if (p.pre_act) W2S_CUDA_OK(launch_pdl(conv0_mma_kernel<10, true, BG>, grid, dim3(p.C / 2), (size_t)FT * 80, s, 1, p, FT));
+    else W2S_CUDA_OK(launch_pdl(conv0_mma_kernel<10, false, BG>, grid, dim3(p.C / 2), (size_t)FT * 80, s, 1, p, FT));
     W2S_CUDA_OK(cudaGetLastError());
     return "";
   }
@@ -523,14 +564,14 @@ std::string launch_conv0(const Conv0Params& p, bool layer_norm, cudaStream_t s) 
     const size_t smem = (size_t)FT * C0L_LDA + (size_t)(FT * p.stride + p.kw + 4) * sizeof(float);
     static bool attr = false;
     if (!attr) {
-      W2S_CUDA_OK(cudaFuncSetAttribute(conv0_ln_mma_kernel<10, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-      W2S_CUDA_OK(cudaFuncSetAttribute(conv0_ln_mma_kernel<10, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
+      W2S_CUDA_OK(cudaFuncSetAttribute(conv0_ln_mma_kernel<10, false, BG>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
+      W2S_CUDA_OK(cudaFuncSetAttribute(conv0_ln_mma_kernel<10, true, BG>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
       attr = true;
     }
     if (smem > 100 * 1024) return "conv0 (layer norm): stride too large for the staged window";
     dim3 grid((p.T0 + FT - 1) / FT, p.n);
-    if (p.pre_act) W2S_CUDA_OK(launch_pdl(conv0_ln_mma_kernel<10, true>, grid, dim3(p.C / 2), smem, s, 1, p, FT));
-    else W2S_CUDA_OK(launch_pdl(conv0_ln_mma_kernel<10, false>, grid, dim3(p.C / 2), smem, s, 1, p, FT));
+    if (p.pre_act) W2S_CUDA_OK(launch_pdl(conv0_ln_mma_kernel<10, true, BG>, grid, dim3(p.C / 2), smem, s, 1, p, FT));
+    else W2S_CUDA_OK(launch_pdl(conv0_ln_mma_kernel<10, false, BG>, grid, dim3(p.C / 2), smem, s, 1, p, FT));
     W2S_CUDA_OK(cudaGetLastError());
     return "";
   }
@@ -540,10 +581,15 @@ std::string launch_conv0(const Conv0Params& p, bool layer_norm, cudaStream_t s) 
   const int FT = p.T0 >= 4096 ? 512 : 128;
   dim3 grid((p.T0 + FT - 1) / FT, p.n);
   const size_t smem = (size_t)(3 * (FT * p.stride + p.kw) + 2 * FT + 2) * sizeof(float);
-  if (layer_norm) W2S_CUDA_OK(launch_pdl(conv0_kernel<10, true>, grid, dim3(256), smem, s, 1, p, FT));
-  else W2S_CUDA_OK(launch_pdl(conv0_kernel<10, false>, grid, dim3(256), smem, s, 1, p, FT));
+  if (layer_norm) W2S_CUDA_OK(launch_pdl(conv0_kernel<10, true, BG>, grid, dim3(256), smem, s, 1, p, FT));
+  else W2S_CUDA_OK(launch_pdl(conv0_kernel<10, false, BG>, grid, dim3(256), smem, s, 1, p, FT));
   W2S_CUDA_OK(cudaGetLastError());
   return "";
+}
+
+std::string launch_conv0(const Conv0Params& p, bool layer_norm, cudaStream_t s, bool bg) {
+  if (p.kw != 10) return "conv0: only kernel width 10 is implemented for layer 0";
+  return bg ? launch_conv0_t<true>(p, layer_norm, s) : launch_conv0_t<false>(p, layer_norm, s);
 }
 
 // filter-bank statistics for the layer-norm variant: one CTA, trivially small

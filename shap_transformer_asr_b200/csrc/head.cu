@@ -53,6 +53,8 @@ __device__ __forceinline__ long long head_items(const DynArgs& d, int n, int T) 
 __global__ void __launch_bounds__(256) head_kernel(const HeadParams p) {
   extern __shared__ uint8_t smem[];
   const DynArgs d = *p.dyn;
+  // the pointers of the argument block are device allocations: keeps the stores and target loads global (LDG / STG)
+  __builtin_assume(__isGlobal(d.out) && __isGlobal(d.frames) && __isGlobal(d.tokens));
   const int ldw = p.H + 2;  // bf16 elements; (H+2)/2 odd -> conflict-free row stride
   __nv_bfloat16* ws = reinterpret_cast<__nv_bfloat16*>(smem);
   __nv_bfloat16* hs = ws + (size_t)p.V * ldw;  // 8 warps x H
@@ -123,6 +125,7 @@ __global__ void __launch_bounds__(256) head_kernel(const HeadParams p) {
 // second stage of the tensor-core head: logits[rows, ldl] (fp32, bias included) -> reduction; one warp per work item
 __global__ void __launch_bounds__(256) head_reduce_kernel(const float* __restrict__ logits, const HeadParams p) {
   const DynArgs d = *p.dyn;
+  __builtin_assume(__isGlobal(d.out) && __isGlobal(d.frames) && __isGlobal(d.tokens));   // as in head_kernel
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const bool targeted = (d.mode == W2S_OUT_LOGIT || d.mode == W2S_OUT_LOGPROB);
   const long long items = head_items(d, p.n, p.T);
@@ -192,6 +195,29 @@ std::string launch_head(const HeadParams& p, cudaStream_t s) {
   }
   if (smem > 200 * 1024) return "head: vocab * hidden too large for shared memory";
   head_kernel<<<head_grid(p, 148 * 4), 256, smem, s>>>(p);
+  W2S_CUDA_OK(cudaGetLastError());
+  return "";
+}
+
+// Background mean of a w2s_eval call with a background: the K * B per-row outputs (coalition-major) -> out[K, width].
+// One thread per (coalition, column); the terms are added in the documented order b = 0 .. B-1, one fmaf each from 0, so
+// the result does not depend on the batch tile or on how the coalitions are spread over GPUs.
+__global__ void __launch_bounds__(256) bg_mean_kernel(const float* __restrict__ rows, const float* __restrict__ w, int B,
+                                                      long long K, long long width, float* __restrict__ out) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= K * width) return;
+  const long long k = i / width, c = i - k * width;
+  const float* r = rows + k * B * width + c;
+  float acc = 0.f;
+  for (int b = 0; b < B; ++b) acc = fmaf(__ldg(w + b), __ldg(r + (long long)b * width), acc);
+  out[i] = acc;
+}
+
+std::string launch_bg_mean(const float* rows, const float* w, int B, long long K, long long width, float* out,
+                           cudaStream_t s) {
+  const long long n = K * width;
+  if (n == 0) return "";
+  bg_mean_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(rows, w, B, K, width, out);
   W2S_CUDA_OK(cudaGetLastError());
   return "";
 }

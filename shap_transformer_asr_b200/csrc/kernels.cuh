@@ -8,6 +8,9 @@ namespace w2s {
 // out[k, i] = bit(z[k], seg_id[i]) ? x[i] : baseline
 std::string launch_mask(const float* x, const uint16_t* seg_id, const uint32_t* zbits, int zwords, long long K,
                         long long L, float baseline, float* out, long long ld, cudaStream_t s);
+// the same with a background bg[B, bg_ld]: out[k * B + b, i] = bit(z[k], seg_id[i]) ? x[i] : bg[b, i]
+std::string launch_mask_bg(const float* x, const uint16_t* seg_id, const uint32_t* zbits, int zwords, long long K,
+                           long long L, const float* bg, int B, long long bg_ld, float* out, long long ld, cudaStream_t s);
 
 // ---- per-call arguments, read by the kernels from device memory ---------------------------------------------
 // Everything that may change between two evaluations of the same batch-tile plan lives here instead of in kernel
@@ -16,7 +19,7 @@ std::string launch_mask(const float* x, const uint16_t* seg_id, const uint32_t* 
 struct DynArgs {
   // input rows of this tile: explicit waveforms x[n, ld] (w2s_eval_waveforms) ...
   const float* x;
-  long long ld;
+  long long ld;             // row stride of x, or of bg when a background is set
   // ... or the masker folded into the consumer's load (w2s_eval): row r = keep-bit(zbits[r], seg_id[i]) ? clip[i] :
   // baseline, so the [n, L] masked waveforms are never materialised (conformer_test.ipynb:138-141 semantics)
   const float* clip;        // [L]; null selects `x`
@@ -29,6 +32,11 @@ struct DynArgs {
   int mode, D;
   const int* frames;        // [D] device
   const int* tokens;        // [D] device
+  // background fill (w2s_set_background; read only by the BG instantiations of the conv0 kernels): global row g =
+  // row0 + r of the call is coalition g / B filled from background row g % B, bg[b, i] = bg[b * ld + i]
+  const float* bg;
+  int B;
+  long long row0;
 };
 
 // ---- K1: conv0 (Cin = 1) + GroupNorm-over-time / LayerNorm-over-channels + GELU ------------------------
@@ -55,8 +63,9 @@ struct Conv0Params {
                                  // as bf16 hi/lo rows
   __nv_bfloat16* out;    // [n, T0, C] channels-last
 };
-std::string launch_conv0_stats(const Conv0Params& p, cudaStream_t s);         // group-norm statistics
-std::string launch_conv0(const Conv0Params& p, bool layer_norm, cudaStream_t s);
+// bg: the background-fill instantiations (DynArgs::bg); false selects the baseline-fill / explicit-waveform kernels
+std::string launch_conv0_stats(const Conv0Params& p, cudaStream_t s, bool bg = false);   // group-norm statistics
+std::string launch_conv0(const Conv0Params& p, bool layer_norm, cudaStream_t s, bool bg = false);
 // B operand of the tensor-core layer-norm variant (run once at create)
 std::string launch_conv0_ln_b(const float* w, const float* bias, const float* gamma, const float* beta, int C, int kw,
                               __nv_bfloat16* out, cudaStream_t s);
@@ -161,6 +170,9 @@ struct HeadParams {
 std::string launch_head(const HeadParams& p, cudaStream_t s);
 // tensor-core variant: the contraction kernel writes logits[n*T, ldl] (fp32, bias added), this reduces them
 std::string launch_head_reduce(const float* logits, const HeadParams& p, cudaStream_t s);
+// background mean: out[k, c] = sum_b w[b] * rows[k * B + b, c] (fp32, one fmaf per term from 0, b = 0 .. B-1)
+std::string launch_bg_mean(const float* rows, const float* w, int B, long long K, long long width, float* out,
+                           cudaStream_t s);
 
 // ---- K12: KernelSHAP constrained WLS -----------------------------------------------------------------------
 std::string launch_wls(const uint32_t* zbits, int zwords, const double* w, const float* y, long long K, int M,

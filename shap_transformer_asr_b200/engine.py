@@ -35,6 +35,31 @@ def _fold_pos_conv(sd: Dict[str, torch.Tensor], prefix: str) -> None:
         sd[p + "weight"] = v * (g / v.pow(2).sum(dim=(0, 1), keepdim=True).sqrt())
 
 
+def background_arrays(bg, weights=None, num_samples: Optional[int] = None):
+    """Validated background set: (rows float32 [B, L], weights float64 [B]).  ``bg`` is [B, L] (or one row [L]), numpy or
+    torch; ``weights`` default to uniform.  Raises ValueError naming the problem: no rows, more than
+    ``_lib.MAX_BACKGROUND``, a length other than ``num_samples``, or weights that are negative, not finite, of the wrong
+    count or summing to zero.  Host only (the rows stay where they are when ``bg`` is a tensor)."""
+    data = bg if isinstance(bg, torch.Tensor) else np.asarray(bg, dtype=np.float32)
+    if data.ndim == 1:
+        data = data[None]
+    if data.ndim != 2:
+        raise ValueError(f"background must be [B, L], got shape {tuple(data.shape)}")
+    B, L = data.shape
+    if B < 1 or B > _lib.MAX_BACKGROUND:
+        raise ValueError(f"background has {B} rows; need 1 <= B <= {_lib.MAX_BACKGROUND}")
+    if num_samples is not None and L != num_samples:
+        raise ValueError(f"background rows have {L} samples, the clip has {num_samples}")
+    w = np.ones(B, dtype=np.float64) if weights is None else np.ascontiguousarray(weights, dtype=np.float64).reshape(-1)
+    if w.shape != (B,):
+        raise ValueError(f"{w.size} background weights for {B} rows")
+    if not np.all(np.isfinite(w)) or np.any(w < 0):
+        raise ValueError("background weights must be finite and >= 0")
+    if not w.sum() > 0:
+        raise ValueError("background weights sum to zero")
+    return data, np.ascontiguousarray(w)
+
+
 class Engine:
     """B200 evaluation engine for one model.  ``model`` may be a ``transformers`` Wav2Vec2ForCTC /
     Wav2Vec2ConformerForCTC / WavLMForCTC instance (what the reference builds at shap_calculation.py:218-219) or a
@@ -113,6 +138,8 @@ class Engine:
         self.num_samples = 0
         self.num_segments = 0
         self.mode = "max"
+        self.background_rows = 0
+        self.background_weights = None
         del keep
 
     # -- lifetime ----------------------------------------------------------------------------------
@@ -151,6 +178,25 @@ class Engine:
                                           float(baseline), self._stream()), "w2s_set_clip")
         self.num_samples, self.num_segments = L, M
         self.bounds = bounds
+
+    def set_background(self, bg, weights=None):
+        """Background dataset of ``shap.KernelExplainer(f, data)``: ``bg`` [B, L] (numpy or torch, the clip's normalised
+        input space, L = the current clip's length) with ``weights`` [B] (default uniform; >= 0, positive sum).  Dropped
+        segments of coalition k are then filled from each background row in turn, and ``eval_bits`` returns the weighted
+        mean over the B rows (w2s_set_background).  The baseline of ``set_clip`` is ignored while a background is set."""
+        data, w = background_arrays(bg, weights, num_samples=self.num_samples or None)
+        bt = torch.as_tensor(data).to(device=self.device, dtype=torch.float32).contiguous()
+        B, L = bt.shape
+        self._check(self.lib.w2s_set_background(self._h, bt.data_ptr(), B, L, L, w.ctypes.data_as(C.POINTER(C.c_double)),
+                                                self._stream()), "w2s_set_background")
+        self.background_rows = B
+        self.background_weights = w / w.sum()
+
+    def clear_background(self):
+        """Back to the baseline fill of ``set_clip`` (bit-identical to never having set a background)."""
+        self._check(self.lib.w2s_set_background(self._h, None, 0, 0, 0, None, self._stream()), "w2s_set_background")
+        self.background_rows = 0
+        self.background_weights = None
 
     def set_targets(self, mode: str = "max", frames=None, tokens=None):
         mid = _lib.MODE_IDS[mode]
@@ -242,8 +288,9 @@ class Engine:
         return out
 
     def mask(self, zbits: torch.Tensor) -> torch.Tensor:
+        """The rows ``eval_bits`` evaluates: [K, L], or [K * B, L] (row k * B + b) with a background."""
         K = zbits.shape[0]
-        out = torch.empty((K, self.num_samples), dtype=torch.float32, device=self.device)
+        out = torch.empty((K * max(1, self.background_rows), self.num_samples), dtype=torch.float32, device=self.device)
         self._check(self.lib.w2s_mask(self._h, zbits.data_ptr(), K, out.data_ptr(), self._stream()), "w2s_mask")
         return out
 

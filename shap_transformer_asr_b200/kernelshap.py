@@ -19,6 +19,7 @@ import torch
 
 from . import _lib
 from . import dist as wdist
+from .engine import background_arrays
 from .targets import char_targets
 
 
@@ -169,14 +170,33 @@ class KernelShapExplainer:
         return frames, tokens, logits
 
     def explain(self, clip, num_segments: int, mode: str = "logprob", targets=None, baseline: float = 0.0,
-                check: bool = True):
-        """-> dict(phi[M, D] fp64 device, fx, fnull, frames, tokens, Z, weights, y, status, info).
+                check: bool = True, background=None, background_weights=None):
+        """-> dict(phi[M, D] fp64 device, fx, fnull, frames, tokens, Z, weights, y, status, info, background_weights).
 
         ``check`` reads the solve's status word back (one 4-byte D2H after the solve) and raises if the regression
         did not produce a usable answer; a rank-deficient design (status 2: fewer distinct coalitions than segments)
-        is solved for the minimum-norm attributions exactly as shap's ``lstsq`` fallback does and only warns."""
+        is solved for the minimum-norm attributions exactly as shap's ``lstsq`` fallback does and only warns.
+
+        ``background``: ``shap.KernelExplainer(f, data)``'s background set, an array [B, L] in the clip's normalised
+        input space, or the ``(data, weights)`` pair :func:`kmeans_background` returns; ``background_weights`` (default
+        uniform, or the pair's) weight its rows.  Every coalition (the empty and the full one included) is then
+        evaluated once per background row with the dropped segments taken from that row, and its output is the
+        weighted mean over the rows; ``baseline`` is not used.  The targets are selected on the clip itself.  With
+        ``background=None`` dropped segments are filled with ``baseline``; ``background_weights`` in the result is then
+        None, else the normalised float64 weights."""
         eng = self.engine
         eng.set_clip(clip, num_segments=num_segments, baseline=baseline)
+        bg = None
+        if background is not None:
+            if isinstance(background, tuple):
+                if background_weights is not None:
+                    raise ValueError("pass the weights either in the (data, weights) pair or as background_weights")
+                background, background_weights = background
+            bg = background_arrays(background, background_weights, num_samples=eng.num_samples)
+        elif background_weights is not None:
+            raise ValueError("background_weights given without a background")
+        if getattr(eng, "background_rows", 0):
+            eng.clear_background()
         M = eng.num_segments
         sampled = None
         if mode in ("max", "mean", "logits"):
@@ -199,6 +219,8 @@ class KernelShapExplainer:
             sampled = self._coalitions(M)
         words, kw, info = sampled["words"], sampled["kw"], sampled["info"]
         K = words.shape[0]
+        if bg is not None:
+            eng.set_background(*bg)
         # rows 0 / 1 of the evaluated matrix are the empty and the full coalition (fnull, fx): fx comes from the same
         # reduction kernel as every y row, so the efficiency constraint is consistent to the last bit
         rank, world = wdist.rank_world() if self.shard_coalitions else (0, 1)
@@ -212,6 +234,10 @@ class KernelShapExplainer:
         fnull = y_all[0].double()
         fx = y_all[1].double()
         phi, status = eng.wls(bits_all[2:], sampled["w_dev"], y_all[2:], fx, fnull, M)
+        bg_w = None
+        if bg is not None:
+            bg_w = eng.background_weights
+            eng.clear_background()      # the engine is left as it was found: baseline fill
         if check:
             st = int(status.item())
             if st == 1:
@@ -221,7 +247,33 @@ class KernelShapExplainer:
                 warnings.warn(f"KernelSHAP design is rank deficient ({K} coalitions for {M} segments): minimum-norm "
                               "attributions returned (shap's lstsq fallback)", RuntimeWarning)
         return dict(phi=phi, fx=fx, fnull=fnull, frames=frames, tokens=tokens, Z=unpack_coalitions(words, M), weights=kw,
-                    y=y_all[2:], status=status, info=info, words=words)
+                    y=y_all[2:], status=status, info=info, words=words, background_weights=bg_w)
+
+
+def kmeans_background(X, k: int, round_values: bool = True):
+    """``shap.kmeans(X, k, round_values)`` restated (from memory of shap's ``utils/_legacy.py``; shap is not installed, so
+    parity with shap itself is unpinned): ``sklearn.cluster.KMeans(n_clusters=k, random_state=0)`` over the rows of
+    ``X`` [n, L]; with ``round_values`` every centre coordinate is replaced by the nearest value its column takes in
+    ``X``; the weights are the cluster sizes.  -> (data float32 [k, L], weights float64 [k]), the pair
+    ``KernelShapExplainer.explain(background=...)`` accepts."""
+    from sklearn.cluster import KMeans
+
+    X = np.asarray(X, dtype=np.float64)
+    if X.ndim != 2:
+        raise ValueError(f"X must be [n, L], got shape {X.shape}")
+    k = int(k)
+    if k < 1 or k > X.shape[0]:
+        raise ValueError(f"k = {k} clusters for {X.shape[0]} rows")
+    km = KMeans(n_clusters=k, random_state=0).fit(X)
+    centres = km.cluster_centers_.copy()
+    if round_values:
+        cols = np.arange(X.shape[1])
+        for j0 in range(0, X.shape[1], 4096):     # [k, n, 4096] distances per chunk of columns
+            c = cols[j0:j0 + 4096]
+            nearest = np.abs(centres[:, None, c] - X[None, :, c]).argmin(axis=1)     # [k, chunk]: row index
+            centres[:, c] = X[nearest, c[None, :]]
+    weights = np.bincount(km.labels_, minlength=k).astype(np.float64)
+    return centres.astype(np.float32), weights
 
 
 def expand_to_samples(phi: np.ndarray, bounds: np.ndarray, per_sample: bool = False) -> np.ndarray:

@@ -40,7 +40,7 @@ def make_test_set(num_clips: int = 2, num_samples: int = 102400, snrs=(5, 2, 1),
 
 
 def explain_test_set(engine, test_set: List[Dict], out_dir: str = "data", num_segments: int = 128, nsamples=2048,
-                     seed: int = 0, mode: str = "max", save_limit=None, on_item=None) -> List[Dict]:
+                     seed: int = 0, mode: str = "max", save_limit=None, on_item=None, background=None) -> List[Dict]:
     """Explain every item and write ``{shap_values,audio,noise,text}_sample_{i}_{type}_{snr}.npy``
     (shap_calculation.py:200-210).  ``mode="max"`` explains the max logit of every output frame, which is what the
     reference's wrapper returns (shap_calculation.py:50), so the saved array has the reference's ``[1, L, T']`` shape.
@@ -49,7 +49,11 @@ def explain_test_set(engine, test_set: List[Dict], out_dir: str = "data", num_se
     Every item is explained on THIS rank's GPU (clip-level sharding: the caller hands each rank its items).
     ``save_limit``: write the files of the first N items only (a 6.4 s item is 130 MB of float32 attributions);
     ``on_item(index, item, phi, bounds, result)`` is called for every item, saved or not, with the segment-level
-    attributions ``phi [M, T']`` (the ``[1, L, T']`` expansion is only materialised for the items that are written)."""
+    attributions ``phi [M, T']`` (the ``[1, L, T']`` expansion is only materialised for the items that are written).
+    ``background``: passed to every ``KernelShapExplainer.explain`` call -- an array [B, L] or a ``(data, weights)`` pair,
+    e.g. the reference's noise background ``make_background(L, 5, seed)`` (shap_calculation.py:125-127) -- so the
+    KernelSHAP attributions are taken against the same background as the expected-gradients ones; None fills the dropped
+    segments with zeros."""
     os.makedirs(out_dir, exist_ok=True)
     explainer = KernelShapExplainer(engine, nsamples=nsamples, seed=seed, shard_coalitions=False)
     results, clean_text = [], None
@@ -65,7 +69,8 @@ def explain_test_set(engine, test_set: List[Dict], out_dir: str = "data", num_se
         text = item["text"] if item["text"] is not None else clean_text
         T = logits.shape[0]
         targets = None if mode == "max" else (np.arange(T, dtype=np.int32), logits.argmax(-1).astype(np.int32))
-        res = explainer.explain(x, num_segments=num_segments, mode=mode, targets=targets if mode != "max" else ((), ()))
+        res = explainer.explain(x, num_segments=num_segments, mode=mode, targets=targets if mode != "max" else ((), ()),
+                                background=background)
         phi = res["phi"].cpu().numpy()
         tag = f"sample_{i + 1}_{item['type']}_{item['snr']}"
         saved = save_limit is None or i < save_limit

@@ -19,7 +19,8 @@ import torch
 import torch.distributed as td
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from shap_transformer_asr_b200 import MODELS, Engine, dist as wdist, eta_raw_segments, explain_test_set, make_test_set, wer
+from shap_transformer_asr_b200 import (MODELS, Engine, dist as wdist, eta_raw_segments, explain_test_set, make_background,
+                                       make_test_set, wer)
 from shap_transformer_asr_b200.modelzoo import build_random_init_model
 
 
@@ -33,6 +34,8 @@ def main():
     ap.add_argument("--model", default="wav2vec2-base")
     ap.add_argument("--save-limit", type=int, default=-1, help="write the four .npy files of the first N items per rank "
                     "only (a 6.4 s item is 130 MB of attributions); -1 = all, as the reference does")
+    ap.add_argument("--background", type=int, default=0, help="explain against the reference's noise background "
+                    "(make_background: N rows of 0.01 * randn, shap_calculation.py:125-127) instead of zero fill; 0 = zero fill")
     args = ap.parse_args()
     rank, world = wdist.init_from_env("cuda") if int(os.environ.get("WORLD_SIZE", "1")) > 1 else (0, 1)
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -55,7 +58,8 @@ def main():
 
     explain_test_set(eng, [test_set[i] for i in mine], out_dir=os.path.join(args.out, f"rank{rank}"),
                      num_segments=args.segments, nsamples=args.coalitions, seed=0,
-                     save_limit=None if args.save_limit < 0 else args.save_limit, on_item=consume)
+                     save_limit=None if args.save_limit < 0 else args.save_limit, on_item=consume,
+                     background=make_background(args.samples, args.background, seed=0) if args.background > 0 else None)
     torch.cuda.synchronize()
     dt = time.perf_counter() - t0
     gathered = [None] * world
