@@ -33,7 +33,8 @@ enum {
   W2S_OUT_LOGIT   = 1, /* logits[:, t_d, tok_d]          -> [n, D]   feasability_tests/w2v2conformer.py:40-42 */
   W2S_OUT_LOGPROB = 2, /* log_softmax(logits)[t_d,tok_d] -> [n, D]   north-star per-character CTC output      */
   W2S_OUT_MEAN    = 3, /* mean over vocab and time       -> [n, 1]   lime_shap_wav2vec2_comparison.py:68-70   */
-  W2S_OUT_LOGITS  = 4  /* raw logits                     -> [n, T', V]  (target selection, parity tests)      */
+  W2S_OUT_LOGITS  = 4, /* raw logits                     -> [n, T', V]  (target selection, parity tests)      */
+  W2S_OUT_CTC     = 5  /* log p_CTC(y_d | all frames)     -> [n, D]   set by w2s_set_transcripts only            */
 };
 
 /* w2s_config.flags */
@@ -116,6 +117,22 @@ int w2s_set_background(w2s_handle* h, const float* bg_dev, int64_t B, int64_t L,
 int w2s_set_targets(w2s_handle* h, const int32_t* frame_idx_host, const int32_t* token_idx_host, int D,
                     int mode, void* stream);
 
+/* Transcript-level output W2S_OUT_CTC: D >= 1 label sequences y_d = labels[offsets[d] .. offsets[d + 1]) (host arrays,
+ * offsets[0] = 0, non-decreasing, 0 <= U_d <= W2S_MAX_TRANSCRIPT; every label in [0, V) and != blank; blank in [0, V), the
+ * model's pad_token_id).  Row r then reports out[r, d] = log p_CTC(y_d | logits of row r over all T' frames) in natural
+ * log: the log of the sum over all alignments of y_d to the T' frames, i.e. -WavXForCTC(x, labels=y_d).loss with
+ * ctc_loss_reduction = "sum".  The empty transcript gives sum_t log_softmax(z_t)[blank].  Transcript d needs U_d + (number
+ * of adjacent equal labels) frames: w2s_eval / w2s_eval_waveforms fail before any launch when the clip of the call has
+ * fewer, naming the transcript, so no accepted transcript yields -inf or NaN.  Each value is one fixed sequence of fp32
+ * operations on that row's logits (log-domain forward recursion, one warp per (row, transcript)): bit-identical for any
+ * batch tile, position in the tile, number of GPUs and across calls.  With a background the usual weighted mean applies.
+ * Everything but the clip length is validated before the device is touched; the upload is ordered on `stream` as in
+ * w2s_set_targets.  The transcripts stay stored when w2s_set_targets later selects another mode (w2s_grad_transcripts
+ * uses them). */
+#define W2S_MAX_TRANSCRIPT 512
+int w2s_set_transcripts(w2s_handle* h, const int32_t* labels_host, const int32_t* offsets_host, int D, int blank,
+                        void* stream);
+
 /* Number of fp32 values one evaluated row produces under the current mode for clips of L samples. */
 int64_t w2s_out_width(const w2s_handle* h, int64_t num_samples);
 
@@ -146,6 +163,14 @@ int w2s_grad_waveforms(w2s_handle* h, const float* x_dev, int64_t n, int64_t L, 
  * reference's shap.GradientExplainer(wrapped_model, ...) runs unmodified on callbacks.ModelWrapper. */
 int w2s_vjp_waveforms(w2s_handle* h, const float* x_dev, int64_t n, int64_t L, int64_t ld, const float* gout_dev,
                       float* grad_dev, float* out_dev, void* stream);
+/* The same backward pass for the transcript-level output: out[r] = log p_CTC(y_{which[r]} | x_r) (see
+ * w2s_set_transcripts) and grad[r, :] = d out[r] / d x[r, :].  which[n] (host) indexes the transcripts last set.  The seed
+ * d log p / d logits[t, v] = gamma_t(v) - softmax(logits_t)_v, with gamma the CTC state occupation from the log-domain
+ * alpha / beta recursions, reaches every frame.  Refused before any launch: no transcripts set, an index out of range,
+ * a transcript infeasible for the clip, w2s_grad_rules on (DeepLIFT on transcripts is not built), and every model the
+ * gradient path refuses (WavLMForCTC included).  out may be NULL. */
+int w2s_grad_transcripts(w2s_handle* h, const float* x_dev, int64_t n, int64_t L, int64_t ld, const int32_t* which_host,
+                         float* grad_dev, float* out_dev, void* stream);
 /* Test hooks of the gradient path.  `on` bit 0: keep snapshots of the gradient after every encoder layer / conv layer
  * ("layer<l>", "h0", "conv<l>", "convu<l>", forward activations "f.*"); bit 1: run attention backward on the CUDA-core
  * cross-check kernels, bit 2: as batched tensor-core contractions + row kernels, instead of the fused tcgen05 kernel.  w2s_grad_peek copies a snapshot out (returns bytes copied, 0 = unknown name, < 0 = buffer
@@ -220,6 +245,13 @@ int w2s_debug_attention_bias(int use_tcgen05, const void* qkv, const float* rel_
  * the stream. */
 int w2s_debug_attention_bwd(int use_tcgen05, const void* qkv, const void* ctx, const void* dctx, const float* lse, int B,
                             int T, int heads, float scale, void* dqkv, void* stream);
+/* The CTC code of W2S_OUT_CTC on caller logits [n, T, ldl] (fp32, device; V <= ldl used): out[n, D] (device) =
+ * log p_CTC(y_d | logits[r]) through the head reduction kernel.  With dlogits [n, T, V] (device, may be NULL), also the
+ * gradient seed of w2s_grad_transcripts: dlogits[r] = d out[r, which[r]] / d logits[r].  labels / offsets [D + 1] / which [n]
+ * are host arrays, validated as in w2s_set_transcripts plus feasibility for T.  The call synchronises the stream.  Errors via
+ * w2s_last_error(NULL). */
+int w2s_debug_ctc(const float* logits, int n, int T, int V, int ldl, const int32_t* labels_host, const int32_t* offsets_host,
+                  int D, int blank, const int32_t* which_host, float* out_dev, float* dlogits_dev, void* stream);
 /* Per-launch CUDA-event profile on the launching stream (bench.py roofline leg): enable, run evaluations,
  * then read per launch class (newline-separated names) total milliseconds, algorithmic FLOPs / bytes and
  * launch counts.  Returns the number of classes, or -1 if `names_cap` is too small. */

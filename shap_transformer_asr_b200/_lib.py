@@ -14,10 +14,11 @@ LIB_PATH = os.path.join(_HERE, "libw2s.so")
 
 MAX_CONV_LAYERS = 8
 
-OUT_MAX, OUT_LOGIT, OUT_LOGPROB, OUT_MEAN, OUT_LOGITS = 0, 1, 2, 3, 4
+OUT_MAX, OUT_LOGIT, OUT_LOGPROB, OUT_MEAN, OUT_LOGITS, OUT_CTC = 0, 1, 2, 3, 4, 5
 MODE_IDS = {"max": OUT_MAX, "logit": OUT_LOGIT, "logprob": OUT_LOGPROB, "mean": OUT_MEAN, "logits": OUT_LOGITS}
 FLAG_VALIDATE_GEMM, FLAG_VALIDATE_ATTN, FLAG_FP32_PRELN, FLAG_NO_GRAPH = 1, 2, 4, 16
 MAX_BACKGROUND = 256      # W2S_MAX_BACKGROUND: rows of a background set
+MAX_TRANSCRIPT = 512      # W2S_MAX_TRANSCRIPT: labels of one transcript (OUT_CTC, set by w2s_set_transcripts only)
 
 
 class W2SConfig(C.Structure):
@@ -62,6 +63,8 @@ SIGNATURES = {
                                      C.c_void_p]),
     "w2s_set_targets": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int, C.c_int,
                                   C.c_void_p]),
+    "w2s_set_transcripts": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int, C.c_int,
+                                      C.c_void_p]),
     "w2s_out_width": (C.c_int64, [C.c_void_p, C.c_int64]),
     "w2s_eval": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "w2s_eval_waveforms": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
@@ -70,6 +73,8 @@ SIGNATURES = {
                                      C.c_void_p, C.c_void_p, C.c_void_p]),
     "w2s_vjp_waveforms": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p,
                                     C.c_void_p, C.c_void_p]),
+    "w2s_grad_transcripts": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.POINTER(C.c_int32),
+                                       C.c_void_p, C.c_void_p, C.c_void_p]),
     "w2s_grad_debug": (C.c_int, [C.c_void_p, C.c_int]),
     "w2s_grad_rules": (C.c_int, [C.c_void_p, C.c_int]),
     "w2s_grad_peek": (C.c_int64, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_int64, C.c_void_p]),
@@ -87,6 +92,8 @@ SIGNATURES = {
                                            C.c_void_p, C.c_void_p, C.c_void_p]),
     "w2s_debug_attention_bwd": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                           C.c_float, C.c_void_p, C.c_void_p]),
+    "w2s_debug_ctc": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
+                                C.c_int, C.c_int, C.POINTER(C.c_int32), C.c_void_p, C.c_void_p, C.c_void_p]),
     "w2s_profile_enable": (C.c_int, [C.c_void_p, C.c_int]),
     "w2s_profile_read": (C.c_int64, [C.c_void_p, C.c_char_p, C.c_int64, C.POINTER(C.c_double), C.POINTER(C.c_double),
                                      C.POINTER(C.c_double), C.POINTER(C.c_int64), C.c_int64]),

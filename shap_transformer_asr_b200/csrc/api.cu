@@ -4,6 +4,7 @@
 #include "../../include/w2s.h"
 #include "gemm.cuh"
 #include "kernels.cuh"
+#include "ctc.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -137,6 +138,15 @@ struct w2s_handle {
   int targets_cap = 0;
   std::vector<int32_t> targets_host;   // staging of the last w2s_set_targets arrays (source of the async upload)
 
+  // transcripts (w2s_set_transcripts): kept across w2s_set_targets, so the gradient entry can use them in any mode
+  int ctc_D = 0, ctc_blank = 0, ctc_smax = 1;   // count, blank id, largest 2U + 1
+  int *ctc_labels = nullptr, *ctc_offsets = nullptr;
+  int ctc_labels_cap = 0, ctc_offsets_cap = 0;
+  std::vector<int32_t> ctc_host;        // staging of the upload: offsets [D + 1], then the labels
+  std::vector<int> ctc_need;            // frames each transcript needs
+  float *ctc_alpha = nullptr, *ctc_lse = nullptr, *ctc_dz = nullptr;   // gradient-seed scratch, grown on demand
+  long long ctc_alpha_cap = 0, ctc_lse_cap = 0, ctc_dz_cap = 0;
+
   // workspace (sized for max_batch rows of the current clip length)
   long long ws_L = -1;
   int T = 0, Tp = 0;
@@ -182,6 +192,7 @@ struct w2s_handle {
   unsigned grad_frames_next = 0;
   float *grad_out = nullptr, *grad_out_val = nullptr;
   const float* grad_gout = nullptr;
+  bool grad_ctc = false;              // w2s_grad_transcripts: the head_bwd step seeds from the CTC log-likelihood
 
   // per-call arguments of the plan's kernels (kernels.cuh: DynArgs), rewritten before every tile
   DynArgs* dyn_dev = nullptr;
@@ -210,6 +221,8 @@ struct w2s_handle {
     if (bg_rows) cudaFree(bg_rows);
     if (frames) cudaFree(frames);
     if (tokens) cudaFree(tokens);
+    for (void* p : {(void*)ctc_labels, (void*)ctc_offsets, (void*)ctc_alpha, (void*)ctc_lse, (void*)ctc_dz})
+      if (p) cudaFree(p);
     if (wls_work) cudaFree(wls_work);
     for (void* p : ws_allocs) cudaFree(p);
     for (void* p : allocs) cudaFree(p);
@@ -932,6 +945,7 @@ int64_t out_width(const w2s_handle* h, int64_t L) {
     case W2S_OUT_MAX: return T;
     case W2S_OUT_MEAN: return 1;
     case W2S_OUT_LOGITS: return T * h->cfg.vocab_size;
+    case W2S_OUT_CTC: return h->ctc_D;
     default: return h->D;
   }
 }
@@ -1018,7 +1032,8 @@ std::string run_batches(w2s_handle* h, const uint32_t* zbits, const float* x, lo
       d.x = x + k0 * ld; d.ld = ld;
     }
     d.out = dst + k0 * width;
-    d.mode = h->mode; d.D = h->D; d.frames = h->frames; d.tokens = h->tokens;
+    d.mode = h->mode; d.D = h->mode == W2S_OUT_CTC ? h->ctc_D : h->D; d.frames = h->frames; d.tokens = h->tokens;
+    d.ctc_labels = h->ctc_labels; d.ctc_offsets = h->ctc_offsets; d.blank = h->ctc_blank;
     set_dyn_kernel<<<1, 1, 0, s>>>(h->dyn_dev, d);
     W2S_CUDA_OK(cudaGetLastError());
     h->launches += 1 + (long long)pl->steps.size();
@@ -1040,11 +1055,47 @@ std::string run_batches(w2s_handle* h, const uint32_t* zbits, const float* x, lo
   return "";
 }
 
+// the first transcript that needs more frames than T, as an error
+std::string check_transcripts(const w2s_handle* h, int64_t T) {
+  if (h->ctc_D <= 0) return "no transcripts set (w2s_set_transcripts)";
+  for (int d = 0; d < h->ctc_D; ++d)
+    if (h->ctc_need[d] > T)
+      return "transcript " + std::to_string(d) + " needs " + std::to_string(h->ctc_need[d]) + " frames, the clip has " +
+             std::to_string(T);
+  return "";
+}
+
 std::string check_targets(const w2s_handle* h) {
+  if (h->mode == W2S_OUT_CTC) return check_transcripts(h, h->T);
   if (h->mode == W2S_OUT_LOGIT || h->mode == W2S_OUT_LOGPROB) {
     if (h->D <= 0 || !h->frames || !h->tokens) return "targets not set (w2s_set_targets)";
     if (h->max_frame >= h->T)
       return "target frame " + std::to_string(h->max_frame) + " beyond the clip's " + std::to_string(h->T) + " frames";
+  }
+  return "";
+}
+
+// w2s_set_transcripts / w2s_debug_ctc argument checks (host only); fills need[d] with the frames transcript d needs
+std::string validate_transcripts(const int32_t* labels, const int32_t* offsets, int D, int blank, int V,
+                                 std::vector<int>* need) {
+  if (D < 1 || !offsets) return "need D >= 1 transcripts and their offsets";
+  if (blank < 0 || blank >= V) return "blank " + std::to_string(blank) + " outside the vocabulary [0, " + std::to_string(V) + ")";
+  if (offsets[0] != 0) return "offsets[0] must be 0";
+  need->assign((size_t)D, 0);
+  for (int d = 0; d < D; ++d) {
+    const int U = offsets[d + 1] - offsets[d];
+    if (U < 0) return "offsets must be non-decreasing (transcript " + std::to_string(d) + ")";
+    if (U > W2S_MAX_TRANSCRIPT)
+      return "transcript " + std::to_string(d) + " has " + std::to_string(U) + " labels, at most " +
+             std::to_string(W2S_MAX_TRANSCRIPT) + " are supported";
+    if (U > 0 && !labels) return "labels missing";
+    for (int u = offsets[d]; u < offsets[d + 1]; ++u) {
+      if (labels[u] < 0 || labels[u] >= V)
+        return "transcript " + std::to_string(d) + ": label " + std::to_string(labels[u]) + " outside the vocabulary [0, " +
+               std::to_string(V) + ")";
+      if (labels[u] == blank) return "transcript " + std::to_string(d) + ": label equal to the blank " + std::to_string(blank);
+    }
+    (*need)[(size_t)d] = ctc_frames_needed(labels + offsets[d], U);
   }
   return "";
 }
@@ -1288,6 +1339,54 @@ int w2s_set_targets(w2s_handle* h, const int32_t* frame_idx_host, const int32_t*
   return 0;
 }
 
+int w2s_set_transcripts(w2s_handle* h, const int32_t* labels_host, const int32_t* offsets_host, int D, int blank,
+                        void* stream) {
+  cudaStream_t s = (cudaStream_t)stream;
+  std::vector<int> need;
+  const std::string e = validate_transcripts(labels_host, offsets_host, D, blank, h->cfg.vocab_size, &need);
+  if (!e.empty()) return fail(h, "set_transcripts: " + e);
+  const int total = offsets_host[D];
+  const int label_slots = total > 0 ? total : 1;   // all transcripts empty: the kernels still take a valid pointer
+  if (h->ctc_offsets_cap < D + 1 || h->ctc_labels_cap < label_slots) {
+    // evaluations in flight on the stream still read the old arrays
+    if (cudaStreamSynchronize(s) != cudaSuccess) return fail(h, "set_transcripts: stream error");
+    h->ctc_D = 0;   // the old arrays go now: a failed allocation below leaves no transcripts set, not dangling ones
+    if (h->ctc_offsets_cap < D + 1) {
+      if (h->ctc_offsets) cudaFree(h->ctc_offsets);
+      h->ctc_offsets = nullptr;
+      h->ctc_offsets_cap = 0;
+      const int cap = D + 1 < 64 ? 64 : D + 1;
+      if (cudaMalloc((void**)&h->ctc_offsets, sizeof(int) * cap) != cudaSuccess) return fail(h, "set_transcripts: out of device memory");
+      h->ctc_offsets_cap = cap;
+    }
+    if (h->ctc_labels_cap < label_slots) {
+      if (h->ctc_labels) cudaFree(h->ctc_labels);
+      h->ctc_labels = nullptr;
+      h->ctc_labels_cap = 0;
+      const int cap = total < 1024 ? 1024 : total;
+      if (cudaMalloc((void**)&h->ctc_labels, sizeof(int) * cap) != cudaSuccess) return fail(h, "set_transcripts: out of device memory");
+      h->ctc_labels_cap = cap;
+    }
+  }
+  // ordered on the caller's stream, staged in the handle (as w2s_set_targets)
+  h->ctc_host.assign(offsets_host, offsets_host + D + 1);
+  h->ctc_host.insert(h->ctc_host.end(), labels_host, labels_host + total);
+  if (cudaMemcpyAsync(h->ctc_offsets, h->ctc_host.data(), sizeof(int) * (D + 1), cudaMemcpyHostToDevice, s) != cudaSuccess ||
+      (total > 0 && cudaMemcpyAsync(h->ctc_labels, h->ctc_host.data() + D + 1, sizeof(int) * total, cudaMemcpyHostToDevice,
+                                    s) != cudaSuccess))
+    return fail(h, "set_transcripts: copy failed");
+  h->ctc_D = D;
+  h->ctc_blank = blank;
+  h->ctc_need = need;
+  h->ctc_smax = 1;
+  for (int d = 0; d < D; ++d) {
+    const int S = 2 * (offsets_host[d + 1] - offsets_host[d]) + 1;
+    h->ctc_smax = S > h->ctc_smax ? S : h->ctc_smax;
+  }
+  h->mode = W2S_OUT_CTC;
+  return 0;
+}
+
 int64_t w2s_out_width(const w2s_handle* h, int64_t num_samples) { return out_width(h, num_samples); }
 
 int w2s_eval(w2s_handle* h, const uint32_t* z_bits_dev, int64_t K, float* out_dev, void* stream) {
@@ -1322,6 +1421,28 @@ int w2s_grad_waveforms(w2s_handle* h, const float* x_dev, int64_t n, int64_t L, 
   if (ld < L) return fail(h, "grad_waveforms: row stride smaller than the row length");
   std::string e = run_grad(h, x_dev, ld, L, n, frames_host, nullptr, grad_dev, out_dev, (cudaStream_t)stream);
   return e.empty() ? 0 : fail(h, "grad_waveforms: " + e);
+}
+
+int w2s_grad_transcripts(w2s_handle* h, const float* x_dev, int64_t n, int64_t L, int64_t ld, const int32_t* which_host,
+                         float* grad_dev, float* out_dev, void* stream) {
+  if (n == 0) return 0;
+  if (n < 0 || !x_dev || !which_host || !grad_dev) return fail(h, "grad_transcripts: null buffer");
+  if (ld < L) return fail(h, "grad_transcripts: row stride smaller than the row length");
+  std::string e = grad_supported(h);
+  if (e.empty() && h->grad_rules) e = "DeepLIFT rules (w2s_grad_rules) are not built for transcripts: switch them off";
+  const int64_t T = num_frames(h->cfg, L, nullptr);
+  if (e.empty() && T <= 0) e = "clip shorter than the conv receptive field";
+  if (e.empty()) e = h->ctc_D > 0 ? "" : "no transcripts set (w2s_set_transcripts)";
+  for (int64_t i = 0; e.empty() && i < n; ++i)
+    if (which_host[i] < 0 || which_host[i] >= h->ctc_D)
+      e = "transcript index " + std::to_string(which_host[i]) + " outside the " + std::to_string(h->ctc_D) + " set";
+  if (e.empty()) e = check_transcripts(h, T);
+  if (e.empty()) {
+    h->grad_ctc = true;
+    e = run_grad(h, x_dev, ld, L, n, which_host, nullptr, grad_dev, out_dev, (cudaStream_t)stream);
+    h->grad_ctc = false;
+  }
+  return e.empty() ? 0 : fail(h, "grad_transcripts: " + e);
 }
 
 int w2s_vjp_waveforms(w2s_handle* h, const float* x_dev, int64_t n, int64_t L, int64_t ld, const float* gout_dev,
@@ -1515,6 +1636,68 @@ int w2s_debug_attention_bwd(int use_tcgen05, const void* qkv, const void* ctx, c
   if (se != cudaSuccess && e.empty()) e = std::string("debug_attention_bwd: ") + cudaGetErrorString(se);
   for (float* p : {delta, dq, stats})
     if (p) cudaFree(p);
+  if (!e.empty()) {
+    g_create_error = e;
+    return 1;
+  }
+  return 0;
+}
+
+int w2s_debug_ctc(const float* logits, int n, int T, int V, int ldl, const int32_t* labels_host, const int32_t* offsets_host,
+                  int D, int blank, const int32_t* which_host, float* out_dev, float* dlogits_dev, void* stream) {
+  g_create_error.clear();
+  const cudaStream_t s = (cudaStream_t)stream;
+  std::vector<int> need;
+  std::string e;
+  if (n <= 0 || T <= 0 || V <= 0 || V > 128 || ldl < V || !logits || !out_dev)
+    e = "debug_ctc: need n, T >= 1, 1 <= V <= 128, ldl >= V and logits / out buffers";
+  if (e.empty()) e = validate_transcripts(labels_host, offsets_host, D, blank, V, &need);
+  if (!e.empty() && e.compare(0, 10, "debug_ctc:") != 0) e = "debug_ctc: " + e;
+  for (int d = 0; e.empty() && d < D; ++d)
+    if (need[d] > T) e = "debug_ctc: transcript " + std::to_string(d) + " needs " + std::to_string(need[d]) + " frames, T = " + std::to_string(T);
+  for (int r = 0; e.empty() && dlogits_dev && r < n; ++r)
+    if (!which_host || which_host[r] < 0 || which_host[r] >= D) e = "debug_ctc: which[r] must index a transcript";
+  if (e.empty() && n * (long long)D > 0) {
+    const int total = offsets_host[D];
+    int smax = 1;
+    for (int d = 0; d < D; ++d) smax = std::max(smax, 2 * (offsets_host[d + 1] - offsets_host[d]) + 1);
+    int *lab = nullptr, *off = nullptr, *wh = nullptr;
+    DynArgs* dyn = nullptr;
+    float *alpha = nullptr, *lse = nullptr, *val = nullptr;
+    auto al = [&](void** p, size_t bytes) {
+      if (e.empty() && cudaMalloc(p, bytes) != cudaSuccess) e = "debug_ctc: out of device memory";
+    };
+    al((void**)&lab, sizeof(int) * (total + 1));
+    al((void**)&off, sizeof(int) * (D + 1));
+    al((void**)&wh, sizeof(int) * n);
+    al((void**)&dyn, sizeof(DynArgs));
+    DynArgs d{};
+    d.out = out_dev; d.mode = W2S_OUT_CTC; d.D = D; d.ctc_labels = lab; d.ctc_offsets = off; d.blank = blank;
+    if (e.empty() && (cudaMemcpyAsync(off, offsets_host, sizeof(int) * (D + 1), cudaMemcpyHostToDevice, s) != cudaSuccess ||
+                      (total && cudaMemcpyAsync(lab, labels_host, sizeof(int) * total, cudaMemcpyHostToDevice, s) != cudaSuccess) ||
+                      cudaMemcpyAsync(dyn, &d, sizeof(DynArgs), cudaMemcpyHostToDevice, s) != cudaSuccess))
+      e = "debug_ctc: copy failed";
+    if (e.empty()) {
+      HeadParams hp{};
+      hp.n = n; hp.T = T; hp.V = V; hp.ldl = ldl; hp.dyn = dyn;
+      e = launch_head_reduce(logits, hp, s);
+    }
+    if (e.empty() && dlogits_dev) {
+      al((void**)&alpha, sizeof(float) * (size_t)n * T * smax);
+      al((void**)&lse, sizeof(float) * (size_t)n * T);
+      al((void**)&val, sizeof(float) * (size_t)n);
+      if (e.empty() && cudaMemcpyAsync(wh, which_host, sizeof(int) * n, cudaMemcpyHostToDevice, s) != cudaSuccess)
+        e = "debug_ctc: copy failed";
+      if (e.empty())
+        e = launch_ctc_seed(logits, ldl, V, nullptr, n, T, 0, lab, off, wh, blank, smax, alpha, lse, dlogits_dev, V, nullptr,
+                            val, s);
+    }
+    // the buffers live for this call only
+    const cudaError_t se = cudaStreamSynchronize(s);
+    if (se != cudaSuccess && e.empty()) e = std::string("debug_ctc: ") + cudaGetErrorString(se);
+    for (void* p : {(void*)lab, (void*)off, (void*)wh, (void*)dyn, (void*)alpha, (void*)lse, (void*)val})
+      if (p) cudaFree(p);
+  }
   if (!e.empty()) {
     g_create_error = e;
     return 1;

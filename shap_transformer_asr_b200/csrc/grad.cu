@@ -9,6 +9,7 @@
 // Conventions: activations saved by the forward pass are bf16 unless stated; gradients between contractions are bf16
 // (they feed a tensor-core A operand), gradients that are accumulated across a residual branch are fp32.
 #include "kernels.cuh"
+#include "ctc.cuh"
 
 namespace w2s {
 
@@ -328,6 +329,128 @@ std::string launch_head_vjp(const float* logits, int ldl, int V, const __nv_bflo
   if (blocks > 148 * 8) blocks = 148 * 8;
   head_vjp_kernel<<<(unsigned)blocks, 256, 0, s>>>(logits, ldl, V, w_head, items, H, gout, dh, out_all);
   W2S_CUDA_OK(cudaGetLastError());
+  return "";
+}
+
+// Start of the backward pass for the transcript-level output W2S_OUT_CTC (ctc.cuh), one warp per row r: the forward
+// recursion stores alpha_t(s) and lse_t; the backward one carries beta_t(s) = log of the paths from (t, s) to the end,
+// emissions after t only.  At every frame the state occupation q_s = exp(alpha_t(s) + beta_t(s) - log p) is summed per
+// vocabulary entry -- blank over the even states, label v over the positions u with y_u = v in ascending u (a per-label
+// list built once) -- so no atomics and a fixed order: gamma_t(v).  dz[r, t, v] = gamma_t(v) - softmax(z_t)_v.
+__global__ void __launch_bounds__(32) ctc_grad_kernel(const float* __restrict__ logits, int ldl, int V, int T,
+                                                      const int* __restrict__ labels, const int* __restrict__ offsets,
+                                                      const int* __restrict__ which, int blank, int s_max,
+                                                      float* __restrict__ alpha_all, float* __restrict__ lse_all,
+                                                      float* __restrict__ dz, int ldz, float* __restrict__ out_val) {
+  extern __shared__ float ctc_smem[];
+  float* alpha = ctc_smem;                 // [s_max] working row of the forward recursion
+  float* beta = alpha + s_max;             // [s_max]
+  float* q = beta + s_max;                 // [s_max] occupation, then beta + emission
+  int* pos = reinterpret_cast<int*>(q + s_max);   // [CTC_MAX_U] label positions grouped by label
+  int* start = pos + CTC_MAX_U;            // [V + 1]
+  int* cur = start + V + 1;                // [V] fill cursors
+  const int b = blockIdx.x, lane = threadIdx.x;
+  const int d = which[b];
+  const int* lab = labels + offsets[d];
+  const int U = offsets[d + 1] - offsets[d], S = 2 * U + 1;
+  const int k = (S + 31) >> 5, s0 = lane * k, s1 = min(S, s0 + k);
+  const float* rows = logits + (long long)b * T * ldl;
+  float* alpha_row = alpha_all + (long long)b * T * s_max;
+  float* lse = lse_all + (long long)b * T;
+  const float logp = ctc_forward_warp<4>(T, V, lab, U, blank, lane, alpha,
+                                         [&](int t, float(&lg)[4]) -> const float* {
+                                           const float* row = rows + (long long)t * ldl;
+#pragma unroll
+                                           for (int j = 0; j < 4; ++j) lg[j] = lane + 32 * j < V ? row[lane + 32 * j] : -INFINITY;
+                                           return row;
+                                         },
+                                         alpha_row, lse);
+  if (lane == 0) {
+    if (out_val) out_val[b] = logp;
+    for (int v = 0; v <= V; ++v) start[v] = 0;
+    for (int u = 0; u < U; ++u) ++start[lab[u] + 1];
+    for (int v = 0; v < V; ++v) start[v + 1] += start[v];
+    for (int v = 0; v < V; ++v) cur[v] = start[v];
+    for (int u = 0; u < U; ++u) pos[cur[lab[u]]++] = u;
+  }
+  __syncwarp();
+  for (int s = s0; s < s1; ++s) beta[s] = s >= S - 2 ? 0.f : -INFINITY;
+  __syncwarp();
+  for (int t = T - 1; t >= 0; --t) {
+    const float* z = rows + (long long)t * ldl;
+    const float* a = alpha_row + (long long)t * S;
+    const float lt = lse[t];
+    // occupation normalised per frame: sum_s q_s = 1 exactly in exact arithmetic (every path passes through one state
+    // at t), so dividing by the computed sum instead of exp(log p) removes the rounding that alpha_t + beta_t and log p
+    // accumulate in common over the frames (a nats-scale error of log p at |log p| ~ 1e4 would otherwise scale every q)
+    float m = -INFINITY;
+    for (int s = s0; s < s1; ++s) m = fmaxf(m, a[s] + beta[s]);   // -inf when either is; never (-inf) - (-inf)
+    m = warp_max(m);
+    float zs = 0.f;
+    for (int s = s0; s < s1; ++s) {
+      const float e = a[s] + beta[s];
+      const float o = e == -INFINITY ? 0.f : expf(e - m);
+      q[s] = o;
+      zs += o;
+    }
+    const float inv = 1.f / warp_sum(zs);
+    float gb = 0.f;
+    for (int s = s0; s < s1; ++s) {
+      q[s] *= inv;
+      if (!(s & 1)) gb += q[s];
+    }
+    gb = warp_sum(gb);
+    __syncwarp();
+    for (int v = lane; v < V; v += 32) {
+      float g = 0.f;
+      if (v == blank) {
+        g = gb;
+      } else {
+        for (int i = start[v]; i < start[v + 1]; ++i) g += q[2 * pos[i] + 1];
+      }
+      dz[((long long)b * T + t) * ldz + v] = g - expf(z[v] - lt);
+    }
+    __syncwarp();
+    if (t == 0) break;
+    // beta_{t-1}(s) = logsumexp over s' in {s, s + 1, s + 2 (skip)} of beta_t(s') + y_t(s')
+    for (int s = s0; s < s1; ++s)
+      q[s] = beta[s] == -INFINITY ? -INFINITY : beta[s] + (z[ctc_label(lab, blank, s)] - lt);
+    __syncwarp();
+    for (int s = s0; s < s1; ++s) {
+      const float w1 = s + 1 < S ? q[s + 1] : -INFINITY;
+      const float w2 = s + 2 < S && ctc_skip(lab, s + 2) ? q[s + 2] : -INFINITY;
+      beta[s] = ctc_lae3(q[s], w1, w2);
+    }
+    __syncwarp();
+  }
+}
+
+// dh[r, t, :] = dz[r, t, :] W_head (W_head [V, H] bf16): one block per (row, frame), the V terms added in order
+__global__ void __launch_bounds__(256) ctc_seed_dh_kernel(const float* __restrict__ dz, int ldz, int V,
+                                                          const __nv_bfloat16* __restrict__ w_head, int H, float* __restrict__ dh) {
+  __shared__ float g[128];
+  const long long rt = blockIdx.x;
+  for (int v = threadIdx.x; v < V; v += blockDim.x) g[v] = dz[rt * ldz + v];
+  __syncthreads();
+  for (int c = threadIdx.x; c < H; c += blockDim.x) {
+    float acc = 0.f;
+    for (int v = 0; v < V; ++v) acc = fmaf(g[v], __bfloat162float(w_head[(long long)v * H + c]), acc);
+    dh[rt * H + c] = acc;
+  }
+}
+
+std::string launch_ctc_seed(const float* logits, int ldl, int V, const __nv_bfloat16* w_head, int n, int T, int H,
+                            const int* labels, const int* offsets, const int* which, int blank, int s_max, float* alpha,
+                            float* lse, float* dz, int ldz, float* dh, float* out_val, cudaStream_t s) {
+  if (n == 0) return "";
+  if (V > 128) return "ctc: vocab_size > 128 not supported";
+  const size_t smem = sizeof(float) * 3 * (size_t)s_max + sizeof(int) * (CTC_MAX_U + 2 * V + 1);
+  ctc_grad_kernel<<<n, 32, smem, s>>>(logits, ldl, V, T, labels, offsets, which, blank, s_max, alpha, lse, dz, ldz, out_val);
+  W2S_CUDA_OK(cudaGetLastError());
+  if (dh) {
+    ctc_seed_dh_kernel<<<(unsigned)((long long)n * T), 256, 0, s>>>(dz, ldz, V, w_head, H, dh);
+    W2S_CUDA_OK(cudaGetLastError());
+  }
   return "";
 }
 

@@ -704,8 +704,12 @@ struct GradBuilder {
       const int* fr = plan->frames;
       float* seed = (stable || conf) ? dT : dA;
       // per-row target frame (w2s_grad_waveforms), or an upstream gradient over all frames (w2s_vjp_waveforms)
+      // or the transcript log-likelihood of w2s_grad_transcripts, whose frame slots carry the transcript indices
       add("head_bwd", [=](cudaStream_t s) {
         if (hh->grad_gout) return launch_head_vjp(lg, ldl, V, hw, nn, T, H, hh->grad_gout, seed, hh->grad_out_val, s);
+        if (hh->grad_ctc)
+          return launch_ctc_seed(lg, ldl, V, hw, nn, T, H, hh->ctc_labels, hh->ctc_offsets, fr, hh->ctc_blank, hh->ctc_smax,
+                                 hh->ctc_alpha, hh->ctc_lse, hh->ctc_dz, ldl, seed, hh->grad_out_val, s);
         return launch_head_bwd(lg, ldl, V, hw, nn, T, H, fr, seed, hh->grad_out_val, s, active_rows);
       });
       if (stable || conf) {   // final encoder LayerNorm: dA = d (residual stream after the last layer)
@@ -973,8 +977,24 @@ std::string run_grad(w2s_handle* h, const float* x, long long ld, long long L, i
   W2S_TRY(grad_prepare_weights(h));
   const int64_t T = num_frames(h->cfg, L, nullptr);
   if (T <= 0) return "clip shorter than the conv receptive field";
+  if (h->grad_ctc) {   // transcript indices, checked by w2s_grad_transcripts; seed scratch for one tile
+    const long long tile_rows = n < h->grad_tile ? n : h->grad_tile;
+    auto grow = [&](float** p, long long* cap, long long need) -> std::string {
+      if (*cap >= need) return "";
+      W2S_CUDA_OK(cudaStreamSynchronize(s));   // earlier calls may still use the old scratch
+      if (*p) cudaFree(*p);
+      *p = nullptr;
+      *cap = 0;
+      W2S_CUDA_OK(cudaMalloc((void**)p, sizeof(float) * need));
+      *cap = need;
+      return "";
+    };
+    W2S_TRY(grow(&h->ctc_alpha, &h->ctc_alpha_cap, tile_rows * T * h->ctc_smax));
+    W2S_TRY(grow(&h->ctc_lse, &h->ctc_lse_cap, tile_rows * T));
+    W2S_TRY(grow(&h->ctc_dz, &h->ctc_dz_cap, tile_rows * T * h->head_ldl));
+  }
   if (frames_host) {
-    for (int64_t i = 0; i < n; ++i)
+    for (int64_t i = 0; i < n && !h->grad_ctc; ++i)
       if (frames_host[i] < 0 || frames_host[i] >= T)
         return "target frame " + std::to_string(frames_host[i]) + " outside the clip's " + std::to_string(T) + " frames";
     if (!h->grad_frames_pinned) {
@@ -1021,7 +1041,7 @@ std::string run_grad(w2s_handle* h, const float* x, long long ld, long long L, i
       }
       if (!e.empty()) return st.name + ": " + e;
     }
-    h->launches += (long long)pl->steps.size() + 1;
+    h->launches += (long long)pl->steps.size() + 1 + (h->grad_ctc ? 1 : 0);   // the CTC seed step launches two kernels
   }
   return "";
 }

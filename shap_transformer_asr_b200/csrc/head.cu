@@ -3,9 +3,11 @@
 //   logit at (frame, token)        feasability_tests/w2v2conformer.py:40-42
 //   log-softmax at (frame, token)  north-star per-character CTC log-probability
 //   mean over vocab and time       feasability_tests/lime_shap_wav2vec2_comparison.py:68-70
+//   CTC log-likelihood of a transcript over all frames (ctc.cuh), -Wav2Vec2ForCTC(x, labels=y).loss
 // One warp per (row, frame) work item: lane = vocabulary entry, so log-softmax and gather are warp
 // shuffles (HF wav2vec2/modeling_wav2vec2.py:1705-1708 for the linear layer).
 #include "kernels.cuh"
+#include "ctc.cuh"
 #include "../../include/w2s.h"
 
 namespace w2s {
@@ -41,10 +43,10 @@ __device__ __forceinline__ void head_reduce_frame(const float (&logit)[HEAD_MAXJ
   if (lane == 0) *dst = sel;
 }
 
-// Work items per mode: MAX / LOGITS one per (row, frame); LOGIT / LOGPROB one per (row, target); MEAN one per row
-// (the warp walks the frames in order, so the sum is bit-reproducible -- no atomics).
+// Work items per mode: MAX / LOGITS one per (row, frame); LOGIT / LOGPROB one per (row, target); CTC one per (row,
+// transcript); MEAN one per row (the warp walks the frames in order, so the sum is bit-reproducible -- no atomics).
 __device__ __forceinline__ long long head_items(const DynArgs& d, int n, int T) {
-  if (d.mode == W2S_OUT_LOGIT || d.mode == W2S_OUT_LOGPROB) return (long long)n * d.D;
+  if (d.mode == W2S_OUT_LOGIT || d.mode == W2S_OUT_LOGPROB || d.mode == W2S_OUT_CTC) return (long long)n * d.D;
   if (d.mode == W2S_OUT_MEAN) return n;
   return (long long)n * T;
 }
@@ -58,6 +60,7 @@ __global__ void __launch_bounds__(256) head_kernel(const HeadParams p) {
   const int ldw = p.H + 2;  // bf16 elements; (H+2)/2 odd -> conflict-free row stride
   __nv_bfloat16* ws = reinterpret_cast<__nv_bfloat16*>(smem);
   __nv_bfloat16* hs = ws + (size_t)p.V * ldw;  // 8 warps x H
+  float* ctc_alpha = reinterpret_cast<float*>(hs + 8 * (size_t)p.H);   // 8 warps x CTC_MAX_S, then 8 warps x 128 logits
   for (int i = threadIdx.x; i < p.V * p.H; i += blockDim.x) {
     const int v = i / p.H, k = i - v * p.H;
     ws[v * ldw + k] = p.w[i];
@@ -93,6 +96,22 @@ __global__ void __launch_bounds__(256) head_kernel(const HeadParams p) {
   };
   for (long long it = (long long)blockIdx.x * 8 + warp; it < items; it += (long long)gridDim.x * 8) {
     float logit[HEAD_MAXJ];
+    if (d.mode == W2S_OUT_CTC) {
+      const int b = (int)(it / d.D), dd = (int)(it - (long long)b * d.D);
+      float* zs = ctc_alpha + 8 * CTC_MAX_S + warp * 32 * HEAD_MAXJ;   // the frame's logits, indexed by vocabulary id
+      const float r = ctc_forward_warp<HEAD_MAXJ>(
+          p.T, p.V, d.ctc_labels + d.ctc_offsets[dd], d.ctc_offsets[dd + 1] - d.ctc_offsets[dd], d.blank, lane,
+          ctc_alpha + warp * CTC_MAX_S, [&](int t, float(&lg)[HEAD_MAXJ]) -> const float* {
+            frame_logits(b, t, lg);
+#pragma unroll
+            for (int j = 0; j < HEAD_MAXJ; ++j)
+              if (lane + 32 * j < p.V) zs[lane + 32 * j] = lg[j];
+            __syncwarp();
+            return zs;
+          });
+      if (lane == 0) d.out[(long long)b * d.D + dd] = r;
+      continue;
+    }
     if (d.mode == W2S_OUT_MEAN) {
       float sm = 0.f;
       for (int t = 0; t < p.T; ++t) {
@@ -122,8 +141,11 @@ __global__ void __launch_bounds__(256) head_kernel(const HeadParams p) {
   }
 }
 
-// second stage of the tensor-core head: logits[rows, ldl] (fp32, bias included) -> reduction; one warp per work item
-__global__ void __launch_bounds__(256) head_reduce_kernel(const float* __restrict__ logits, const HeadParams p) {
+// second stage of the tensor-core head: logits[rows, ldl] (fp32, bias included) -> reduction; one warp per work item.
+// Six blocks per SM, as before the CTC branch was added: its alpha rows take 32.8 KB of shared memory per block, and the
+// bound keeps the register count of every mode at 40.
+__global__ void __launch_bounds__(256, 6) head_reduce_kernel(const float* __restrict__ logits, const HeadParams p) {
+  __shared__ float ctc_alpha[8][CTC_MAX_S];
   const DynArgs d = *p.dyn;
   __builtin_assume(__isGlobal(d.out) && __isGlobal(d.frames) && __isGlobal(d.tokens));   // as in head_kernel
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -132,6 +154,20 @@ __global__ void __launch_bounds__(256) head_reduce_kernel(const float* __restric
   const int per = targeted ? d.D : p.T;
   for (long long it = (long long)blockIdx.x * 8 + warp; it < items; it += (long long)gridDim.x * 8) {
     float logit[HEAD_MAXJ];
+    if (d.mode == W2S_OUT_CTC) {
+      const int b = (int)(it / d.D), dd = (int)(it - (long long)b * d.D);
+      const float* rows = logits + (long long)b * p.T * p.ldl;
+      const float r = ctc_forward_warp<HEAD_MAXJ>(
+          p.T, p.V, d.ctc_labels + d.ctc_offsets[dd], d.ctc_offsets[dd + 1] - d.ctc_offsets[dd], d.blank, lane,
+          ctc_alpha[warp], [&](int t, float(&lg)[HEAD_MAXJ]) -> const float* {
+            const float* row = rows + (long long)t * p.ldl;
+#pragma unroll
+            for (int j = 0; j < HEAD_MAXJ; ++j) lg[j] = lane + 32 * j < p.V ? row[lane + 32 * j] : -INFINITY;
+            return row;
+          });
+      if (lane == 0) d.out[(long long)b * d.D + dd] = r;
+      continue;
+    }
     if (d.mode == W2S_OUT_MEAN) {
       const float* row = logits + it * p.T * p.ldl;
       float sm = 0.f;
@@ -188,7 +224,9 @@ std::string launch_head(const HeadParams& p, cudaStream_t s) {
   if (p.V > 32 * HEAD_MAXJ) return "head: vocab_size > 128 not supported";
   if (p.H % 2) return "head: hidden size must be even";
   if (p.n == 0) return "";
-  const size_t smem = ((size_t)p.V * (p.H + 2) + 8 * (size_t)p.H) * sizeof(__nv_bfloat16);
+  // weights and hidden rows (bf16), then the CTC scratch of every warp: alpha and one frame of logits (fp32)
+  const size_t smem = ((size_t)p.V * (p.H + 2) + 8 * (size_t)p.H) * sizeof(__nv_bfloat16) +
+                      8 * (size_t)(CTC_MAX_S + 32 * HEAD_MAXJ) * sizeof(float);
   if (!g_head_attr) {
     W2S_CUDA_OK(cudaFuncSetAttribute(head_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     g_head_attr = true;

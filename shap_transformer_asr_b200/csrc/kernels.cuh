@@ -37,6 +37,11 @@ struct DynArgs {
   const float* bg;
   int B;
   long long row0;
+  // CTC transcripts (w2s_set_transcripts; mode W2S_OUT_CTC, D transcripts): transcript d is ctc_labels[ctc_offsets[d] ..
+  // ctc_offsets[d + 1]), with blank id `blank`
+  const int* ctc_labels;
+  const int* ctc_offsets;   // [D + 1]
+  int blank;
 };
 
 // ---- K1: conv0 (Cin = 1) + GroupNorm-over-time / LayerNorm-over-channels + GELU ------------------------
@@ -193,6 +198,12 @@ std::string launch_conv0_ln_bwd(const __nv_bfloat16* du, const __nv_bfloat16* u,
                                 long long ld, cudaStream_t s);
 std::string launch_head_bwd(const float* logits, int ldl, int V, const __nv_bfloat16* w_head, int n, int T, int H,
                             const int* frames, float* dh, float* out_val, cudaStream_t s, int active = -1);
+// CTC seed (ctc.cuh) of w2s_grad_transcripts: for row r and transcript which[r], out_val[r] = log p and
+// dz[r, t, v] = d log p / d logits[r, t, v] (row stride ldz), then, when dh is given, dh[r, t, :] = dz[r, t, :] W_head.
+// alpha: scratch [n, T, s_max] with s_max >= 2 U + 1 of every transcript used, lse: scratch [n, T]
+std::string launch_ctc_seed(const float* logits, int ldl, int V, const __nv_bfloat16* w_head, int n, int T, int H,
+                            const int* labels, const int* offsets, const int* which, int blank, int s_max, float* alpha,
+                            float* lse, float* dz, int ldz, float* dh, float* out_val, cudaStream_t s);
 std::string launch_head_vjp(const float* logits, int ldl, int V, const __nv_bfloat16* w_head, int n, int T, int H,
                             const float* gout, float* dh, float* out_all, cudaStream_t s);
 std::string launch_attn_bwd(const __nv_bfloat16* qkv, const __nv_bfloat16* dctx, int B, int T, int H, int heads, float scale,

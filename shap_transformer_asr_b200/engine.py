@@ -14,6 +14,7 @@ import torch
 from . import _lib
 from .config import ModelConfig
 from .preprocess import pack_coalitions, segment_bounds
+from .targets import PAD_ID, check_offsets, transcript_arrays
 
 
 # ModelConfig.kind -> w2s_config.kind and the HF state_dict prefix of the encoder
@@ -212,6 +213,24 @@ class Engine:
         self._check(rc, "w2s_set_targets")
         self.mode = mode
 
+    def set_transcripts(self, transcripts, blank: int = PAD_ID, offsets=None):
+        """Transcript-level output (w2s_set_transcripts): ``transcripts`` is a list of D label-id sequences (or, with
+        ``offsets`` [D + 1], one flat label array).  Each evaluated row then yields D values, out[r, d] = log p_CTC(y_d |
+        row r) = -WavXForCTC(x, labels=y_d).loss with ctc_loss_reduction="sum".  ``blank`` is the model's pad_token_id.
+        Arguments are validated on the host before the library is called."""
+        if offsets is not None:
+            labels = np.ascontiguousarray(np.asarray(transcripts).reshape(-1), dtype=np.int32)
+            offsets = check_offsets(offsets, labels.size)
+            transcript_arrays([labels[a:b] for a, b in zip(offsets[:-1], offsets[1:])], blank, self.config.vocab_size)
+        else:
+            labels, offsets = transcript_arrays(transcripts, blank, self.config.vocab_size)
+        self._check(self.lib.w2s_set_transcripts(self._h, labels.ctypes.data_as(C.POINTER(C.c_int32)),
+                                                 offsets.ctypes.data_as(C.POINTER(C.c_int32)), len(offsets) - 1, int(blank),
+                                                 self._stream()), "w2s_set_transcripts")
+        self.mode = "transcript"
+        self.transcripts = [labels[a:b].copy() for a, b in zip(offsets[:-1], offsets[1:])]
+        self.blank = int(blank)
+
     def out_width(self, num_samples: Optional[int] = None) -> int:
         return int(self.lib.w2s_out_width(self._h, int(num_samples or self.num_samples)))
 
@@ -251,6 +270,20 @@ class Engine:
         self._check(self.lib.w2s_grad_waveforms(self._h, x.data_ptr(), n, L, x.stride(0),
                                                 f.ctypes.data_as(C.POINTER(C.c_int32)), grad.data_ptr(), out.data_ptr(),
                                                 self._stream()), "w2s_grad_waveforms")
+        return grad, out
+
+    def grad_transcripts(self, x: torch.Tensor, which):
+        """x: float32 device tensor [n, L]; which: one transcript index per row (of the last ``set_transcripts``) ->
+        (grad [n, L], out [n]) with out[r] = log p_CTC(y_which[r] | x[r]) and grad[r] = d out[r] / d x[r]."""
+        if x.dim() != 2 or x.stride(1) != 1 or x.dtype != torch.float32 or not x.is_cuda:
+            raise ValueError("expected a float32 CUDA tensor [n, L] with contiguous rows")
+        n, L = x.shape
+        w = np.ascontiguousarray(np.broadcast_to(np.asarray(which, dtype=np.int32), (n,)))
+        grad = torch.empty((n, L), dtype=torch.float32, device=self.device)
+        out = torch.empty((n,), dtype=torch.float32, device=self.device)
+        self._check(self.lib.w2s_grad_transcripts(self._h, x.data_ptr(), n, L, x.stride(0),
+                                                  w.ctypes.data_as(C.POINTER(C.c_int32)), grad.data_ptr(), out.data_ptr(),
+                                                  self._stream()), "w2s_grad_transcripts")
         return grad, out
 
     def vjp_waveforms(self, x: torch.Tensor, gout: torch.Tensor) -> torch.Tensor:
@@ -431,6 +464,26 @@ def debug_attention_bias(qkv: torch.Tensor, B: int, heads: int, rel_bias: torch.
     if rc != 0:
         raise RuntimeError("w2s_debug_attention_bias: " + lib.w2s_last_error(None).decode())
     return ctx
+
+
+def debug_ctc(logits: torch.Tensor, transcripts, blank: int = PAD_ID, which=None, grad: bool = False):
+    """The library's CTC code on caller logits (tests only): logits fp32 [n, T, V] (CUDA) -> out [n, D] =
+    log p_CTC(y_d | logits[r]) through the head reduction kernel; with ``grad``, also d out[r, which[r]] / d logits[r] as
+    [n, T, V] from the gradient seed kernel (``which`` defaults to 0 for every row)."""
+    lib = _lib.load()
+    n, T, V = logits.shape
+    _check_buffer("logits", logits, torch.float32, n * T * V)
+    labels, offsets = transcript_arrays(transcripts, blank, V)
+    D = len(offsets) - 1
+    out = torch.empty((n, D), dtype=torch.float32, device=logits.device)
+    dl = torch.empty((n, T, V), dtype=torch.float32, device=logits.device) if grad else None
+    w = np.ascontiguousarray(np.broadcast_to(np.asarray(0 if which is None else which, dtype=np.int32), (n,)))
+    rc = lib.w2s_debug_ctc(logits.data_ptr(), n, T, V, V, labels.ctypes.data_as(C.POINTER(C.c_int32)),
+                           offsets.ctypes.data_as(C.POINTER(C.c_int32)), D, int(blank), w.ctypes.data_as(C.POINTER(C.c_int32)),
+                           out.data_ptr(), dl.data_ptr() if dl is not None else None, torch.cuda.current_stream().cuda_stream)
+    if rc != 0:
+        raise RuntimeError("w2s_debug_ctc: " + lib.w2s_last_error(None).decode())
+    return (out, dl) if grad else out
 
 
 def relative_buckets(T: int, num_buckets: int = 320, max_distance: int = 800) -> np.ndarray:

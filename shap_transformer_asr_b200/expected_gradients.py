@@ -27,6 +27,7 @@ import numpy as np
 import torch
 
 from . import dist as wdist
+from .targets import PAD_ID
 
 
 def make_background(num_samples: int, num_background: int = 5, seed: Optional[int] = None) -> np.ndarray:
@@ -47,17 +48,32 @@ class ExpectedGradientsExplainer:
         self.batch = int(batch)
         self.shard_outputs = bool(shard_outputs)     # split the output frames over the ranks of torch.distributed
 
-    def shap_values(self, x, frames=None) -> np.ndarray:
+    def shap_values(self, x, frames=None, transcripts=None, blank: int = PAD_ID) -> np.ndarray:
         """x: normalised clip [L] -> attributions [1, L, D] (the reference's on-disk layout, D = T' when ``frames`` is
         None: every output frame, as ``ranked_outputs=None``).
 
-        The (output frame, sample) passes of ALL outputs form one list that is cut into device calls of ``batch`` rows
-        (every row carries its own target frame), so no call is ragged except the last."""
+        ``transcripts`` (a list of D label-id sequences, exclusive with ``frames``) explains transcript-level outputs
+        instead: output d is log p_CTC(y_d | x) (-WavXForCTC(x, labels=y_d).loss, reduction "sum"; ``blank`` = the model's
+        pad_token_id), one output per transcript, so 200 passes explain a whole transcript where the per-frame question
+        takes T' x 200.  The transcripts are set on the engine (``Engine.set_transcripts``).  Draws are seeded per output
+        index d as per frame; under torch.distributed the outputs are split over the ranks as the frames are, so with D
+        smaller than the world size some ranks idle (sharding the samples of one output is not built).
+
+        The (output, sample) passes of ALL outputs form one list that is cut into device calls of ``batch`` rows
+        (every row carries its own target frame or transcript), so no call is ragged except the last."""
         eng = self.engine
         x = np.ascontiguousarray(np.asarray(x, dtype=np.float32).reshape(-1))
         L = x.size
         T = eng.num_frames(L)
-        frames = np.arange(T, dtype=np.int32) if frames is None else np.asarray(frames, dtype=np.int32)
+        if transcripts is not None:
+            if frames is not None:
+                raise ValueError("frames and transcripts are mutually exclusive")
+            eng.set_transcripts(transcripts, blank)
+            frames = np.arange(len(eng.transcripts), dtype=np.int32)     # output d <-> transcript d
+            grad_rows = eng.grad_transcripts
+        else:
+            frames = np.arange(T, dtype=np.int32) if frames is None else np.asarray(frames, dtype=np.int32)
+            grad_rows = eng.grad_waveforms
         D, S = len(frames), self.nsamples
         bg = torch.from_numpy(self.background).to(eng.device)
         xt = torch.from_numpy(x).to(eng.device)
@@ -80,7 +96,7 @@ class ExpectedGradientsExplainer:
             b = bg[rind_t[r0:r1]]
             delta = xt[None] - b
             xs = torch.addcmul(b, alpha_t[r0:r1, None], delta)
-            g, _ = eng.grad_waveforms(xs, row_frames[r0:r1])
+            g, _ = grad_rows(xs, row_frames[r0:r1])
             phi.index_add_(0, out_of[r0:r1], g * delta)
         phi /= S
         phi = wdist.all_gather_rows(phi, D, rank, world)                       # [D, L] on every rank

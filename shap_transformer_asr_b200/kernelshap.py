@@ -20,7 +20,7 @@ import torch
 from . import _lib
 from . import dist as wdist
 from .engine import background_arrays
-from .targets import char_targets
+from .targets import MAX_TRANSCRIPT, PAD_ID, char_targets, greedy_transcript
 
 
 def unpack_coalitions(words: np.ndarray, M: int) -> np.ndarray:
@@ -169,9 +169,28 @@ class KernelShapExplainer:
         eng.set_targets(mode, frames, tokens)
         return frames, tokens, logits
 
+    def _clip_logits(self, M: int):
+        """-> (logits [T', V] of the unmasked clip, the sampled coalitions).  The one-row forward (one graph replay) is
+        asynchronous on the engine's stream: the coalitions are drawn on the host while it runs, the logits are read
+        back afterwards."""
+        eng = self.engine
+        eng.set_targets("logits")
+        logits_dev = eng.eval_bits(eng.bits_to_device(np.ones((1, M), dtype=np.uint8)))
+        sampled = self._coalitions(M)
+        return logits_dev.view(-1, eng.config.vocab_size).cpu().numpy(), sampled
+
     def explain(self, clip, num_segments: int, mode: str = "logprob", targets=None, baseline: float = 0.0,
-                check: bool = True, background=None, background_weights=None):
-        """-> dict(phi[M, D] fp64 device, fx, fnull, frames, tokens, Z, weights, y, status, info, background_weights).
+                check: bool = True, background=None, background_weights=None, blank: int = PAD_ID):
+        """-> dict(phi[M, D] fp64 device, fx, fnull, frames, tokens, Z, weights, y, status, info, background_weights,
+        transcripts).
+
+        ``mode="transcript"`` explains whole transcripts: output d is log p_CTC(y_d | clip), the log-likelihood the model
+        was trained on (-WavXForCTC(x, labels=y_d).loss, reduction "sum"), with ``blank`` its pad_token_id.  ``targets``
+        is then a list of label-id sequences; by default the greedy transcript of the unmasked clip (the model's own
+        transcription, from the same one-row logits pass that selects per-character targets).  ``transcripts`` in the
+        result lists them (None in the other modes).  A transcript holds at most W2S_MAX_TRANSCRIPT = 512 labels: when
+        the greedy transcript of the clip is longer, explain raises ValueError (pass ``targets`` explicitly, e.g. the
+        transcripts of shorter clips).
 
         ``check`` reads the solve's status word back (one 4-byte D2H after the solve) and raises if the regression
         did not produce a usable answer; a rank-deficient design (status 2: fewer distinct coalitions than segments)
@@ -199,17 +218,23 @@ class KernelShapExplainer:
             eng.clear_background()
         M = eng.num_segments
         sampled = None
+        transcripts = None
         if mode in ("max", "mean", "logits"):
             frames, tokens = (), ()
             eng.set_targets(mode)
+        elif mode == "transcript":
+            frames, tokens = (), ()
+            if targets is None:
+                logits, sampled = self._clip_logits(M)
+                greedy = greedy_transcript(logits, blank)
+                if greedy.size > MAX_TRANSCRIPT:
+                    raise ValueError(f"the greedy transcript of this clip has {greedy.size} labels, more than "
+                                     f"W2S_MAX_TRANSCRIPT = {MAX_TRANSCRIPT}: pass the transcripts as targets")
+                targets = [greedy]
+            eng.set_transcripts(targets, blank)
+            transcripts = eng.transcripts
         elif targets is None:
-            # the one-row target-selection forward (one graph replay) is asynchronous on the engine's stream: the
-            # coalitions are drawn on the host while it runs, the logits are read back afterwards
-            eng.set_targets("logits")
-            ones = eng.bits_to_device(np.ones((1, M), dtype=np.uint8))
-            logits_dev = eng.eval_bits(ones)
-            sampled = self._coalitions(M)
-            logits = logits_dev.view(-1, eng.config.vocab_size).cpu().numpy()
+            logits, sampled = self._clip_logits(M)
             frames, tokens = char_targets(logits)
             eng.set_targets(mode, frames, tokens)
         else:
@@ -247,7 +272,7 @@ class KernelShapExplainer:
                 warnings.warn(f"KernelSHAP design is rank deficient ({K} coalitions for {M} segments): minimum-norm "
                               "attributions returned (shap's lstsq fallback)", RuntimeWarning)
         return dict(phi=phi, fx=fx, fnull=fnull, frames=frames, tokens=tokens, Z=unpack_coalitions(words, M), weights=kw,
-                    y=y_all[2:], status=status, info=info, words=words, background_weights=bg_w)
+                    y=y_all[2:], status=status, info=info, words=words, background_weights=bg_w, transcripts=transcripts)
 
 
 def kmeans_background(X, k: int, round_values: bool = True):
