@@ -111,6 +111,24 @@ int w2s_set_clip(w2s_handle* h, const float* x_dev, int64_t L, const int32_t* se
 int w2s_set_background(w2s_handle* h, const float* bg_dev, int64_t B, int64_t L, int64_t ld, const double* weights_host,
                        void* stream);
 
+/* Time-frequency cells: F band components comp[F, L] of the clip (fp32, device, row stride `ld` elements; copied into the
+ * handle, so the caller may free them when this returns), 1 <= F <= W2S_MAX_BANDS.  Component b is the clip filtered by the
+ * band-b filter H_b of edges 0 = e_0 < e_1 < ... < e_F = sr / 2 (neighbouring edges >= 100 Hz apart): each interior edge e
+ * has the crossover c_e(f) = 1 for f <= e - 50 Hz, 0 for f >= e + 50 Hz and cos^2(pi (f - e + 50) / 200) in between, and
+ * H_b = c_{e_(b+1)} - c_{e_b} with c_{e_0} = 0, c_{e_F} = 1, so sum_b H_b = 1 at every frequency.  x_b = irfft(rfft(x) H_b,
+ * n = L) in float64 (circular over the clip), cast to fp32 (preprocess.band_components computes them).
+ * While bands are set, w2s_eval and w2s_mask take coalitions over M * F cells (M = the segments of w2s_set_clip, M * F <=
+ * 2048): bit s * F + b of a row keeps cell (segment s, band b), and sample i of coalition row k is
+ *   row_k[i] = sum_{b = 0 .. F-1} (keep(k, seg(i) * F + b) ? x_b[i] : 0),
+ * fp32 adds in the order b = 0 .. F-1 from +0.0 (a dropped cell adds +0.0).  The clip itself and the baseline are not read:
+ * the full coalition is f(sum_b x_b), within fp32 rounding of the clip, the empty one f(zeros).  Everything downstream of the
+ * first convolution is unchanged.  w2s_eval_waveforms and the gradient entry points ignore the bands.  Refused before any
+ * launch: F out of range, a null buffer, a background set (bands and a background do not combine), L other than the clip's
+ * (checked again by w2s_eval / w2s_mask when w2s_set_clip has changed it since) and M * F > 2048.  F = 0 clears the bands
+ * and restores the time-only coalitions exactly.  The call synchronises `stream`. */
+#define W2S_MAX_BANDS 16
+int w2s_set_bands(w2s_handle* h, const float* comp_dev, int64_t F, int64_t L, int64_t ld, void* stream);
+
 /* Replaces timestep_to_explain / token_id_to_explain (w2v2conformer.py:93-110) and the character-frame
  * list of visualization.py:319-327: D (frame, token) pairs (host arrays, copied before the call returns; ignored
  * for MAX/MEAN/LOGITS).  The upload is ordered on `stream` behind evaluations already queued there. */
@@ -138,7 +156,8 @@ int64_t w2s_out_width(const w2s_handle* h, int64_t num_samples);
 
 /* The fused masker + model callable: coalition bit matrix z_bits[K, ceil(M/32)] (device; bit m of row k
  * set = segment m KEPT, clear = replaced by the baseline) -> out[K, width] fp32 (device).  With a background
- * (w2s_set_background) K * B rows are evaluated and out[K, width] holds their weighted means. */
+ * (w2s_set_background) K * B rows are evaluated and out[K, width] holds their weighted means.  With bands
+ * (w2s_set_bands) z_bits is [K, ceil(M * F / 32)], one bit per time-frequency cell. */
 int w2s_eval(w2s_handle* h, const uint32_t* z_bits_dev, int64_t K, float* out_dev, void* stream);
 
 /* Replaces ModelWrapper.forward (shap_calculation.py:31-50), predict_function
@@ -190,7 +209,7 @@ int64_t w2s_grad_peek(w2s_handle* h, const char* name, void* dst_dev, int64_t ma
 
 /* Standalone masker (conformer_test.ipynb:138-141 semantics with keep-bits): materialise
  * out[K, L] = keep ? x : baseline for the clip set by w2s_set_clip; with a background, out[K * B, L] with row k * B + b =
- * keep ? x : bg[b] -- the rows w2s_eval evaluates, in its order. */
+ * keep ? x : bg[b]; with bands, out[K, L] = the cell sums of w2s_set_bands -- the rows w2s_eval evaluates, in its order. */
 int w2s_mask(w2s_handle* h, const uint32_t* z_bits_dev, int64_t K, float* out_dev, void* stream);
 
 /* KernelSHAP constrained weighted least squares (shap KernelExplainer.solve with l1_reg=False; SURVEY.md

@@ -18,6 +18,7 @@ OUT_MAX, OUT_LOGIT, OUT_LOGPROB, OUT_MEAN, OUT_LOGITS, OUT_CTC = 0, 1, 2, 3, 4, 
 MODE_IDS = {"max": OUT_MAX, "logit": OUT_LOGIT, "logprob": OUT_LOGPROB, "mean": OUT_MEAN, "logits": OUT_LOGITS}
 FLAG_VALIDATE_GEMM, FLAG_VALIDATE_ATTN, FLAG_FP32_PRELN, FLAG_NO_GRAPH = 1, 2, 4, 16
 MAX_BACKGROUND = 256      # W2S_MAX_BACKGROUND: rows of a background set
+MAX_BANDS = 16            # W2S_MAX_BANDS: frequency bands of time-frequency cells
 MAX_TRANSCRIPT = 512      # W2S_MAX_TRANSCRIPT: labels of one transcript (OUT_CTC, set by w2s_set_transcripts only)
 
 
@@ -61,6 +62,7 @@ SIGNATURES = {
                                C.c_void_p]),
     "w2s_set_background": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.POINTER(C.c_double),
                                      C.c_void_p]),
+    "w2s_set_bands": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p]),
     "w2s_set_targets": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int, C.c_int,
                                   C.c_void_p]),
     "w2s_set_transcripts": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int, C.c_int,

@@ -99,7 +99,8 @@ def masker(x, mask, baseline: float = 0.0):
 class CoalitionCallback:
     """The fused masker + model callable handed to an explainer: f(Z[n, M]) -> [n, D].
 
-    ``Z`` is a host numpy {0,1} matrix (1 = segment kept).  Each call bit-packs it, copies it to the
+    ``Z`` is a host numpy {0,1} matrix [n, engine.num_features] (1 = segment, or with bands time-frequency cell, kept).
+    Each call bit-packs it, copies it to the
     device through pinned memory, runs mask -> Wav2Vec2 -> per-character reduction on the B200 and
     copies the [n, D] result back -- the end-to-end path timed as ``e2e`` by bench.py."""
 
@@ -112,6 +113,8 @@ class CoalitionCallback:
 
     def __call__(self, Z):
         eng = self.engine
+        Z = np.atleast_2d(np.asarray(Z))
+        eng.check_coalition_width(Z.shape[1], packed=False)
         words = pack_coalitions(Z).view(np.int32)
         if self._pin_in is None or self._pin_in.shape != words.shape:
             self._pin_in = torch.empty(words.shape, dtype=torch.int32).pin_memory()

@@ -132,6 +132,12 @@ struct w2s_handle {
   float* bg_rows = nullptr;         // [K * bg_B, width] per-row outputs of the last w2s_eval, reduced by bg_mean_kernel
   long long bg_rows_cap = 0;        // floats; only grows
 
+  // time-frequency cells (w2s_set_bands): bands_F components of bands_L samples; bands_F == 0: time-only coalitions
+  int bands_F = 0;
+  long long bands_L = 0;
+  float* bands = nullptr;           // [bands_F, bands_L]
+  long long bands_cap = 0;          // floats
+
   // targets
   int mode = W2S_OUT_MAX, D = 0, max_frame = 0;
   int *frames = nullptr, *tokens = nullptr;
@@ -163,7 +169,7 @@ struct w2s_handle {
   float* gate = nullptr;        // WavLM: [max_batch, heads, T'] gate of the current layer
   double* wls_work = nullptr;
   long long wls_cap = 0;
-  std::map<std::pair<int, bool>, std::unique_ptr<Plan>> plans;   // keyed by (tile rows, background fill)
+  std::map<std::pair<int, int>, std::unique_ptr<Plan>> plans;   // keyed by (tile rows, fill kind): a graph keeps its conv0
 
   // optional per-launch CUDA-event profile (bench.py roofline leg)
   bool profiling = false;
@@ -219,6 +225,7 @@ struct w2s_handle {
     if (bg) cudaFree(bg);
     if (bg_w) cudaFree(bg_w);
     if (bg_rows) cudaFree(bg_rows);
+    if (bands) cudaFree(bands);
     if (frames) cudaFree(frames);
     if (tokens) cudaFree(tokens);
     for (void* p : {(void*)ctc_labels, (void*)ctc_offsets, (void*)ctc_alpha, (void*)ctc_lse, (void*)ctc_dz})
@@ -584,7 +591,7 @@ struct PlanBuilder {
   Plan* plan;
   int n;
   bool simt_gemm, simt_attn;
-  bool bg;   // conv0 fills dropped samples from the background (DynArgs::bg)
+  int fill;   // which conv0 instantiation reads the input rows (kernels.cuh: Fill)
 
   std::string add_gemm(const std::string& name, const GemmProblem& p) {
     GemmLaunch* gl = new GemmLaunch();
@@ -659,9 +666,10 @@ struct PlanBuilder {
       cp.ln_wbar = h->ln0_wbar; cp.ln_gram = h->ln0_gram; cp.ln_wb = h->ln0_wb;
       cp.ln_bmean = h->ln0_bmean; cp.ln_b2mean = h->ln0_b2mean; cp.ln_wb48 = h->ln0_wb48;
       cp.out = h->bufA;
-      const bool fill = bg;
-      // with a background every row reads its background row besides the clip (both L2-resident across the tile)
-      const double wave_bytes = (fill ? 8.0 : 4.0) * (double)h->ws_L;
+      const int fill = this->fill;
+      // with a background every row reads its background row besides the clip, with cells the F band components (all
+      // L2-resident across the tile)
+      const double wave_bytes = (fill == FILL_BANDS ? 4.0 * h->bands_F : fill == FILL_BG ? 8.0 : 4.0) * (double)h->ws_L;
       if (!layer)
         add("conv0_stats", [=](cudaStream_t s) { return launch_conv0_stats(cp, s, fill); }, 0.0,
             (wave_bytes + (double)cp.C * (8.0 + 64.0)) * n);
@@ -923,8 +931,8 @@ std::string PlanBuilder::build_conformer() {
   return "";
 }
 
-std::string get_plan(w2s_handle* h, int n, bool bg, Plan** out) {
-  auto it = h->plans.find({n, bg});
+std::string get_plan(w2s_handle* h, int n, int fill, Plan** out) {
+  auto it = h->plans.find({n, fill});
   if (it != h->plans.end()) {
     *out = it->second.get();
     return "";
@@ -932,10 +940,10 @@ std::string get_plan(w2s_handle* h, int n, bool bg, Plan** out) {
   std::unique_ptr<Plan> pl(new Plan());
   pl->n = n;
   PlanBuilder b{h, pl.get(), n, (h->cfg.flags & W2S_FLAG_VALIDATE_GEMM) != 0, (h->cfg.flags & W2S_FLAG_VALIDATE_ATTN) != 0,
-                bg};
+                fill};
   W2S_TRY(b.build());
   *out = pl.get();
-  h->plans[{n, bg}] = std::move(pl);
+  h->plans[{n, fill}] = std::move(pl);
   return "";
 }
 
@@ -997,12 +1005,16 @@ std::string run_step(w2s_handle* h, const Step& st, cudaStream_t s) {
 // One evaluation call: rows in tiles of max_batch (the last tile ragged), each tile = one DynArgs update + the plan.
 // With a background (zbits set and bg_B > 0) the call evaluates K * B rows, row g = (coalition g / B, background row
 // g % B), into the handle's per-row scratch, and bg_mean_kernel reduces each coalition's B rows into out[K, width].
+// With time-frequency cells (zbits set and bands_F > 0) each coalition is one row whose bit row has one bit per cell.
 std::string run_batches(w2s_handle* h, const uint32_t* zbits, const float* x, long long ld, int64_t K, float* out,
                         cudaStream_t s) {
   const int64_t width = out_width(h, h->ws_L);
   if (width <= 0) return "no outputs selected (w2s_set_targets)";
   const bool graphs = h->use_graphs && !h->profiling;
   const bool bg = zbits && h->bg_B > 0;
+  const bool cells = zbits && h->bands_F > 0;
+  const int fill = bg ? FILL_BG : cells ? FILL_BANDS : FILL_PLAIN;
+  const int zwords = cells ? (h->M * h->bands_F + 31) / 32 : h->zwords;
   const int64_t rows = bg ? K * h->bg_B : K;
   float* dst = out;
   if (bg) {
@@ -1020,9 +1032,12 @@ std::string run_batches(w2s_handle* h, const uint32_t* zbits, const float* x, lo
   for (int64_t k0 = 0; k0 < rows; k0 += h->cfg.max_batch) {
     const int n = (int)((rows - k0) < h->cfg.max_batch ? (rows - k0) : h->cfg.max_batch);
     Plan* pl = nullptr;
-    W2S_TRY(get_plan(h, n, bg, &pl));
+    W2S_TRY(get_plan(h, n, fill, &pl));
     DynArgs d{};
-    if (bg) {
+    if (cells) {
+      d.seg_id = h->seg_id; d.zbits = zbits + k0 * zwords; d.zwords = zwords;
+      d.bands = h->bands; d.F = h->bands_F; d.ld = h->bands_L;
+    } else if (bg) {
       d.clip = h->clip; d.seg_id = h->seg_id; d.zbits = zbits; d.zwords = h->zwords;
       d.bg = h->bg; d.B = h->bg_B; d.ld = h->bg_L; d.row0 = k0;
     } else if (zbits) {
@@ -1062,6 +1077,18 @@ std::string check_transcripts(const w2s_handle* h, int64_t T) {
     if (h->ctc_need[d] > T)
       return "transcript " + std::to_string(d) + " needs " + std::to_string(h->ctc_need[d]) + " frames, the clip has " +
              std::to_string(T);
+  return "";
+}
+
+// the band components against the clip of the call (w2s_set_clip may have changed it since w2s_set_bands)
+std::string check_bands(const w2s_handle* h) {
+  if (h->bands_F <= 0) return "";
+  if (h->bands_L != h->L)
+    return "the band components have " + std::to_string(h->bands_L) + " samples, the clip has " + std::to_string(h->L) +
+           " (w2s_set_bands again, or clear them with F = 0)";
+  if ((long long)h->M * h->bands_F > 2048)
+    return std::to_string(h->M) + " segments x " + std::to_string(h->bands_F) + " bands = " +
+           std::to_string((long long)h->M * h->bands_F) + " cells; at most 2048 are supported";
   return "";
 }
 
@@ -1262,6 +1289,9 @@ int w2s_set_background(w2s_handle* h, const float* bg_dev, int64_t B, int64_t L,
   if (B < 0 || B > W2S_MAX_BACKGROUND)
     return fail(h, "set_background: B = " + std::to_string(B) + " rows; need 1 <= B <= " +
                        std::to_string(W2S_MAX_BACKGROUND) + " (B = 0 clears the background)");
+  if (h->bands_F > 0)
+    return fail(h, "set_background: frequency bands are set (w2s_set_bands); a background cannot be combined with them "
+                   "(clear the bands with F = 0 first)");
   if (h->L <= 0) return fail(h, "set_background: no clip set (w2s_set_clip)");
   if (L != h->L)
     return fail(h, "set_background: background rows have " + std::to_string(L) + " samples, the clip has " +
@@ -1297,6 +1327,46 @@ int w2s_set_background(w2s_handle* h, const float* bg_dev, int64_t B, int64_t L,
     return fail(h, std::string("set_background: copy failed: ") + cudaGetErrorString(cudaGetLastError()));
   h->bg_B = (int)B;
   h->bg_L = L;
+  return 0;
+}
+
+int w2s_set_bands(w2s_handle* h, const float* comp_dev, int64_t F, int64_t L, int64_t ld, void* stream) {
+  cudaStream_t s = (cudaStream_t)stream;
+  if (F == 0) {
+    h->bands_F = 0;
+    h->bands_L = 0;
+    return 0;
+  }
+  if (F < 0 || F > W2S_MAX_BANDS)
+    return fail(h, "set_bands: F = " + std::to_string(F) + " bands; need 1 <= F <= " + std::to_string(W2S_MAX_BANDS) +
+                       " (F = 0 clears the bands)");
+  if (!comp_dev) return fail(h, "set_bands: null buffer");
+  if (h->bg_B > 0)
+    return fail(h, "set_bands: a background is set (w2s_set_background); bands cannot be combined with it "
+                   "(clear the background with B = 0 first)");
+  if (h->L <= 0) return fail(h, "set_bands: no clip set (w2s_set_clip)");
+  if (L != h->L)
+    return fail(h, "set_bands: band components have " + std::to_string(L) + " samples, the clip has " + std::to_string(h->L));
+  if (ld < L) return fail(h, "set_bands: row stride smaller than the row length");
+  if ((long long)h->M * F > 2048)
+    return fail(h, "set_bands: " + std::to_string(h->M) + " segments x " + std::to_string(F) + " bands = " +
+                       std::to_string((long long)h->M * F) + " cells; at most 2048 are supported");
+  // evaluations in flight on the stream still read the old components
+  if (cudaStreamSynchronize(s) != cudaSuccess) return fail(h, "set_bands: stream error");
+  if (h->bands_cap < F * L) {
+    h->bands_F = 0;   // the old buffer goes now: a failed allocation leaves no bands set, not dangling ones
+    if (h->bands) cudaFree(h->bands);
+    h->bands = nullptr;
+    h->bands_cap = 0;
+    if (cudaMalloc((void**)&h->bands, sizeof(float) * F * L) != cudaSuccess) return fail(h, "set_bands: out of device memory");
+    h->bands_cap = F * L;
+  }
+  if (cudaMemcpy2DAsync(h->bands, sizeof(float) * L, comp_dev, sizeof(float) * ld, sizeof(float) * L, (size_t)F,
+                        cudaMemcpyDeviceToDevice, s) != cudaSuccess ||
+      cudaStreamSynchronize(s) != cudaSuccess)
+    return fail(h, std::string("set_bands: copy failed: ") + cudaGetErrorString(cudaGetLastError()));
+  h->bands_F = (int)F;
+  h->bands_L = L;
   return 0;
 }
 
@@ -1396,8 +1466,10 @@ int w2s_eval(w2s_handle* h, const uint32_t* z_bits_dev, int64_t K, float* out_de
   if (h->bg_B > 0 && h->bg_L != h->L)
     return fail(h, "eval: the background rows have " + std::to_string(h->bg_L) + " samples, the clip has " +
                        std::to_string(h->L) + " (w2s_set_background again, or clear it with B = 0)");
+  std::string e = check_bands(h);
+  if (!e.empty()) return fail(h, "eval: " + e);
   // the workspace (and with it T') follows the clip of THIS call: w2s_eval_waveforms may have left it at another length
-  std::string e = ensure_workspace(h, h->L);
+  e = ensure_workspace(h, h->L);
   if (e.empty()) e = check_targets(h);
   if (e.empty()) e = run_batches(h, z_bits_dev, nullptr, 0, K, out_dev, (cudaStream_t)stream);
   return e.empty() ? 0 : fail(h, "eval: " + e);
@@ -1488,10 +1560,16 @@ int w2s_mask(w2s_handle* h, const uint32_t* z_bits_dev, int64_t K, float* out_de
   if (h->bg_B > 0 && h->bg_L != h->L)
     return fail(h, "mask: the background rows have " + std::to_string(h->bg_L) + " samples, the clip has " +
                        std::to_string(h->L) + " (w2s_set_background again, or clear it with B = 0)");
-  std::string e = h->bg_B > 0 ? launch_mask_bg(h->clip, h->seg_id, z_bits_dev, h->zwords, K, h->L, h->bg, h->bg_B, h->bg_L,
-                                               out_dev, h->L, (cudaStream_t)stream)
-                              : launch_mask(h->clip, h->seg_id, z_bits_dev, h->zwords, K, h->L, h->baseline, out_dev, h->L,
-                                            (cudaStream_t)stream);
+  std::string e = check_bands(h);
+  if (!e.empty()) return fail(h, "mask: " + e);
+  if (h->bands_F > 0)
+    e = launch_mask_bands(h->seg_id, z_bits_dev, (h->M * h->bands_F + 31) / 32, K, h->L, h->bands, h->bands_F, h->bands_L,
+                          out_dev, h->L, (cudaStream_t)stream);
+  else
+    e = h->bg_B > 0 ? launch_mask_bg(h->clip, h->seg_id, z_bits_dev, h->zwords, K, h->L, h->bg, h->bg_B, h->bg_L, out_dev,
+                                     h->L, (cudaStream_t)stream)
+                    : launch_mask(h->clip, h->seg_id, z_bits_dev, h->zwords, K, h->L, h->baseline, out_dev, h->L,
+                                  (cudaStream_t)stream);
   return e.empty() ? 0 : fail(h, e);
 }
 

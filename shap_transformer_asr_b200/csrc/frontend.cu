@@ -8,12 +8,15 @@ namespace w2s {
 // K0  mask + baseline fill.  One thread = 4 consecutive samples (float4 store, 128 B per 8 lanes).
 // Follows feasability_tests/conformer_test.ipynb:138-141 (fill value) with keep-bit convention.
 // =================================================================================================
-// BG: global row g = row0 + blockIdx.y is coalition g / B filled from background row g % B (w2s_set_background)
-template <bool BG>
+// FILL_BG: global row g = row0 + blockIdx.y is coalition g / B filled from background row g % B (w2s_set_background).
+// FILL_BANDS: `bg` holds the B = F band components (row stride bg_ld) and bit s * F + b of the row keeps cell (s, b); the
+// clip and the baseline are not read.
+template <int FILL>
 __global__ void __launch_bounds__(256) mask_kernel(const float* __restrict__ x, const uint16_t* __restrict__ seg_id,
                                                     const uint32_t* __restrict__ zbits, int zwords, long long L,
                                                     float baseline, float* __restrict__ out, long long ld,
                                                     const float* __restrict__ bg, int B, long long bg_ld, long long row0) {
+  constexpr bool BG = FILL == FILL_BG;
   __shared__ uint32_t z[64];
   const long long g = BG ? row0 + blockIdx.y : blockIdx.y;
   const long long k = BG ? g / B : g;
@@ -22,6 +25,30 @@ __global__ void __launch_bounds__(256) mask_kernel(const float* __restrict__ x, 
   const long long i0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * 4;
   if (i0 >= L) return;
   float* o = out + g * ld + i0;
+  if constexpr (FILL == FILL_BANDS) {
+    const int F = B;
+    auto keep = [&](uint32_t sgm, int b) { const uint32_t c = sgm * F + b; return (z[c >> 5] >> (c & 31)) & 1u; };
+    if (i0 + 4 <= L && ((ld & 3) == 0) && (bg_ld & 3) == 0) {
+      const ushort4 sv = *reinterpret_cast<const ushort4*>(seg_id + i0);
+      float4 r = make_float4(0.f, 0.f, 0.f, 0.f);
+      for (int b = 0; b < F; ++b) {
+        const float4 cv = *reinterpret_cast<const float4*>(bg + b * bg_ld + i0);
+        r.x += keep(sv.x, b) ? cv.x : 0.f;
+        r.y += keep(sv.y, b) ? cv.y : 0.f;
+        r.z += keep(sv.z, b) ? cv.z : 0.f;
+        r.w += keep(sv.w, b) ? cv.w : 0.f;
+      }
+      *reinterpret_cast<float4*>(o) = r;
+    } else {
+      for (int j = 0; j < 4 && i0 + j < L; ++j) {
+        const uint32_t sgm = seg_id[i0 + j];
+        float v = 0.f;
+        for (int b = 0; b < F; ++b) v += keep(sgm, b) ? bg[b * bg_ld + i0 + j] : 0.f;
+        o[j] = v;
+      }
+    }
+    return;
+  }
   const float* f = BG ? bg + (g - k * B) * bg_ld : nullptr;
   if (i0 + 4 <= L && ((ld & 3) == 0) && (!BG || (bg_ld & 3) == 0)) {
     const float4 xv = *reinterpret_cast<const float4*>(x + i0);
@@ -48,7 +75,7 @@ std::string launch_mask(const float* x, const uint16_t* seg_id, const uint32_t* 
   if (zwords > 64) return "mask: more than 2048 segments are not supported";
   if (K == 0) return "";
   dim3 grid((unsigned)((L + 1023) / 1024), (unsigned)K);
-  W2S_CUDA_OK(launch_pdl(mask_kernel<false>, grid, dim3(256), 0, s, 1, x, seg_id, zbits, zwords, L, baseline, out, ld,
+  W2S_CUDA_OK(launch_pdl(mask_kernel<FILL_PLAIN>, grid, dim3(256), 0, s, 1, x, seg_id, zbits, zwords, L, baseline, out, ld,
                          (const float*)nullptr, 0, 0LL, 0LL));
   W2S_CUDA_OK(cudaGetLastError());
   return "";
@@ -61,47 +88,79 @@ std::string launch_mask_bg(const float* x, const uint16_t* seg_id, const uint32_
   for (long long r0 = 0; r0 < rows; r0 += 65535) {   // grid.y limit
     const long long n = rows - r0 < 65535 ? rows - r0 : 65535;
     dim3 grid((unsigned)((L + 1023) / 1024), (unsigned)n);
-    W2S_CUDA_OK(launch_pdl(mask_kernel<true>, grid, dim3(256), 0, s, 1, x, seg_id, zbits, zwords, L, 0.f, out, ld, bg, B,
+    W2S_CUDA_OK(launch_pdl(mask_kernel<FILL_BG>, grid, dim3(256), 0, s, 1, x, seg_id, zbits, zwords, L, 0.f, out, ld, bg, B,
                            bg_ld, r0));
     W2S_CUDA_OK(cudaGetLastError());
   }
   return "";
 }
 
-// The same selection folded into a consumer's load: `zs` is the coalition's bit row staged in shared memory.  BG: dropped
-// samples come from a background row instead of the constant (a compile-time variant, so that the baseline-fill kernels
-// keep their code).
-template <bool BG = false>
+std::string launch_mask_bands(const uint16_t* seg_id, const uint32_t* zbits, int zwords, long long K, long long L,
+                              const float* comp, int F, long long comp_ld, float* out, long long ld, cudaStream_t s) {
+  if (zwords > 64) return "mask: more than 2048 cells are not supported";
+  for (long long k0 = 0; k0 < K; k0 += 65535) {   // grid.y limit
+    const long long n = K - k0 < 65535 ? K - k0 : 65535;
+    dim3 grid((unsigned)((L + 1023) / 1024), (unsigned)n);
+    W2S_CUDA_OK(launch_pdl(mask_kernel<FILL_BANDS>, grid, dim3(256), 0, s, 1, (const float*)nullptr, seg_id,
+                           zbits + k0 * zwords, zwords, L, 0.f, out + k0 * ld, ld, comp, F, comp_ld, 0LL));
+    W2S_CUDA_OK(cudaGetLastError());
+  }
+  return "";
+}
+
+// The same selection folded into a consumer's load: `zs` is the coalition's bit row staged in shared memory.  FILL_BG:
+// dropped samples come from a background row instead of the constant; FILL_BANDS: sample i is the sum over bands b of
+// component b where cell (seg(i), b) is kept (compile-time variants, so that the baseline-fill kernels keep their code).
+template <int FILL = FILL_PLAIN>
 struct WaveRow {
-  const float* x;
+  const float* x;        // FILL_BANDS: the band components, rows `ld` apart
   const uint16_t* seg;   // null: plain waveform row
   const uint32_t* zs;
   float baseline;
-  const float* fill;     // BG: background row
+  const float* fill;     // FILL_BG: background row
+  long long ld;          // FILL_BANDS
+  int F;                 // FILL_BANDS
   __device__ __forceinline__ float at(long long i) const {
-    const float v = __ldg(x + i);
-    if constexpr (BG) {
-      const uint32_t sgm = __ldg(seg + i);
-      return (zs[sgm >> 5] >> (sgm & 31)) & 1u ? v : __ldg(fill + i);
+    if constexpr (FILL == FILL_BANDS) {
+      // one L2-resident load and one shared-memory bit test per band; fp32 adds in band order from +0.0
+      const uint32_t c0 = (uint32_t)__ldg(seg + i) * (uint32_t)F;
+      float v = 0.f;
+      for (int b = 0; b < F; ++b) {
+        const uint32_t c = c0 + b;
+        const float t = __ldg(x + b * ld + i);
+        v += (zs[c >> 5] >> (c & 31)) & 1u ? t : 0.f;
+      }
+      return v;
     } else {
-      if (!seg) return v;
-      const uint32_t sgm = __ldg(seg + i);
-      return (zs[sgm >> 5] >> (sgm & 31)) & 1u ? v : baseline;
+      const float v = __ldg(x + i);
+      if constexpr (FILL == FILL_BG) {
+        const uint32_t sgm = __ldg(seg + i);
+        return (zs[sgm >> 5] >> (sgm & 31)) & 1u ? v : __ldg(fill + i);
+      } else {
+        if (!seg) return v;
+        const uint32_t sgm = __ldg(seg + i);
+        return (zs[sgm >> 5] >> (sgm & 31)) & 1u ? v : baseline;
+      }
     }
   }
 };
-// Row `row` of the tile described by the per-call argument block; ends with a CTA-wide barrier.  BG: tile row r is global
-// row g = row0 + r of the call, coalition g / B with background row g % B.
-template <bool BG = false>
-__device__ __forceinline__ WaveRow<BG> wave_row(const DynArgs* __restrict__ dyn, int row, uint32_t* zs) {
-  WaveRow<BG> w;
+// Row `row` of the tile described by the per-call argument block; ends with a CTA-wide barrier.  FILL_BG: tile row r is
+// global row g = row0 + r of the call, coalition g / B with background row g % B.  FILL_BANDS: tile row r is coalition r,
+// its bit row has one bit per time-frequency cell.
+template <int FILL = FILL_PLAIN>
+__device__ __forceinline__ WaveRow<FILL> wave_row(const DynArgs* __restrict__ dyn, int row, uint32_t* zs) {
+  WaveRow<FILL> w;
   w.zs = zs;
-  if constexpr (BG) {
+  if constexpr (FILL == FILL_BG) {
     const long long g = dyn->row0 + row, B = dyn->B, k = g / B;
     const int zw = dyn->zwords;
     for (int i = threadIdx.x; i < zw; i += blockDim.x) zs[i] = dyn->zbits[k * zw + i];
     w.x = dyn->clip; w.seg = dyn->seg_id; w.baseline = 0.f;
     w.fill = dyn->bg + (g - k * B) * dyn->ld;
+  } else if constexpr (FILL == FILL_BANDS) {
+    const int zw = dyn->zwords;
+    for (int i = threadIdx.x; i < zw; i += blockDim.x) zs[i] = dyn->zbits[(long long)row * zw + i];
+    w.x = dyn->bands; w.seg = dyn->seg_id; w.ld = dyn->ld; w.F = dyn->F;
   } else if (dyn->clip) {
     const int zw = dyn->zwords;
     for (int i = threadIdx.x; i < zw; i += blockDim.x) zs[i] = dyn->zbits[(long long)row * zw + i];
@@ -129,7 +188,7 @@ __device__ __forceinline__ double warp_sum_f64(double v) {
   return v;
 }
 
-template <int KW, bool BG>
+template <int KW, int FILL>
 __global__ void __launch_bounds__(256, 1) conv0_stats_kernel(const Conv0Params p) {
   constexpr int NR = KW * (KW + 1) / 2;
   constexpr int NACC = KW + NR;
@@ -137,7 +196,7 @@ __global__ void __launch_bounds__(256, 1) conv0_stats_kernel(const Conv0Params p
   __shared__ double tot[NACC];
   __shared__ uint32_t zs[64];
   const int row = blockIdx.x;
-  const WaveRow<BG> x = wave_row<BG>(p.dyn, row, zs);
+  const WaveRow<FILL> x = wave_row<FILL>(p.dyn, row, zs);
   double acc[NACC];
 #pragma unroll
   for (int i = 0; i < NACC; ++i) acc[i] = 0.0;
@@ -216,11 +275,12 @@ __global__ void __launch_bounds__(256, 1) conv0_stats_kernel(const Conv0Params p
   }
 }
 
-std::string launch_conv0_stats(const Conv0Params& p, cudaStream_t s, bool bg) {
+std::string launch_conv0_stats(const Conv0Params& p, cudaStream_t s, int fill) {
   if (p.kw != 10) return "conv0: only kernel width 10 is implemented for layer 0";
   if (p.n == 0) return "";
-  if (bg) W2S_CUDA_OK(launch_pdl(conv0_stats_kernel<10, true>, dim3(p.n), dim3(256), 0, s, 1, p));
-  else W2S_CUDA_OK(launch_pdl(conv0_stats_kernel<10, false>, dim3(p.n), dim3(256), 0, s, 1, p));
+  if (fill == FILL_BANDS) W2S_CUDA_OK(launch_pdl(conv0_stats_kernel<10, FILL_BANDS>, dim3(p.n), dim3(256), 0, s, 1, p));
+  else if (fill == FILL_BG) W2S_CUDA_OK(launch_pdl(conv0_stats_kernel<10, FILL_BG>, dim3(p.n), dim3(256), 0, s, 1, p));
+  else W2S_CUDA_OK(launch_pdl(conv0_stats_kernel<10, FILL_PLAIN>, dim3(p.n), dim3(256), 0, s, 1, p));
   W2S_CUDA_OK(cudaGetLastError());
   return "";
 }
@@ -232,7 +292,7 @@ std::string launch_conv0_stats(const Conv0Params& p, cudaStream_t s, bool bg) {
 // affine constants in registers; all lanes of a warp work on the same frame, so window reads broadcast.
 // HF wav2vec2/modeling_wav2vec2.py:302-323 (group) / :275-299 (layer).
 // =================================================================================================
-template <int KW, bool LAYER, bool BG>
+template <int KW, bool LAYER, int FILL>
 __global__ void __launch_bounds__(256, 2) conv0_kernel(const Conv0Params p, int FT) {
   extern __shared__ float sm[];
   float* xs = sm;                      // FT*stride + KW window
@@ -243,7 +303,7 @@ __global__ void __launch_bounds__(256, 2) conv0_kernel(const Conv0Params p, int 
   const int row = blockIdx.y;
   const int f0 = blockIdx.x * FT;
   const int nf = min(FT, p.T0 - f0);
-  const WaveRow<BG> x = wave_row<BG>(p.dyn, row, zs);
+  const WaveRow<FILL> x = wave_row<FILL>(p.dyn, row, zs);
   const long long x0 = (long long)f0 * p.stride;
   const int nwin = (nf - 1) * p.stride + KW;
   for (int i = threadIdx.x; i < nwin; i += blockDim.x) {
@@ -330,7 +390,7 @@ __global__ void __launch_bounds__(256, 2) conv0_kernel(const Conv0Params p, int 
 // conflict-free ldmatrix), each warp owns 64 channels whose B fragments stay in registers, and the channel
 // permutation inside a warp is chosen so that a thread ends up with 8 consecutive channels per (frame, half):
 // one 16-byte store, 64 contiguous bytes per quad.
-template <int KW, bool PRE, bool BG>
+template <int KW, bool PRE, int FILL>
 __global__ void __launch_bounds__(256, 2) conv0_mma_kernel(const Conv0Params p, int FT) {
   extern __shared__ __align__(16) uint8_t im2col[];
   constexpr int LDA = 80;
@@ -340,7 +400,7 @@ __global__ void __launch_bounds__(256, 2) conv0_mma_kernel(const Conv0Params p, 
   const int f0 = blockIdx.x * FT;
   const int nf = min(FT, p.T0 - f0);
   const int nfp = (nf + 15) & ~15;
-  const WaveRow<BG> x = wave_row<BG>(p.dyn, row, zs);
+  const WaveRow<FILL> x = wave_row<FILL>(p.dyn, row, zs);
   const long long x0 = (long long)f0 * p.stride;
   for (int i = threadIdx.x; i < nfp * KW; i += blockDim.x) {
     const int f = i / KW, j = i - f * KW;
@@ -413,7 +473,7 @@ __global__ void __launch_bounds__(256, 2) conv0_mma_kernel(const Conv0Params p, 
 // window through the Gram matrix of the filter bank, as in the CUDA-core kernel this replaces.
 constexpr int C0L_K = 48, C0L_LDA = 112;   // 112-byte row pitch: 7 x 16 B, conflict-free ldmatrix
 
-template <int KW, bool PRE, bool BG>
+template <int KW, bool PRE, int FILL>
 __global__ void __launch_bounds__(256, 2) conv0_ln_mma_kernel(const Conv0Params p, int FT) {
   extern __shared__ __align__(16) uint8_t smem_ln[];
   __shared__ uint32_t zs[64];
@@ -423,7 +483,7 @@ __global__ void __launch_bounds__(256, 2) conv0_ln_mma_kernel(const Conv0Params 
   const int f0 = blockIdx.x * FT;
   const int nf = min(FT, p.T0 - f0);
   const int nfp = (nf + 15) & ~15;
-  const WaveRow<BG> x = wave_row<BG>(p.dyn, row, zs);
+  const WaveRow<FILL> x = wave_row<FILL>(p.dyn, row, zs);
   const long long x0 = (long long)f0 * p.stride;
   const int nwin = (nf - 1) * p.stride + KW;
   for (int i = threadIdx.x; i < nwin; i += blockDim.x) xs[i] = x.at(x0 + i);
@@ -549,13 +609,21 @@ std::string launch_conv0_ln_b(const float* w, const float* bias, const float* ga
   return "";
 }
 
-template <bool BG>
+// The gradient path's pre-activation variants (PRE = true) exist for the plain and background fills only: time-frequency
+// cells are an evaluation-path input.
+template <int FILL>
 std::string launch_conv0_t(const Conv0Params& p, bool layer_norm, cudaStream_t s) {
+  constexpr bool kPre = FILL != FILL_BANDS;
+  if (!kPre && p.pre_act) return "conv0: the band-cell fill has no pre-activation variant";
   if (!layer_norm && p.gn_wb && p.C % 64 == 0 && p.C <= 512 && p.n > 0) {
     const int FT = 512;
     dim3 grid((p.T0 + FT - 1) / FT, p.n);
-    if (p.pre_act) W2S_CUDA_OK(launch_pdl(conv0_mma_kernel<10, true, BG>, grid, dim3(p.C / 2), (size_t)FT * 80, s, 1, p, FT));
-    else W2S_CUDA_OK(launch_pdl(conv0_mma_kernel<10, false, BG>, grid, dim3(p.C / 2), (size_t)FT * 80, s, 1, p, FT));
+    if constexpr (kPre) {
+      if (p.pre_act) W2S_CUDA_OK(launch_pdl(conv0_mma_kernel<10, true, FILL>, grid, dim3(p.C / 2), (size_t)FT * 80, s, 1, p, FT));
+      else W2S_CUDA_OK(launch_pdl(conv0_mma_kernel<10, false, FILL>, grid, dim3(p.C / 2), (size_t)FT * 80, s, 1, p, FT));
+    } else {
+      W2S_CUDA_OK(launch_pdl(conv0_mma_kernel<10, false, FILL>, grid, dim3(p.C / 2), (size_t)FT * 80, s, 1, p, FT));
+    }
     W2S_CUDA_OK(cudaGetLastError());
     return "";
   }
@@ -564,14 +632,19 @@ std::string launch_conv0_t(const Conv0Params& p, bool layer_norm, cudaStream_t s
     const size_t smem = (size_t)FT * C0L_LDA + (size_t)(FT * p.stride + p.kw + 4) * sizeof(float);
     static bool attr = false;
     if (!attr) {
-      W2S_CUDA_OK(cudaFuncSetAttribute(conv0_ln_mma_kernel<10, false, BG>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-      W2S_CUDA_OK(cudaFuncSetAttribute(conv0_ln_mma_kernel<10, true, BG>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
+      W2S_CUDA_OK(cudaFuncSetAttribute(conv0_ln_mma_kernel<10, false, FILL>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
+      if constexpr (kPre)
+        W2S_CUDA_OK(cudaFuncSetAttribute(conv0_ln_mma_kernel<10, true, FILL>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
       attr = true;
     }
     if (smem > 100 * 1024) return "conv0 (layer norm): stride too large for the staged window";
     dim3 grid((p.T0 + FT - 1) / FT, p.n);
-    if (p.pre_act) W2S_CUDA_OK(launch_pdl(conv0_ln_mma_kernel<10, true, BG>, grid, dim3(p.C / 2), smem, s, 1, p, FT));
-    else W2S_CUDA_OK(launch_pdl(conv0_ln_mma_kernel<10, false, BG>, grid, dim3(p.C / 2), smem, s, 1, p, FT));
+    if constexpr (kPre) {
+      if (p.pre_act) W2S_CUDA_OK(launch_pdl(conv0_ln_mma_kernel<10, true, FILL>, grid, dim3(p.C / 2), smem, s, 1, p, FT));
+      else W2S_CUDA_OK(launch_pdl(conv0_ln_mma_kernel<10, false, FILL>, grid, dim3(p.C / 2), smem, s, 1, p, FT));
+    } else {
+      W2S_CUDA_OK(launch_pdl(conv0_ln_mma_kernel<10, false, FILL>, grid, dim3(p.C / 2), smem, s, 1, p, FT));
+    }
     W2S_CUDA_OK(cudaGetLastError());
     return "";
   }
@@ -581,15 +654,16 @@ std::string launch_conv0_t(const Conv0Params& p, bool layer_norm, cudaStream_t s
   const int FT = p.T0 >= 4096 ? 512 : 128;
   dim3 grid((p.T0 + FT - 1) / FT, p.n);
   const size_t smem = (size_t)(3 * (FT * p.stride + p.kw) + 2 * FT + 2) * sizeof(float);
-  if (layer_norm) W2S_CUDA_OK(launch_pdl(conv0_kernel<10, true, BG>, grid, dim3(256), smem, s, 1, p, FT));
-  else W2S_CUDA_OK(launch_pdl(conv0_kernel<10, false, BG>, grid, dim3(256), smem, s, 1, p, FT));
+  if (layer_norm) W2S_CUDA_OK(launch_pdl(conv0_kernel<10, true, FILL>, grid, dim3(256), smem, s, 1, p, FT));
+  else W2S_CUDA_OK(launch_pdl(conv0_kernel<10, false, FILL>, grid, dim3(256), smem, s, 1, p, FT));
   W2S_CUDA_OK(cudaGetLastError());
   return "";
 }
 
-std::string launch_conv0(const Conv0Params& p, bool layer_norm, cudaStream_t s, bool bg) {
+std::string launch_conv0(const Conv0Params& p, bool layer_norm, cudaStream_t s, int fill) {
   if (p.kw != 10) return "conv0: only kernel width 10 is implemented for layer 0";
-  return bg ? launch_conv0_t<true>(p, layer_norm, s) : launch_conv0_t<false>(p, layer_norm, s);
+  if (fill == FILL_BANDS) return launch_conv0_t<FILL_BANDS>(p, layer_norm, s);
+  return fill == FILL_BG ? launch_conv0_t<FILL_BG>(p, layer_norm, s) : launch_conv0_t<FILL_PLAIN>(p, layer_norm, s);
 }
 
 // filter-bank statistics for the layer-norm variant: one CTA, trivially small

@@ -11,6 +11,15 @@ std::string launch_mask(const float* x, const uint16_t* seg_id, const uint32_t* 
 // the same with a background bg[B, bg_ld]: out[k * B + b, i] = bit(z[k], seg_id[i]) ? x[i] : bg[b, i]
 std::string launch_mask_bg(const float* x, const uint16_t* seg_id, const uint32_t* zbits, int zwords, long long K,
                            long long L, const float* bg, int B, long long bg_ld, float* out, long long ld, cudaStream_t s);
+// the same over time-frequency cells with band components comp[F, comp_ld]: out[k, i] = sum_{b = 0 .. F-1} (bit(z[k],
+// seg_id[i] * F + b) ? comp[b, i] : 0), fp32 adds in band order from +0.0
+std::string launch_mask_bands(const uint16_t* seg_id, const uint32_t* zbits, int zwords, long long K, long long L,
+                              const float* comp, int F, long long comp_ld, float* out, long long ld, cudaStream_t s);
+
+// Where the kernels that read the masked waveform take a dropped sample from (a compile-time variant of each of them):
+// FILL_PLAIN the baseline (and the explicit-waveform rows), FILL_BG a background row (DynArgs::bg), FILL_BANDS the band
+// components of the kept time-frequency cells (DynArgs::bands)
+enum Fill : int { FILL_PLAIN = 0, FILL_BG = 1, FILL_BANDS = 2 };
 
 // ---- per-call arguments, read by the kernels from device memory ---------------------------------------------
 // Everything that may change between two evaluations of the same batch-tile plan lives here instead of in kernel
@@ -42,6 +51,10 @@ struct DynArgs {
   const int* ctc_labels;
   const int* ctc_offsets;   // [D + 1]
   int blank;
+  // time-frequency cells (w2s_set_bands; read only by the FILL_BANDS instantiations): F band components bands[b * ld + i],
+  // zbits rows hold one bit per cell, bit s * F + b for time segment s and band b
+  const float* bands;
+  int F;
 };
 
 // ---- K1: conv0 (Cin = 1) + GroupNorm-over-time / LayerNorm-over-channels + GELU ------------------------
@@ -68,9 +81,9 @@ struct Conv0Params {
                                  // as bf16 hi/lo rows
   __nv_bfloat16* out;    // [n, T0, C] channels-last
 };
-// bg: the background-fill instantiations (DynArgs::bg); false selects the baseline-fill / explicit-waveform kernels
-std::string launch_conv0_stats(const Conv0Params& p, cudaStream_t s, bool bg = false);   // group-norm statistics
-std::string launch_conv0(const Conv0Params& p, bool layer_norm, cudaStream_t s, bool bg = false);
+// fill: which instantiation reads the input rows (Fill); FILL_PLAIN serves the baseline fill and explicit waveforms
+std::string launch_conv0_stats(const Conv0Params& p, cudaStream_t s, int fill = FILL_PLAIN);   // group-norm statistics
+std::string launch_conv0(const Conv0Params& p, bool layer_norm, cudaStream_t s, int fill = FILL_PLAIN);
 // B operand of the tensor-core layer-norm variant (run once at create)
 std::string launch_conv0_ln_b(const float* w, const float* bias, const float* gamma, const float* beta, int C, int kw,
                               __nv_bfloat16* out, cudaStream_t s);

@@ -61,6 +61,28 @@ def background_arrays(bg, weights=None, num_samples: Optional[int] = None):
     return data, np.ascontiguousarray(w)
 
 
+def band_arrays(components, num_samples: Optional[int] = None, num_segments: Optional[int] = None,
+                background_rows: int = 0):
+    """Validated band components of time-frequency cells: [F, L] (numpy or torch; preprocess.band_components makes them).
+    Raises ValueError naming the problem: not [F, L], F outside 1 .. ``_lib.MAX_BANDS``, a length other than
+    ``num_samples``, ``num_segments * F`` above 2048 cells, or a background set.  Host only."""
+    if components is None:
+        raise ValueError("band components are None")
+    data = components if isinstance(components, torch.Tensor) else np.asarray(components, dtype=np.float32)
+    if data.ndim != 2:
+        raise ValueError(f"band components must be [F, L], got shape {tuple(data.shape)}")
+    F, L = data.shape
+    if F < 1 or F > _lib.MAX_BANDS:
+        raise ValueError(f"{F} bands; need 1 <= F <= {_lib.MAX_BANDS}")
+    if num_samples is not None and L != num_samples:
+        raise ValueError(f"band components have {L} samples, the clip has {num_samples}")
+    if num_segments is not None and num_segments * F > 2048:
+        raise ValueError(f"{num_segments} segments x {F} bands = {num_segments * F} cells; at most 2048 are supported")
+    if background_rows:
+        raise ValueError("a background is set: bands and a background cannot be combined (clear_background first)")
+    return data
+
+
 class Engine:
     """B200 evaluation engine for one model.  ``model`` may be a ``transformers`` Wav2Vec2ForCTC /
     Wav2Vec2ConformerForCTC / WavLMForCTC instance (what the reference builds at shap_calculation.py:218-219) or a
@@ -141,6 +163,7 @@ class Engine:
         self.mode = "max"
         self.background_rows = 0
         self.background_weights = None
+        self.num_bands = 0
         del keep
 
     # -- lifetime ----------------------------------------------------------------------------------
@@ -186,6 +209,8 @@ class Engine:
         segments of coalition k are then filled from each background row in turn, and ``eval_bits`` returns the weighted
         mean over the B rows (w2s_set_background).  The baseline of ``set_clip`` is ignored while a background is set."""
         data, w = background_arrays(bg, weights, num_samples=self.num_samples or None)
+        if self.num_bands:
+            raise ValueError("frequency bands are set: a background cannot be combined with them (clear_bands first)")
         bt = torch.as_tensor(data).to(device=self.device, dtype=torch.float32).contiguous()
         B, L = bt.shape
         self._check(self.lib.w2s_set_background(self._h, bt.data_ptr(), B, L, L, w.ctypes.data_as(C.POINTER(C.c_double)),
@@ -198,6 +223,37 @@ class Engine:
         self._check(self.lib.w2s_set_background(self._h, None, 0, 0, 0, None, self._stream()), "w2s_set_background")
         self.background_rows = 0
         self.background_weights = None
+
+    def set_bands(self, components):
+        """Time-frequency cells (w2s_set_bands): ``components`` [F, L] are the clip's band components
+        (preprocess.band_components; L = the current clip's length, 1 <= F <= 16, num_segments * F <= 2048).  Coalitions
+        then have ``num_features`` = num_segments * F bits, bit s * F + b keeping cell (segment s, band b), and a row is the
+        fp32 sum, in band order, of the kept cells' components.  The clip and the baseline are not read while bands are
+        set; eval_waveforms and the gradient path ignore them."""
+        data = band_arrays(components, self.num_samples or None, self.num_segments or None, self.background_rows)
+        ct = torch.as_tensor(data).to(device=self.device, dtype=torch.float32).contiguous()
+        F, L = ct.shape
+        self._check(self.lib.w2s_set_bands(self._h, ct.data_ptr(), F, L, L, self._stream()), "w2s_set_bands")
+        self.num_bands = F
+
+    def clear_bands(self):
+        """Back to time-only coalitions (bit-identical to never having set bands)."""
+        self._check(self.lib.w2s_set_bands(self._h, None, 0, 0, 0, self._stream()), "w2s_set_bands")
+        self.num_bands = 0
+
+    @property
+    def num_features(self) -> int:
+        """Bits of one coalition row: num_segments, or num_segments * num_bands with time-frequency cells."""
+        return self.num_segments * max(1, self.num_bands)
+
+    def check_coalition_width(self, cols: int, packed: bool):
+        """With bands set a coalition row must have num_features bits: a time-only row would be read as cells."""
+        if not self.num_bands:
+            return
+        want = (self.num_features + 31) // 32 if packed else self.num_features
+        if cols != want:
+            raise ValueError(f"coalition rows have {cols} {'words' if packed else 'columns'}; with {self.num_segments} "
+                             f"segments x {self.num_bands} bands they need {want}")
 
     def set_targets(self, mode: str = "max", frames=None, tokens=None):
         mid = _lib.MODE_IDS[mode]
@@ -238,6 +294,7 @@ class Engine:
     def eval_bits(self, zbits: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """zbits: int32/uint32 device tensor [K, ceil(M/32)] -> float32 device tensor [K, width]."""
         K = zbits.shape[0]
+        self.check_coalition_width(zbits.shape[-1], packed=True)
         width = self.out_width()
         if out is None:
             out = torch.empty((K, width), dtype=torch.float32, device=self.device)
@@ -323,6 +380,7 @@ class Engine:
     def mask(self, zbits: torch.Tensor) -> torch.Tensor:
         """The rows ``eval_bits`` evaluates: [K, L], or [K * B, L] (row k * B + b) with a background."""
         K = zbits.shape[0]
+        self.check_coalition_width(zbits.shape[-1], packed=True)
         out = torch.empty((K * max(1, self.background_rows), self.num_samples), dtype=torch.float32, device=self.device)
         self._check(self.lib.w2s_mask(self._h, zbits.data_ptr(), K, out.data_ptr(), self._stream()), "w2s_mask")
         return out
@@ -343,6 +401,7 @@ class Engine:
         """Host {0,1} matrix [K, M] (or already packed uint32 words [K, ceil(M/32)]) -> device int32 words.  The
         pinned staging buffer is owned by the engine and re-used (grown geometrically) across calls."""
         Z = np.asarray(Z)
+        self.check_coalition_width(Z.shape[-1], packed=Z.dtype == np.uint32)
         words = (Z if Z.dtype == np.uint32 else pack_coalitions(Z)).view(np.int32)
         n = words.size
         if self._pin_bits is None or self._pin_bits.numel() < n:

@@ -20,6 +20,7 @@ import torch
 from . import _lib
 from . import dist as wdist
 from .engine import background_arrays
+from .preprocess import band_components, check_band_edges
 from .targets import MAX_TRANSCRIPT, PAD_ID, char_targets, greedy_transcript
 
 
@@ -169,20 +170,21 @@ class KernelShapExplainer:
         eng.set_targets(mode, frames, tokens)
         return frames, tokens, logits
 
-    def _clip_logits(self, M: int):
-        """-> (logits [T', V] of the unmasked clip, the sampled coalitions).  The one-row forward (one graph replay) is
-        asynchronous on the engine's stream: the coalitions are drawn on the host while it runs, the logits are read
-        back afterwards."""
+    def _clip_logits(self, M: int, num_features: Optional[int] = None):
+        """-> (logits [T', V] of the unmasked clip, the coalitions sampled over ``num_features`` (default M) features).
+        The one-row forward (one graph replay) is asynchronous on the engine's stream: the coalitions are drawn on the host
+        while it runs, the logits are read back afterwards."""
         eng = self.engine
         eng.set_targets("logits")
         logits_dev = eng.eval_bits(eng.bits_to_device(np.ones((1, M), dtype=np.uint8)))
-        sampled = self._coalitions(M)
+        sampled = self._coalitions(num_features or M)
         return logits_dev.view(-1, eng.config.vocab_size).cpu().numpy(), sampled
 
     def explain(self, clip, num_segments: int, mode: str = "logprob", targets=None, baseline: float = 0.0,
-                check: bool = True, background=None, background_weights=None, blank: int = PAD_ID):
+                check: bool = True, background=None, background_weights=None, blank: int = PAD_ID, band_edges=None,
+                sr: int = 16000):
         """-> dict(phi[M, D] fp64 device, fx, fnull, frames, tokens, Z, weights, y, status, info, background_weights,
-        transcripts).
+        transcripts, phi_cells, band_edges).
 
         ``mode="transcript"`` explains whole transcripts: output d is log p_CTC(y_d | clip), the log-likelihood the model
         was trained on (-WavXForCTC(x, labels=y_d).loss, reduction "sum"), with ``blank`` its pad_token_id.  ``targets``
@@ -202,7 +204,15 @@ class KernelShapExplainer:
         evaluated once per background row with the dropped segments taken from that row, and its output is the
         weighted mean over the rows; ``baseline`` is not used.  The targets are selected on the clip itself.  With
         ``background=None`` dropped segments are filled with ``baseline``; ``background_weights`` in the result is then
-        None, else the normalised float64 weights."""
+        None, else the normalised float64 weights.
+
+        ``band_edges`` (F + 1 edges in Hz from 0 to sr / 2, e.g. ``preprocess.mel_band_edges(F)``) explains time-frequency
+        cells: the clip is split into F band components (``preprocess.band_components``) and feature s * F + b is band b
+        of segment s, so M = num_segments * F.  The targets are selected on the clip itself; the coalitions are then
+        evaluated with the bands set (a row is the sum of its kept cells' components, the empty coalition is silence, the
+        full one the sum of all components) and the engine is left with time-only coalitions.  The result adds
+        ``phi_cells`` = phi viewed as [num_segments, F, D] and the float64 ``band_edges`` (both None without bands).
+        Bands cannot be combined with a background."""
         eng = self.engine
         eng.set_clip(clip, num_segments=num_segments, baseline=baseline)
         bg = None
@@ -214,9 +224,20 @@ class KernelShapExplainer:
             bg = background_arrays(background, background_weights, num_samples=eng.num_samples)
         elif background_weights is not None:
             raise ValueError("background_weights given without a background")
+        edges = None
+        if band_edges is not None:
+            if bg is not None:
+                raise ValueError("band_edges cannot be combined with a background")
+            edges = check_band_edges(band_edges, sr)
+            if eng.num_segments * (edges.size - 1) > 2048:
+                raise ValueError(f"{eng.num_segments} segments x {edges.size - 1} bands = "
+                                 f"{eng.num_segments * (edges.size - 1)} cells; at most 2048 are supported")
         if getattr(eng, "background_rows", 0):
             eng.clear_background()
+        if getattr(eng, "num_bands", 0):
+            eng.clear_bands()
         M = eng.num_segments
+        Mf = M if edges is None else M * (edges.size - 1)     # features: segments, or time-frequency cells
         sampled = None
         transcripts = None
         if mode in ("max", "mean", "logits"):
@@ -225,7 +246,7 @@ class KernelShapExplainer:
         elif mode == "transcript":
             frames, tokens = (), ()
             if targets is None:
-                logits, sampled = self._clip_logits(M)
+                logits, sampled = self._clip_logits(M, Mf)
                 greedy = greedy_transcript(logits, blank)
                 if greedy.size > MAX_TRANSCRIPT:
                     raise ValueError(f"the greedy transcript of this clip has {greedy.size} labels, more than "
@@ -234,18 +255,20 @@ class KernelShapExplainer:
             eng.set_transcripts(targets, blank)
             transcripts = eng.transcripts
         elif targets is None:
-            logits, sampled = self._clip_logits(M)
+            logits, sampled = self._clip_logits(M, Mf)
             frames, tokens = char_targets(logits)
             eng.set_targets(mode, frames, tokens)
         else:
             frames, tokens = targets
             eng.set_targets(mode, frames, tokens)
         if sampled is None:
-            sampled = self._coalitions(M)
+            sampled = self._coalitions(Mf)
         words, kw, info = sampled["words"], sampled["kw"], sampled["info"]
         K = words.shape[0]
         if bg is not None:
             eng.set_background(*bg)
+        if edges is not None:
+            eng.set_bands(band_components(clip, edges, sr))
         # rows 0 / 1 of the evaluated matrix are the empty and the full coalition (fnull, fx): fx comes from the same
         # reduction kernel as every y row, so the efficiency constraint is consistent to the last bit
         rank, world = wdist.rank_world() if self.shard_coalitions else (0, 1)
@@ -258,21 +281,25 @@ class KernelShapExplainer:
         y_all = wdist.all_gather_rows(y_local, K + 2, rank, world)
         fnull = y_all[0].double()
         fx = y_all[1].double()
-        phi, status = eng.wls(bits_all[2:], sampled["w_dev"], y_all[2:], fx, fnull, M)
+        phi, status = eng.wls(bits_all[2:], sampled["w_dev"], y_all[2:], fx, fnull, Mf)
         bg_w = None
         if bg is not None:
             bg_w = eng.background_weights
             eng.clear_background()      # the engine is left as it was found: baseline fill
+        if edges is not None:
+            eng.clear_bands()           # ... and time-only coalitions
         if check:
             st = int(status.item())
             if st == 1:
                 raise RuntimeError("KernelSHAP regression did not converge (w2s_wls status 1)")
             if st == 2:
                 import warnings
-                warnings.warn(f"KernelSHAP design is rank deficient ({K} coalitions for {M} segments): minimum-norm "
+                warnings.warn(f"KernelSHAP design is rank deficient ({K} coalitions for {Mf} features): minimum-norm "
                               "attributions returned (shap's lstsq fallback)", RuntimeWarning)
-        return dict(phi=phi, fx=fx, fnull=fnull, frames=frames, tokens=tokens, Z=unpack_coalitions(words, M), weights=kw,
-                    y=y_all[2:], status=status, info=info, words=words, background_weights=bg_w, transcripts=transcripts)
+        phi_cells = None if edges is None else phi.view(M, edges.size - 1, phi.shape[1])
+        return dict(phi=phi, fx=fx, fnull=fnull, frames=frames, tokens=tokens, Z=unpack_coalitions(words, Mf), weights=kw,
+                    y=y_all[2:], status=status, info=info, words=words, background_weights=bg_w, transcripts=transcripts,
+                    phi_cells=phi_cells, band_edges=edges)
 
 
 def kmeans_background(X, k: int, round_values: bool = True):
