@@ -42,7 +42,8 @@ enum {
   W2S_FLAG_VALIDATE_GEMM = 1,  /* run every contraction on the CUDA-core validation kernels (same bf16 data) */
   W2S_FLAG_VALIDATE_ATTN = 2,  /* run attention on the CUDA-core validation kernel                            */
   W2S_FLAG_FP32_PRELN    = 4,  /* post-LN models: fp32 (instead of bf16) pre-LayerNorm tensors -- A/B measurement */
-  W2S_FLAG_NO_GRAPH      = 16  /* launch the kernels of a tile one by one instead of replaying a CUDA graph        */
+  W2S_FLAG_NO_GRAPH      = 16, /* launch the kernels of a tile one by one instead of replaying a CUDA graph        */
+  W2S_FLAG_DENSE_FRONTEND = 32 /* compute every feature-encoder frame, also those whose input is all baseline -- A/B */
 };
 
 /* Mirrors transformers.Wav2Vec2Config / Wav2Vec2ConformerConfig (the objects the reference
@@ -238,6 +239,14 @@ int64_t w2s_sample_rows(int M, int n_full, int n_paired, const int64_t* ind_set,
  * frames: out[r] = bucket(r - (T - 1)), r = 0 .. 2T-2, computed on the HOST in double precision.  Returns 0, or 1 on a bad
  * argument (T < 1, num_buckets < 4, max_distance <= num_buckets / 4).  No device is touched. */
 int w2s_relative_buckets(int T, int num_buckets, int max_distance, int32_t* out);
+
+/* Block table of the feature encoder's constant-frame skip: for conv layers 1 .. num_layers - 1 of a clip of L samples
+ * cut into M segments (seg_bounds[0 .. M], ascending, 0 .. L), one row of 4 int32 per 128-frame output block, layers in
+ * order: the first and last segment that the receptive field of the block touches, and the first and last 128-frame
+ * block of the layer below that the block reads.  Returns the number of rows (written only when <= cap), or -1 on a bad
+ * argument.  Computed on the HOST; no device is touched. */
+int64_t w2s_frontend_blocks(int num_layers, const int32_t* kernel, const int32_t* stride, int64_t L,
+                            const int32_t* seg_bounds, int M, int32_t* out, int64_t cap);
 
 /* Test / profiling hooks for the individual kernels (used by tests/ and bench.py only). */
 /* out[M, N] = act(a[M, K] w[N, K]^T + bias) * alpha + residual (residual == out with fp32 data: in-place

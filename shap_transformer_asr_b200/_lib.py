@@ -16,7 +16,7 @@ MAX_CONV_LAYERS = 8
 
 OUT_MAX, OUT_LOGIT, OUT_LOGPROB, OUT_MEAN, OUT_LOGITS, OUT_CTC = 0, 1, 2, 3, 4, 5
 MODE_IDS = {"max": OUT_MAX, "logit": OUT_LOGIT, "logprob": OUT_LOGPROB, "mean": OUT_MEAN, "logits": OUT_LOGITS}
-FLAG_VALIDATE_GEMM, FLAG_VALIDATE_ATTN, FLAG_FP32_PRELN, FLAG_NO_GRAPH = 1, 2, 4, 16
+FLAG_VALIDATE_GEMM, FLAG_VALIDATE_ATTN, FLAG_FP32_PRELN, FLAG_NO_GRAPH, FLAG_DENSE_FRONTEND = 1, 2, 4, 16, 32
 MAX_BACKGROUND = 256      # W2S_MAX_BACKGROUND: rows of a background set
 MAX_BANDS = 16            # W2S_MAX_BANDS: frequency bands of time-frequency cells
 MAX_TRANSCRIPT = 512      # W2S_MAX_TRANSCRIPT: labels of one transcript (OUT_CTC, set by w2s_set_transcripts only)
@@ -86,6 +86,8 @@ SIGNATURES = {
     "w2s_sample_rows": (C.c_int64, [C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "w2s_relative_buckets": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "w2s_frontend_blocks": (C.c_int64, [C.c_int, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int, C.c_void_p,
+                                        C.c_int64]),
     "w2s_debug_gemm": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_float,
                                  C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "w2s_debug_attention": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p,

@@ -4,6 +4,7 @@
 #include "../../include/w2s.h"
 #include "gemm.cuh"
 #include "kernels.cuh"
+#include "skip.cuh"
 #include "ctc.cuh"
 
 #include <algorithm>
@@ -44,6 +45,8 @@ struct Step {
   std::function<std::string(cudaStream_t)> run;
   double flops = 0.0;  // algorithmic FLOPs (2*MAC) of this launch, 0 for non-contraction kernels
   double bytes = 0.0;  // algorithmic HBM bytes of this launch (HBM-bound kernels)
+  // launches over a device list (frontend skip): the profile reads the count back and charges flops / bytes per entry
+  const int* work = nullptr;
 };
 
 struct ProfRec {
@@ -169,7 +172,17 @@ struct w2s_handle {
   float* gate = nullptr;        // WavLM: [max_batch, heads, T'] gate of the current layer
   double* wls_work = nullptr;
   long long wls_cap = 0;
-  std::map<std::pair<int, int>, std::unique_ptr<Plan>> plans;   // keyed by (tile rows, fill kind): a graph keeps its conv0
+  std::map<std::pair<int, int>, std::unique_ptr<Plan>> plans;   // keyed by (tile rows, fill kind | PLAN_SKIP): a graph keeps its conv0
+
+  // constant-frame skip of the feature encoder (frontend_skip.cu), sized with the workspace: block table of the clip
+  // (w2s_frontend_blocks, uploaded by w2s_set_clip) and the per-tile block lists of conv1 .. conv_{nl}
+  int4* skip_tab = nullptr;
+  int skip_rows = 0;
+  bool skip_tab_ok = false;                 // skip_tab holds the table of the current clip (w2s_set_clip bounds, L == ws_L)
+  std::vector<int32_t> seg_bounds;          // [M + 1] of the current clip: the table is rebuilt with the workspace
+  int* skip_live[SKIP_MAX_LAYERS] = {};
+  int* skip_fill[SKIP_MAX_LAYERS] = {};
+  int* skip_rep = nullptr;
 
   // optional per-launch CUDA-event profile (bench.py roofline leg)
   bool profiling = false;
@@ -495,6 +508,21 @@ void free_workspace(w2s_handle* h) {
   h->ws_L = -1;
 }
 
+// Block table of the current clip into the workspace (w2s_frontend_blocks); the skip is used only after this succeeded.
+std::string upload_skip_table(w2s_handle* h, cudaStream_t s) {
+  h->skip_tab_ok = false;
+  if (!h->skip_rows || h->ws_L != h->L || h->seg_bounds.size() != (size_t)h->M + 1) return "";
+  const w2s_config& c = h->cfg;
+  std::vector<int32_t> tab((size_t)4 * h->skip_rows);
+  if (w2s_frontend_blocks(c.num_conv_layers, c.conv_kernel, c.conv_stride, h->L, h->seg_bounds.data(), h->M, tab.data(),
+                          h->skip_rows) != h->skip_rows)
+    return "frontend block table: inconsistent clip geometry";
+  W2S_CUDA_OK(cudaMemcpyAsync(h->skip_tab, tab.data(), sizeof(int32_t) * tab.size(), cudaMemcpyHostToDevice, s));
+  W2S_CUDA_OK(cudaStreamSynchronize(s));
+  h->skip_tab_ok = true;
+  return "";
+}
+
 std::string ensure_workspace(w2s_handle* h, long long L) {
   if (h->ws_L == L) return "";
   cudaDeviceSynchronize();
@@ -527,6 +555,26 @@ std::string ensure_workspace(w2s_handle* h, long long L) {
     const size_t s = nb * (size_t)h->Tl[l] * c.conv_dim[l];
     if (l % 2 == 0) szA = s > szA ? s : szA;
     else szB = s > szB ? s : szB;
+  }
+  {
+    std::vector<int32_t> kw(c.conv_kernel, c.conv_kernel + c.num_conv_layers), st(c.conv_stride, c.conv_stride + c.num_conv_layers);
+    const int32_t whole[2] = {0, (int32_t)L};
+    const int64_t nrows = c.num_conv_layers >= 2 && c.num_conv_layers - 1 <= SKIP_MAX_LAYERS
+                              ? w2s_frontend_blocks(c.num_conv_layers, kw.data(), st.data(), L, whole, 1, nullptr, 0) : 0;
+    // list entries pack (coalition << 16) | block: beyond that range the plans stay dense
+    bool fits = nb < 32768;
+    for (int l = 1; l < c.num_conv_layers; ++l) fits = fits && (h->Tl[l] + 127) / 128 < 65536;
+    h->skip_rows = nrows > 0 && fits ? (int)nrows : 0;
+    h->skip_tab_ok = false;
+    if (h->skip_rows) {
+      W2S_TRY(dalloc(pool, &h->skip_tab, (size_t)h->skip_rows));
+      W2S_TRY(dalloc(pool, &h->skip_rep, nb * (c.num_conv_layers - 1)));
+      for (int l = 1; l < c.num_conv_layers; ++l) {
+        const size_t cap = 1 + nb * (size_t)((h->Tl[l] + 127) / 128);
+        W2S_TRY(dalloc(pool, &h->skip_live[l - 1], cap));
+        W2S_TRY(dalloc(pool, &h->skip_fill[l - 1], cap));
+      }
+    }
   }
   W2S_TRY(dalloc(pool, &h->bufA, szA));
   W2S_TRY(dalloc(pool, &h->bufB, szB ? szB : 1));
@@ -580,6 +628,8 @@ std::string ensure_workspace(w2s_handle* h, long long L) {
     }
   }
   h->ws_L = L;
+  // a workspace rebuilt for the clip's length (e.g. after w2s_eval_waveforms at another length) gets the clip's table back
+  if (L == h->L) W2S_TRY(upload_skip_table(h, 0));
   return "";
 }
 
@@ -592,6 +642,7 @@ struct PlanBuilder {
   int n;
   bool simt_gemm, simt_attn;
   int fill;   // which conv0 instantiation reads the input rows (kernels.cuh: Fill)
+  bool skip;  // conv1 .. conv6 contract only the blocks that see kept audio (frontend_skip.cu)
 
   std::string add_gemm(const std::string& name, const GemmProblem& p) {
     GemmLaunch* gl = new GemmLaunch();
@@ -677,6 +728,22 @@ struct PlanBuilder {
           2.0 * cp.T0 * (double)cp.C * cp.kw * n, ((double)cp.T0 * cp.C * 2.0 + wave_bytes) * n);
     }
     // ---- K2: conv1..6 as implicit GEMM over the stride-row view of the previous layer ---------------------
+    // With the skip, the block lists of every layer are built first (one launch), each contraction walks its list and a
+    // fill launch copies the representative row into the blocks of constant frames that the next layer reads.
+    SkipParams sp{};
+    const size_t list_step = plan->steps.size();
+    if (skip) {
+      sp.dyn = h->dyn_dev; sp.tab = h->skip_tab; sp.nl = c.num_conv_layers - 1; sp.n = n; sp.total = h->skip_rows;
+      sp.rep = h->skip_rep;
+      for (int l = 0, o = 0; l < sp.nl; ++l) {
+        sp.nb[l] = (h->Tl[l + 1] + 127) / 128;
+        sp.off[l] = o;
+        o += sp.nb[l];
+        sp.live[l] = h->skip_live[l];
+        sp.fill[l] = h->skip_fill[l];
+      }
+      add("frontend_lists", nullptr, 0.0, (double)n * (h->skip_rows * (16.0 + 8.0) + h->zwords * 4.0));
+    }
     bf16* cur = h->bufA;
     for (int l = 1; l < c.num_conv_layers; ++l) {
       bf16* nxt = (l % 2 == 1) ? h->bufB : h->bufA;
@@ -692,11 +759,29 @@ struct PlanBuilder {
       p.epi.act = layer ? ACT_NONE : ACT_GELU;
       p.epi.out = nxt; p.epi.ldb = (long long)Tout * Cout; p.epi.ldm = Cout;
       W2S_TRY(add_gemm("conv" + std::to_string(l), p));
+      const GemmLaunch* gl = plan->gemms.back();
+      sp.dense[l - 1] = !(gl->mc == 2 && gl->bn == 256 && gl->tma_out && !simt_gemm);
+      if (skip && !sp.dense[l - 1]) {
+        Step& st = plan->steps.back();
+        const int* live = sp.live[l - 1];
+        st.run = [gl, live](cudaStream_t s) { return gemm2_launch_list(*gl, live, s); };
+        st.flops = 2.0 * 128 * (double)p.N * p.K;   // per listed block
+        st.work = live;
+        const int* fl = sp.fill[l - 1];
+        const int* rp = sp.rep + (size_t)(l - 1) * n;
+        const int nsm = h->num_sms;
+        Step f{"conv" + std::to_string(l) + "_fill",
+               [fl, rp, nxt, Tout, Cout, nsm](cudaStream_t s) { return launch_skip_fill(fl, rp, nxt, Tout, Cout, nsm, s); }};
+        f.bytes = 128.0 * Cout * 2.0;   // per filled block (the representative rows are L2-resident)
+        f.work = fl;
+        plan->steps.push_back(std::move(f));
+      }
       if (layer)
         add_ln("conv" + std::to_string(l) + "_ln_gelu", nxt, 0, (long long)n * Tout, Cout, h->conv_ln_g[l],
                h->conv_ln_b[l], 1e-5f, ACT_GELU, nxt, nullptr);
       cur = nxt;
     }
+    if (skip) plan->steps[list_step].run = [sp](cudaStream_t s) { return launch_skip_lists(sp, s); };
     // ---- K3: feature projection ---------------------------------------------------------------------------
     const int Cl = c.conv_dim[c.num_conv_layers - 1];
     add_ln("featproj_ln", cur, 0, rows, Cl, h->fp_ln_g, h->fp_ln_b, c.layer_norm_eps, ACT_NONE, h->fpn, nullptr);
@@ -931,6 +1016,9 @@ std::string PlanBuilder::build_conformer() {
   return "";
 }
 
+// plan kind: the Fill of conv0, plus PLAN_SKIP for coalition evaluations that take the constant-frame skip
+constexpr int PLAN_SKIP = 8;
+
 std::string get_plan(w2s_handle* h, int n, int fill, Plan** out) {
   auto it = h->plans.find({n, fill});
   if (it != h->plans.end()) {
@@ -940,7 +1028,7 @@ std::string get_plan(w2s_handle* h, int n, int fill, Plan** out) {
   std::unique_ptr<Plan> pl(new Plan());
   pl->n = n;
   PlanBuilder b{h, pl.get(), n, (h->cfg.flags & W2S_FLAG_VALIDATE_GEMM) != 0, (h->cfg.flags & W2S_FLAG_VALIDATE_ATTN) != 0,
-                fill};
+                fill & ~PLAN_SKIP, (fill & PLAN_SKIP) != 0};
   W2S_TRY(b.build());
   *out = pl.get();
   h->plans[{n, fill}] = std::move(pl);
@@ -997,6 +1085,13 @@ std::string run_step(w2s_handle* h, const Step& st, cudaStream_t s) {
   std::string e = st.run(s);
   if (h->profiling) {
     cudaEventRecord(rec.e1, s);
+    if (st.work) {   // the work this launch executed: entries of its device list
+      int cnt = 0;
+      cudaMemcpyAsync(&cnt, st.work, sizeof(int), cudaMemcpyDeviceToHost, s);
+      cudaStreamSynchronize(s);
+      rec.flops *= cnt;
+      rec.bytes *= cnt;
+    }
     h->prof.push_back(rec);
   }
   return e.empty() ? "" : st.name + ": " + e;
@@ -1016,6 +1111,9 @@ std::string run_batches(w2s_handle* h, const uint32_t* zbits, const float* x, lo
   const int fill = bg ? FILL_BG : cells ? FILL_BANDS : FILL_PLAIN;
   const int zwords = cells ? (h->M * h->bands_F + 31) / 32 : h->zwords;
   const int64_t rows = bg ? K * h->bg_B : K;
+  // the constant-frame skip: coalitions over the baseline fill, group-norm front end, tensor-core contractions
+  const bool skip = zbits && fill == FILL_PLAIN && h->skip_tab_ok && h->cfg.feat_extract_norm == 0 &&
+                    (h->cfg.flags & (W2S_FLAG_DENSE_FRONTEND | W2S_FLAG_VALIDATE_GEMM)) == 0;
   float* dst = out;
   if (bg) {
     const long long need = rows * width;
@@ -1032,7 +1130,7 @@ std::string run_batches(w2s_handle* h, const uint32_t* zbits, const float* x, lo
   for (int64_t k0 = 0; k0 < rows; k0 += h->cfg.max_batch) {
     const int n = (int)((rows - k0) < h->cfg.max_batch ? (rows - k0) : h->cfg.max_batch);
     Plan* pl = nullptr;
-    W2S_TRY(get_plan(h, n, fill, &pl));
+    W2S_TRY(get_plan(h, n, fill | (skip ? PLAN_SKIP : 0), &pl));
     DynArgs d{};
     if (cells) {
       d.seg_id = h->seg_id; d.zbits = zbits + k0 * zwords; d.zwords = zwords;
@@ -1275,6 +1373,9 @@ int w2s_set_clip(w2s_handle* h, const float* x_dev, int64_t L, const int32_t* se
   h->M = M;
   h->zwords = (M + 31) / 32;
   h->baseline = baseline;
+  h->seg_bounds.assign(seg_bounds_host, seg_bounds_host + M + 1);
+  e = upload_skip_table(h, s);
+  if (!e.empty()) return fail(h, "set_clip: " + e);
   return 0;
 }
 

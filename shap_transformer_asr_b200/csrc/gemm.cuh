@@ -70,6 +70,8 @@ std::string gemm_launch_tc(const GemmLaunch& l, cudaStream_t s);
 std::string gemm_launch_simt(const GemmLaunch& l, cudaStream_t s);
 std::string gemm2_init();
 std::string gemm2_launch(const GemmLaunch& l, cudaStream_t s);
+// the pair kernel over a device list of 128-row blocks (list[0] = count, then (batch << 16) | block); l.grid as prepared
+std::string gemm2_launch_list(const GemmLaunch& l, const int* list, cudaStream_t s);
 std::string gemm_init();  // resolves cuTensorMapEncodeTiled, sets kernel attributes
 
 // shared by other translation units that build their own tensor maps (attention)

@@ -27,14 +27,28 @@ struct Tc2Cfg {
   static constexpr size_t SMEM = (size_t)STAGES * STAGE_BYTES + EPI_BYTES + 1024 + 256;
 };
 
-template <int BN>
+// LIST: the 128-row blocks come from a device list instead of the dense (n-tile, m-pair, batch) walk (feature-encoder
+// convolutions, frontend_skip.cu): list[0] is the count, list[1 + e] = (batch << 16) | block.  Rank r of a pair takes
+// entry 2u + r, so a pair may join blocks of two coalitions (the CTAs share only the W half-tiles); a missing partner of
+// an odd count computes a block past the output and stores nothing.  The grid stays as captured, the count is read here.
+template <int BN, bool LIST = false>
 __global__ void __launch_bounds__(384, 1)
 gemm_tc2_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapW,
-                const __grid_constant__ CUtensorMap mapOut, const GemmDev p, const int tma_out) {
+                const __grid_constant__ CUtensorMap mapOut, const GemmDev p, const int tma_out,
+                const int* __restrict__ list = nullptr) {
   using C = Tc2Cfg<BN>;
   const uint32_t rank = cluster_ctarank();
   const bool leader = rank == 0;
   const int unit0 = (int)(blockIdx.x >> 1), unit_step = (int)(gridDim.x >> 1);
+  const int list_n = LIST ? list[0] : 0;
+  const int num_units = LIST ? (list_n + 1) / 2 * p.tiles_n : p.num_units;
+  // list entry of this CTA in unit `unit`: (batch, first row); a list dummy gets a row past the output
+  auto list_block = [&](int unit, int& b, int& m0) {
+    const int e = 2 * (unit / p.tiles_n) + (int)rank;
+    const int v = e < list_n ? __ldg(list + 1 + e) : -1;
+    b = v < 0 ? 0 : v >> 16;
+    m0 = v < 0 ? p.units_m * 256 : (v & 0xffff) * 128;
+  };
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw = smem_u32(smem_raw);
   const uint32_t tiles = (raw + 1023u) & ~1023u;
@@ -81,13 +95,18 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
     if (elect_one()) {
       int stage = 0;
       uint32_t phase = 0;
-      for (int unit = unit0; unit < p.num_units; unit += unit_step) {
+      for (int unit = unit0; unit < num_units; unit += unit_step) {
         int nt = unit % p.tiles_n;
         int r = unit / p.tiles_n;
         const int mu = r % p.units_m;
         r /= p.units_m;
-        const int b = r % p.Bz, g = r / p.Bz;
-        const int m0 = (2 * mu + (int)rank) * 128, n0 = nt * BN;
+        int b = r % p.Bz, g = r / p.Bz;
+        int m0 = (2 * mu + (int)rank) * 128;
+        if constexpr (LIST) {
+          list_block(unit, b, m0);
+          g = 0;
+        }
+        const int n0 = nt * BN;
         for (int kb = 0; kb < p.num_kb; ++kb) {
           mbar_wait(empty_bar(stage), phase ^ 1u);
           const uint32_t full_leader = mapa_u32(full_bar(stage), 0);
@@ -113,7 +132,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
       uint32_t phase = 0;
       int acc = 0;
       uint32_t acc_phase = 0;
-      for (int unit = unit0; unit < p.num_units; unit += unit_step) {
+      for (int unit = unit0; unit < num_units; unit += unit_step) {
         mbar_wait(tempty_bar(acc), acc_phase ^ 1u);
         tc_fence_after();
         const uint32_t d_tmem = tmem_base + acc * C::ACC_COLS;
@@ -147,13 +166,19 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
     const bool reduce_add = tma_out && f32 && p.epi.res_fp32 && p.epi.residual == p.epi.out;
     int acc = 0;
     uint32_t acc_phase = 0;
-    for (int unit = unit0; unit < p.num_units; unit += unit_step) {
+    for (int unit = unit0; unit < num_units; unit += unit_step) {
       int nt = unit % p.tiles_n;
       int r = unit / p.tiles_n;
       const int mu = r % p.units_m;
       r /= p.units_m;
-      const int b = r % p.Bz, g = r / p.Bz;
-      const int m0 = (2 * mu + (int)rank) * 128, n0 = nt * BN;
+      int b = r % p.Bz, g = r / p.Bz;
+      int m0 = (2 * mu + (int)rank) * 128;
+      if constexpr (LIST) {
+        list_block(unit, b, m0);
+        g = 0;
+      }
+      const int n0 = nt * BN;
+      const bool store = !LIST || m0 < p.M;
       const int m = m0 + q * 32 + lane;
       const bool row_ok = m < p.M;
       const uint32_t t0 = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc * C::ACC_COLS;
@@ -211,7 +236,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
             const int cblk = f32 ? c : c - 32;
             fence_proxy_async();
             __syncwarp();
-            if (lead) {
+            if (lead && store) {
               if (reduce_add) tma_reduce_add_4d(&mapOut, stg, n0 + cblk, m0 + q * 32, b, g);
               else tma_store_4d(&mapOut, stg, n0 + cblk, m0 + q * 32, b, g);   // rows >= M are clipped by the tensor map
               tma_store_commit();
@@ -254,6 +279,9 @@ std::string gemm2_init() {
                                        (int)Tc2Cfg<256>::SMEM);
   if (e == cudaSuccess)
     e = cudaFuncSetAttribute(gemm_tc2_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Tc2Cfg<128>::SMEM);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(gemm_tc2_kernel<256, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)Tc2Cfg<256>::SMEM);
   if (e != cudaSuccess) return std::string("cudaFuncSetAttribute(gemm_tc2_kernel): ") + cudaGetErrorString(e);
   return "";
 }
@@ -263,7 +291,14 @@ size_t gemm2_smem(int bn) { return bn == 256 ? Tc2Cfg<256>::SMEM : Tc2Cfg<128>::
 template <int BN>
 static cudaError_t launch2(const GemmLaunch& l, cudaStream_t s) {
   return launch_pdl(gemm_tc2_kernel<BN>, dim3(l.grid), dim3(384), Tc2Cfg<BN>::SMEM, s, 2, l.mapA, l.mapW,
-                    l.tma_out ? l.mapOut : l.mapA, l.dev, l.tma_out);
+                    l.tma_out ? l.mapOut : l.mapA, l.dev, l.tma_out, (const int*)nullptr);
+}
+
+std::string gemm2_launch_list(const GemmLaunch& l, const int* list, cudaStream_t s) {
+  if (l.mc != 2 || l.bn != 256 || !l.tma_out || l.dev.G != 1) return "gemm (block list): needs the TMA-store pair kernel, BN = 256";
+  W2S_CUDA_OK(launch_pdl(gemm_tc2_kernel<256, true>, dim3(l.grid), dim3(384), Tc2Cfg<256>::SMEM, s, 2, l.mapA, l.mapW,
+                         l.mapOut, l.dev, l.tma_out, list));
+  return "";
 }
 
 std::string gemm2_launch(const GemmLaunch& l, cudaStream_t s) {

@@ -90,7 +90,7 @@ class Engine:
 
     def __init__(self, model, config: Optional[ModelConfig] = None, device: int = 0, max_batch: int = 0,
                  validate_gemm: bool = False, validate_attn: bool = False, preln_fp32: bool = False,
-                 graphs: bool = True):
+                 graphs: bool = True, dense_frontend: bool = False):
         if not torch.cuda.is_available():
             raise RuntimeError("no CUDA device: the masked-coalition path has no CPU fallback")
         self.lib = _lib.load()
@@ -143,7 +143,8 @@ class Engine:
         cfg.max_bucket_distance = config.max_bucket_distance
         cfg.max_batch = int(max_batch)
         cfg.flags = ((_lib.FLAG_VALIDATE_GEMM if validate_gemm else 0) | (_lib.FLAG_VALIDATE_ATTN if validate_attn else 0)
-                     | (_lib.FLAG_FP32_PRELN if preln_fp32 else 0) | (0 if graphs else _lib.FLAG_NO_GRAPH))
+                     | (_lib.FLAG_FP32_PRELN if preln_fp32 else 0) | (0 if graphs else _lib.FLAG_NO_GRAPH)
+                     | (_lib.FLAG_DENSE_FRONTEND if dense_frontend else 0))
         names = list(keep.keys())
         n = len(names)
         c_names = (C.c_char_p * n)(*[s.encode() for s in names])
