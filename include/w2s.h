@@ -34,7 +34,14 @@ enum {
   W2S_OUT_LOGPROB = 2, /* log_softmax(logits)[t_d,tok_d] -> [n, D]   north-star per-character CTC output      */
   W2S_OUT_MEAN    = 3, /* mean over vocab and time       -> [n, 1]   lime_shap_wav2vec2_comparison.py:68-70   */
   W2S_OUT_LOGITS  = 4, /* raw logits                     -> [n, T', V]  (target selection, parity tests)      */
-  W2S_OUT_CTC     = 5  /* log p_CTC(y_d | all frames)     -> [n, D]   set by w2s_set_transcripts only            */
+  W2S_OUT_CTC     = 5, /* log p_CTC(y_d | all frames)     -> [n, D]   set by w2s_set_transcripts only            */
+  W2S_OUT_ERRORS  = 6  /* edit distance greedy -> y_d     -> [n, D]   set by w2s_set_references only             */
+};
+
+/* Units of W2S_OUT_ERRORS (w2s_set_references `unit`). */
+enum {
+  W2S_ERR_LABELS = 0,  /* Levenshtein distance over label ids                                   */
+  W2S_ERR_WORDS  = 1   /* Levenshtein distance over words split on the delimiter label          */
 };
 
 /* w2s_config.flags */
@@ -151,6 +158,25 @@ int w2s_set_targets(w2s_handle* h, const int32_t* frame_idx_host, const int32_t*
 #define W2S_MAX_TRANSCRIPT 512
 int w2s_set_transcripts(w2s_handle* h, const int32_t* labels_host, const int32_t* offsets_host, int D, int blank,
                         void* stream);
+
+/* Recognition errors W2S_OUT_ERRORS: D >= 1 reference label sequences y_d = labels[offsets[d] .. offsets[d + 1]) (host
+ * arrays, validated as in w2s_set_transcripts: 0 <= U_d <= W2S_MAX_TRANSCRIPT, labels in [0, V) and != blank, blank in
+ * [0, V); any U_d is valid whatever the clip's T').  Row r then reports out[r, d] = the edit distance between the row's
+ * greedy transcript and y_d, an integer held in fp32.  The greedy transcript is a_t = argmax_v logits[r, t, v] (the lowest
+ * id among equal maxima, as torch.argmax picks) over the T' frames, with repeats collapsed (a_t dropped when it equals
+ * a_(t-1)) and then blanks dropped.
+ *   unit W2S_ERR_LABELS: the Levenshtein distance over label ids (unit cost per substitution, insertion and deletion);
+ *   unit W2S_ERR_WORDS: both sequences are split on `delimiter` (in [0, V), != blank; ignored for labels) and empty words
+ *   dropped; two words are equal when their label sequences are identical; the output is the word-level Levenshtein
+ *   distance, i.e. WER x N for a reference of N >= 1 words and the number of hypothesis words for an empty reference.
+ * Counts are not normalised.  Each value is one fixed sequence of integer and compare operations on the row's logits:
+ * bit-identical for any batch tile, position in the tile, number of GPUs and across calls.  With a background the usual
+ * weighted mean applies (the expected error count).  The references are kept apart from the transcripts of
+ * w2s_set_transcripts: w2s_grad_transcripts keeps using the transcripts last set there and never sees references, and
+ * this output has no gradient entry point.  Every check runs before the device is touched; the upload is ordered on
+ * `stream` as in w2s_set_targets. */
+int w2s_set_references(w2s_handle* h, const int32_t* labels_host, const int32_t* offsets_host, int D, int blank, int unit,
+                       int delimiter, void* stream);
 
 /* Number of fp32 values one evaluated row produces under the current mode for clips of L samples. */
 int64_t w2s_out_width(const w2s_handle* h, int64_t num_samples);
@@ -280,6 +306,19 @@ int w2s_debug_attention_bwd(int use_tcgen05, const void* qkv, const void* ctx, c
  * w2s_last_error(NULL). */
 int w2s_debug_ctc(const float* logits, int n, int T, int V, int ldl, const int32_t* labels_host, const int32_t* offsets_host,
                   int D, int blank, const int32_t* which_host, float* out_dev, float* dlogits_dev, void* stream);
+/* The code of W2S_OUT_ERRORS on caller logits [n, T, ldl] (fp32, device; V <= ldl used): out[n, D] (device) through the
+ * head reduction kernel; the references are validated as in w2s_set_references.  The call synchronises the stream.  Errors
+ * via w2s_last_error(NULL). */
+int w2s_debug_errors(const float* logits, int n, int T, int V, int ldl, const int32_t* labels_host,
+                     const int32_t* offsets_host, int D, int blank, int unit, int delimiter, float* out_dev, void* stream);
+/* The device tables w2s_set_references builds for these references over a vocabulary of V ids: the number of int32
+ * entries (written to out only when <= cap), or -1 on an argument w2s_set_references refuses.  Layout (csrc/errors.cuh):
+ * 8 header ints per reference (units m, first match-mask row, first distinct-word record, distinct words, longest word,
+ * zeros), the reference labels, (start, length) records of the distinct words, then match-mask rows of 16 words: bit
+ * i % 32 of word i / 32 set when unit i is the row's symbol (V rows per reference for labels, one per distinct word for
+ * words).  Computed on the HOST; no device is touched. */
+int64_t w2s_error_tables(const int32_t* labels_host, const int32_t* offsets_host, int D, int V, int blank, int unit,
+                         int delimiter, int32_t* out, int64_t cap);
 /* Per-launch CUDA-event profile on the launching stream (bench.py roofline leg): enable, run evaluations,
  * then read per launch class (newline-separated names) total milliseconds, algorithmic FLOPs / bytes and
  * launch counts.  Returns the number of classes, or -1 if `names_cap` is too small. */

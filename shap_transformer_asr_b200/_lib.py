@@ -14,7 +14,8 @@ LIB_PATH = os.path.join(_HERE, "libw2s.so")
 
 MAX_CONV_LAYERS = 8
 
-OUT_MAX, OUT_LOGIT, OUT_LOGPROB, OUT_MEAN, OUT_LOGITS, OUT_CTC = 0, 1, 2, 3, 4, 5
+OUT_MAX, OUT_LOGIT, OUT_LOGPROB, OUT_MEAN, OUT_LOGITS, OUT_CTC, OUT_ERRORS = 0, 1, 2, 3, 4, 5, 6
+ERR_UNITS = {"labels": 0, "words": 1}     # W2S_ERR_LABELS / W2S_ERR_WORDS (OUT_ERRORS, set by w2s_set_references only)
 MODE_IDS = {"max": OUT_MAX, "logit": OUT_LOGIT, "logprob": OUT_LOGPROB, "mean": OUT_MEAN, "logits": OUT_LOGITS}
 FLAG_VALIDATE_GEMM, FLAG_VALIDATE_ATTN, FLAG_FP32_PRELN, FLAG_NO_GRAPH, FLAG_DENSE_FRONTEND = 1, 2, 4, 16, 32
 MAX_BACKGROUND = 256      # W2S_MAX_BACKGROUND: rows of a background set
@@ -67,6 +68,8 @@ SIGNATURES = {
                                   C.c_void_p]),
     "w2s_set_transcripts": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int, C.c_int,
                                       C.c_void_p]),
+    "w2s_set_references": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int, C.c_int, C.c_int,
+                                     C.c_int, C.c_void_p]),
     "w2s_out_width": (C.c_int64, [C.c_void_p, C.c_int64]),
     "w2s_eval": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "w2s_eval_waveforms": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
@@ -98,6 +101,10 @@ SIGNATURES = {
                                           C.c_float, C.c_void_p, C.c_void_p]),
     "w2s_debug_ctc": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
                                 C.c_int, C.c_int, C.POINTER(C.c_int32), C.c_void_p, C.c_void_p, C.c_void_p]),
+    "w2s_debug_errors": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
+                                   C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "w2s_error_tables": (C.c_int64, [C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                     C.c_void_p, C.c_int64]),
     "w2s_profile_enable": (C.c_int, [C.c_void_p, C.c_int]),
     "w2s_profile_read": (C.c_int64, [C.c_void_p, C.c_char_p, C.c_int64, C.POINTER(C.c_double), C.POINTER(C.c_double),
                                      C.POINTER(C.c_double), C.POINTER(C.c_int64), C.c_int64]),

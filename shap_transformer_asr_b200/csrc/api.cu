@@ -6,6 +6,7 @@
 #include "kernels.cuh"
 #include "skip.cuh"
 #include "ctc.cuh"
+#include "errors.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -156,6 +157,12 @@ struct w2s_handle {
   float *ctc_alpha = nullptr, *ctc_lse = nullptr, *ctc_dz = nullptr;   // gradient-seed scratch, grown on demand
   long long ctc_alpha_cap = 0, ctc_lse_cap = 0, ctc_dz_cap = 0;
 
+  // references (w2s_set_references): the tables of errors.cuh, apart from the transcripts
+  int err_D = 0, err_blank = 0, err_unit = 0, err_delim = 0;
+  int* err_tab = nullptr;
+  long long err_tab_cap = 0;
+  std::vector<int32_t> err_host;        // staging of the upload
+
   // workspace (sized for max_batch rows of the current clip length)
   long long ws_L = -1;
   int T = 0, Tp = 0;
@@ -241,7 +248,7 @@ struct w2s_handle {
     if (bands) cudaFree(bands);
     if (frames) cudaFree(frames);
     if (tokens) cudaFree(tokens);
-    for (void* p : {(void*)ctc_labels, (void*)ctc_offsets, (void*)ctc_alpha, (void*)ctc_lse, (void*)ctc_dz})
+    for (void* p : {(void*)ctc_labels, (void*)ctc_offsets, (void*)ctc_alpha, (void*)ctc_lse, (void*)ctc_dz, (void*)err_tab})
       if (p) cudaFree(p);
     if (wls_work) cudaFree(wls_work);
     for (void* p : ws_allocs) cudaFree(p);
@@ -1042,6 +1049,7 @@ int64_t out_width(const w2s_handle* h, int64_t L) {
     case W2S_OUT_MEAN: return 1;
     case W2S_OUT_LOGITS: return T * h->cfg.vocab_size;
     case W2S_OUT_CTC: return h->ctc_D;
+    case W2S_OUT_ERRORS: return h->err_D;
     default: return h->D;
   }
 }
@@ -1145,8 +1153,11 @@ std::string run_batches(w2s_handle* h, const uint32_t* zbits, const float* x, lo
       d.x = x + k0 * ld; d.ld = ld;
     }
     d.out = dst + k0 * width;
-    d.mode = h->mode; d.D = h->mode == W2S_OUT_CTC ? h->ctc_D : h->D; d.frames = h->frames; d.tokens = h->tokens;
-    d.ctc_labels = h->ctc_labels; d.ctc_offsets = h->ctc_offsets; d.blank = h->ctc_blank;
+    d.mode = h->mode; d.D = h->mode == W2S_OUT_CTC ? h->ctc_D : h->mode == W2S_OUT_ERRORS ? h->err_D : h->D;
+    d.frames = h->frames; d.tokens = h->tokens;
+    d.ctc_labels = h->ctc_labels; d.ctc_offsets = h->ctc_offsets;
+    d.blank = h->mode == W2S_OUT_ERRORS ? h->err_blank : h->ctc_blank;
+    d.err_tab = h->err_tab; d.err_unit = h->err_unit; d.delim = h->err_delim;
     set_dyn_kernel<<<1, 1, 0, s>>>(h->dyn_dev, d);
     W2S_CUDA_OK(cudaGetLastError());
     h->launches += 1 + (long long)pl->steps.size();
@@ -1221,6 +1232,59 @@ std::string validate_transcripts(const int32_t* labels, const int32_t* offsets, 
       if (labels[u] == blank) return "transcript " + std::to_string(d) + ": label equal to the blank " + std::to_string(blank);
     }
     (*need)[(size_t)d] = ctc_frames_needed(labels + offsets[d], U);
+  }
+  return "";
+}
+
+// w2s_set_references / w2s_debug_errors / w2s_error_tables: the argument checks (host only) and the tables of errors.cuh
+std::string error_tables(const int32_t* labels, const int32_t* offsets, int D, int V, int blank, int unit, int delim,
+                         std::vector<int32_t>* tab) {
+  std::vector<int> need;
+  std::string e = validate_transcripts(labels, offsets, D, blank, V, &need);
+  if (!e.empty()) return e;
+  if (unit != W2S_ERR_LABELS && unit != W2S_ERR_WORDS)
+    return "unit " + std::to_string(unit) + " is neither W2S_ERR_LABELS (0) nor W2S_ERR_WORDS (1)";
+  if (unit == W2S_ERR_WORDS && (delim < 0 || delim >= V || delim == blank))
+    return "delimiter " + std::to_string(delim) + " outside the vocabulary [0, " + std::to_string(V) + ") or equal to the blank";
+  const int total = offsets[D];
+  tab->assign((size_t)ERR_HDR * D, 0);
+  const int lab0 = (int)tab->size();
+  tab->insert(tab->end(), labels, labels + total);
+  for (int d = 0; d < D; ++d) {
+    int* hdr = nullptr;
+    std::vector<int> sym;               // symbol of every unit: its label, or the index of its distinct word
+    std::vector<int32_t> rec;           // (start, length) of every distinct word
+    int maxw = 0;
+    if (unit == W2S_ERR_LABELS) {
+      sym.assign(labels + offsets[d], labels + offsets[d + 1]);
+    } else {
+      std::map<std::vector<int32_t>, int> ids;
+      for (int u = offsets[d]; u < offsets[d + 1];) {
+        if (labels[u] == delim) {
+          ++u;
+          continue;
+        }
+        int v = u;
+        while (v < offsets[d + 1] && labels[v] != delim) ++v;
+        auto it = ids.emplace(std::vector<int32_t>(labels + u, labels + v), (int)ids.size()).first;
+        if (it->second == (int)rec.size() / 2) {
+          rec.push_back(lab0 + u);
+          rec.push_back(v - u);
+        }
+        sym.push_back(it->second);
+        maxw = std::max(maxw, v - u);
+        u = v;
+      }
+    }
+    const int rows = unit == W2S_ERR_LABELS ? V : (int)rec.size() / 2;
+    const int dw = (int)tab->size();
+    tab->insert(tab->end(), rec.begin(), rec.end());
+    const int peq = (int)tab->size();
+    tab->resize(tab->size() + (size_t)rows * ERR_LANES, 0);
+    for (size_t i = 0; i < sym.size(); ++i)
+      (*tab)[peq + (size_t)sym[i] * ERR_LANES + i / 32] |= (int32_t)(1u << (i % 32));
+    hdr = tab->data() + (size_t)ERR_HDR * d;
+    hdr[0] = (int)sym.size(); hdr[1] = peq; hdr[2] = dw; hdr[3] = (int)rec.size() / 2; hdr[4] = maxw;
   }
   return "";
 }
@@ -1558,6 +1622,44 @@ int w2s_set_transcripts(w2s_handle* h, const int32_t* labels_host, const int32_t
   return 0;
 }
 
+int w2s_set_references(w2s_handle* h, const int32_t* labels_host, const int32_t* offsets_host, int D, int blank, int unit,
+                       int delimiter, void* stream) {
+  cudaStream_t s = (cudaStream_t)stream;
+  std::vector<int32_t> tab;
+  const std::string e = error_tables(labels_host, offsets_host, D, h->cfg.vocab_size, blank, unit, delimiter, &tab);
+  if (!e.empty()) return fail(h, "set_references: " + e);
+  if (h->err_tab_cap < (long long)tab.size()) {
+    // evaluations in flight on the stream still read the old tables
+    if (cudaStreamSynchronize(s) != cudaSuccess) return fail(h, "set_references: stream error");
+    h->err_D = 0;   // a failed allocation below leaves no references set, not dangling ones
+    if (h->err_tab) cudaFree(h->err_tab);
+    h->err_tab = nullptr;
+    h->err_tab_cap = 0;
+    const long long cap = std::max<long long>((long long)tab.size(), 4096);
+    if (cudaMalloc((void**)&h->err_tab, sizeof(int) * cap) != cudaSuccess) return fail(h, "set_references: out of device memory");
+    h->err_tab_cap = cap;
+  }
+  // ordered on the caller's stream, staged in the handle (as w2s_set_targets)
+  h->err_host = std::move(tab);
+  if (cudaMemcpyAsync(h->err_tab, h->err_host.data(), sizeof(int) * h->err_host.size(), cudaMemcpyHostToDevice, s) !=
+      cudaSuccess)
+    return fail(h, "set_references: copy failed");
+  h->err_D = D;
+  h->err_blank = blank;
+  h->err_unit = unit;
+  h->err_delim = delimiter;
+  h->mode = W2S_OUT_ERRORS;
+  return 0;
+}
+
+int64_t w2s_error_tables(const int32_t* labels_host, const int32_t* offsets_host, int D, int V, int blank, int unit,
+                         int delimiter, int32_t* out, int64_t cap) {
+  std::vector<int32_t> tab;
+  if (V < 1 || !error_tables(labels_host, offsets_host, D, V, blank, unit, delimiter, &tab).empty()) return -1;
+  if (out && (int64_t)tab.size() <= cap) std::copy(tab.begin(), tab.end(), out);
+  return (int64_t)tab.size();
+}
+
 int64_t w2s_out_width(const w2s_handle* h, int64_t num_samples) { return out_width(h, num_samples); }
 
 int w2s_eval(w2s_handle* h, const uint32_t* z_bits_dev, int64_t K, float* out_dev, void* stream) {
@@ -1879,6 +1981,44 @@ int w2s_debug_ctc(const float* logits, int n, int T, int V, int ldl, const int32
   }
   if (!e.empty()) {
     g_create_error = e;
+    return 1;
+  }
+  return 0;
+}
+
+int w2s_debug_errors(const float* logits, int n, int T, int V, int ldl, const int32_t* labels_host,
+                     const int32_t* offsets_host, int D, int blank, int unit, int delimiter, float* out_dev, void* stream) {
+  g_create_error.clear();
+  const cudaStream_t s = (cudaStream_t)stream;
+  std::vector<int32_t> tab;
+  std::string e;
+  if (n <= 0 || T <= 0 || V <= 0 || V > 128 || ldl < V || !logits || !out_dev)
+    e = "need n, T >= 1, 1 <= V <= 128, ldl >= V and logits / out buffers";
+  if (e.empty()) e = error_tables(labels_host, offsets_host, D, V, blank, unit, delimiter, &tab);
+  if (e.empty()) {
+    int* dtab = nullptr;
+    DynArgs* dyn = nullptr;
+    if (cudaMalloc((void**)&dtab, sizeof(int) * tab.size()) != cudaSuccess ||
+        cudaMalloc((void**)&dyn, sizeof(DynArgs)) != cudaSuccess)
+      e = "out of device memory";
+    DynArgs d{};
+    d.out = out_dev; d.mode = W2S_OUT_ERRORS; d.D = D; d.blank = blank; d.err_tab = dtab; d.err_unit = unit; d.delim = delimiter;
+    if (e.empty() && (cudaMemcpyAsync(dtab, tab.data(), sizeof(int) * tab.size(), cudaMemcpyHostToDevice, s) != cudaSuccess ||
+                      cudaMemcpyAsync(dyn, &d, sizeof(DynArgs), cudaMemcpyHostToDevice, s) != cudaSuccess))
+      e = "copy failed";
+    if (e.empty()) {
+      HeadParams hp{};
+      hp.n = n; hp.T = T; hp.V = V; hp.ldl = ldl; hp.dyn = dyn;
+      e = launch_head_reduce(logits, hp, s);
+    }
+    // the buffers live for this call only
+    const cudaError_t se = cudaStreamSynchronize(s);
+    if (se != cudaSuccess && e.empty()) e = cudaGetErrorString(se);
+    for (void* p : {(void*)dtab, (void*)dyn})
+      if (p) cudaFree(p);
+  }
+  if (!e.empty()) {
+    g_create_error = "debug_errors: " + e;
     return 1;
   }
   return 0;

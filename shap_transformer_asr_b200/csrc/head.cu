@@ -4,10 +4,12 @@
 //   log-softmax at (frame, token)  north-star per-character CTC log-probability
 //   mean over vocab and time       feasability_tests/lime_shap_wav2vec2_comparison.py:68-70
 //   CTC log-likelihood of a transcript over all frames (ctc.cuh), -Wav2Vec2ForCTC(x, labels=y).loss
+//   edit distance of the greedy transcript to a reference (errors.cuh), WER x N of sweep.explain_test_set
 // One warp per (row, frame) work item: lane = vocabulary entry, so log-softmax and gather are warp
 // shuffles (HF wav2vec2/modeling_wav2vec2.py:1705-1708 for the linear layer).
 #include "kernels.cuh"
 #include "ctc.cuh"
+#include "errors.cuh"
 #include "../../include/w2s.h"
 
 namespace w2s {
@@ -44,9 +46,11 @@ __device__ __forceinline__ void head_reduce_frame(const float (&logit)[HEAD_MAXJ
 }
 
 // Work items per mode: MAX / LOGITS one per (row, frame); LOGIT / LOGPROB one per (row, target); CTC one per (row,
-// transcript); MEAN one per row (the warp walks the frames in order, so the sum is bit-reproducible -- no atomics).
+// transcript); ERRORS one per (row, reference); MEAN one per row (the warp walks the frames in order, so the sum is
+// bit-reproducible -- no atomics).
 __device__ __forceinline__ long long head_items(const DynArgs& d, int n, int T) {
-  if (d.mode == W2S_OUT_LOGIT || d.mode == W2S_OUT_LOGPROB || d.mode == W2S_OUT_CTC) return (long long)n * d.D;
+  if (d.mode == W2S_OUT_LOGIT || d.mode == W2S_OUT_LOGPROB || d.mode == W2S_OUT_CTC || d.mode == W2S_OUT_ERRORS)
+    return (long long)n * d.D;
   if (d.mode == W2S_OUT_MEAN) return n;
   return (long long)n * T;
 }
@@ -112,6 +116,19 @@ __global__ void __launch_bounds__(256) head_kernel(const HeadParams p) {
       if (lane == 0) d.out[(long long)b * d.D + dd] = r;
       continue;
     }
+    if (d.mode == W2S_OUT_ERRORS) {
+      const int b = (int)(it / d.D), dd = (int)(it - (long long)b * d.D);
+      const int r = errors_warp<HEAD_MAXJ>(p.T, p.V, d.err_tab, dd, d.err_unit, d.blank, d.delim, lane,
+                                           reinterpret_cast<int*>(ctc_alpha + warp * CTC_MAX_S),
+                                           [&](int t, float(&lg)[HEAD_MAXJ]) {
+                                             frame_logits(b, t, lg);
+#pragma unroll
+                                             for (int j = 0; j < HEAD_MAXJ; ++j)
+                                               if (lane + 32 * j >= p.V) lg[j] = -INFINITY;
+                                           });
+      if (lane == 0) d.out[(long long)b * d.D + dd] = (float)r;
+      continue;
+    }
     if (d.mode == W2S_OUT_MEAN) {
       float sm = 0.f;
       for (int t = 0; t < p.T; ++t) {
@@ -142,8 +159,8 @@ __global__ void __launch_bounds__(256) head_kernel(const HeadParams p) {
 }
 
 // second stage of the tensor-core head: logits[rows, ldl] (fp32, bias included) -> reduction; one warp per work item.
-// Six blocks per SM, as before the CTC branch was added: its alpha rows take 32.8 KB of shared memory per block, and the
-// bound keeps the register count of every mode at 40.
+// Six blocks per SM, as before the CTC branch was added: its alpha rows take 32.8 KB of shared memory per block (the
+// errors branch buffers a hypothesis word in the same rows), and the bound keeps the register count of every mode at 40.
 __global__ void __launch_bounds__(256, 6) head_reduce_kernel(const float* __restrict__ logits, const HeadParams p) {
   __shared__ float ctc_alpha[8][CTC_MAX_S];
   const DynArgs d = *p.dyn;
@@ -166,6 +183,19 @@ __global__ void __launch_bounds__(256, 6) head_reduce_kernel(const float* __rest
             return row;
           });
       if (lane == 0) d.out[(long long)b * d.D + dd] = r;
+      continue;
+    }
+    if (d.mode == W2S_OUT_ERRORS) {
+      const int b = (int)(it / d.D), dd = (int)(it - (long long)b * d.D);
+      const float* rows = logits + (long long)b * p.T * p.ldl;
+      const int r = errors_warp<HEAD_MAXJ>(p.T, p.V, d.err_tab, dd, d.err_unit, d.blank, d.delim, lane,
+                                           reinterpret_cast<int*>(ctc_alpha[warp]), [&](int t, float(&lg)[HEAD_MAXJ]) {
+                                             const float* row = rows + (long long)t * p.ldl;
+#pragma unroll
+                                             for (int j = 0; j < HEAD_MAXJ; ++j)
+                                               lg[j] = lane + 32 * j < p.V ? row[lane + 32 * j] : -INFINITY;
+                                           });
+      if (lane == 0) d.out[(long long)b * d.D + dd] = (float)r;
       continue;
     }
     if (d.mode == W2S_OUT_MEAN) {

@@ -55,6 +55,10 @@ struct DynArgs {
   // zbits rows hold one bit per cell, bit s * F + b for time segment s and band b
   const float* bands;
   int F;
+  // recognition errors (w2s_set_references; mode W2S_OUT_ERRORS, D references, blank id `blank`): the tables of
+  // errors.cuh, the unit (W2S_ERR_*) and the word delimiter
+  const int* err_tab;
+  int err_unit, delim;
 };
 
 // ---- K1: conv0 (Cin = 1) + GroupNorm-over-time / LayerNorm-over-channels + GELU ------------------------

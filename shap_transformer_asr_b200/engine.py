@@ -14,7 +14,7 @@ import torch
 from . import _lib
 from .config import ModelConfig
 from .preprocess import pack_coalitions, segment_bounds
-from .targets import PAD_ID, check_offsets, transcript_arrays
+from .targets import PAD_ID, SPACE_ID, check_offsets, transcript_arrays
 
 
 # ModelConfig.kind -> w2s_config.kind and the HF state_dict prefix of the encoder
@@ -288,6 +288,22 @@ class Engine:
         self.transcripts = [labels[a:b].copy() for a, b in zip(offsets[:-1], offsets[1:])]
         self.blank = int(blank)
 
+    def set_references(self, refs, unit: str = "words", blank: int = PAD_ID, delimiter: int = SPACE_ID):
+        """Recognition-error output (w2s_set_references): ``refs`` is a list of D label-id sequences (or one sequence of
+        ints).  Each evaluated row then yields D values, out[r, d] = the edit distance between the row's greedy transcript
+        (per-frame argmax, repeats collapsed, blanks dropped) and reference d, in labels (``unit="labels"``) or in words
+        split on ``delimiter`` (``unit="words"``: WER x N for a reference of N words).  Arguments are validated on the host
+        before the library is called."""
+        labels, offsets = reference_arrays(refs, unit, blank, delimiter, self.config.vocab_size)
+        self._check(self.lib.w2s_set_references(self._h, labels.ctypes.data_as(C.POINTER(C.c_int32)),
+                                                offsets.ctypes.data_as(C.POINTER(C.c_int32)), len(offsets) - 1, int(blank),
+                                                _lib.ERR_UNITS[unit], int(delimiter), self._stream()), "w2s_set_references")
+        self.mode = "errors"
+        self.references = [labels[a:b].copy() for a, b in zip(offsets[:-1], offsets[1:])]
+        self.reference_unit = unit
+        self.reference_blank = int(blank)
+        self.reference_delimiter = int(delimiter)
+
     def out_width(self, num_samples: Optional[int] = None) -> int:
         return int(self.lib.w2s_out_width(self._h, int(num_samples or self.num_samples)))
 
@@ -544,6 +560,50 @@ def debug_ctc(logits: torch.Tensor, transcripts, blank: int = PAD_ID, which=None
     if rc != 0:
         raise RuntimeError("w2s_debug_ctc: " + lib.w2s_last_error(None).decode())
     return (out, dl) if grad else out
+
+
+def reference_arrays(refs, unit: str = "words", blank: int = PAD_ID, delimiter: int = SPACE_ID, vocab_size: int = None):
+    """Validated packed references for ``w2s_set_references``: (labels int32 [sum U], offsets int32 [D + 1]), checked as
+    transcripts are (``targets.transcript_arrays``), plus the unit and, for words, the delimiter in [0, vocab_size) and
+    not the blank.  Raises ValueError before any library call."""
+    if unit not in _lib.ERR_UNITS:
+        raise ValueError(f"unit must be one of {sorted(_lib.ERR_UNITS)}, got {unit!r}")
+    labels, offsets = transcript_arrays(refs, blank, vocab_size)
+    if unit == "words" and (not 0 <= delimiter < (vocab_size if vocab_size is not None else delimiter + 1)
+                            or delimiter == blank):
+        raise ValueError(f"delimiter {delimiter} outside the vocabulary [0, {vocab_size}) or equal to the blank {blank}")
+    return labels, offsets
+
+
+def error_tables(refs, vocab_size: int, unit: str = "words", blank: int = PAD_ID, delimiter: int = SPACE_ID) -> np.ndarray:
+    """The device tables w2s_set_references builds for ``refs`` (host only, no device; layout in include/w2s.h)."""
+    lib = _lib.load()
+    labels, offsets = reference_arrays(refs, unit, blank, delimiter, vocab_size)
+    args = (labels.ctypes.data_as(C.POINTER(C.c_int32)), offsets.ctypes.data_as(C.POINTER(C.c_int32)), len(offsets) - 1,
+            int(vocab_size), int(blank), _lib.ERR_UNITS[unit], int(delimiter))
+    n = lib.w2s_error_tables(*args, None, 0)
+    if n < 0:
+        raise ValueError("w2s_error_tables: bad argument")
+    out = np.zeros(n, dtype=np.int32)
+    lib.w2s_error_tables(*args, out.ctypes.data, n)
+    return out
+
+
+def debug_errors(logits: torch.Tensor, refs, unit: str = "words", blank: int = PAD_ID, delimiter: int = SPACE_ID):
+    """The library's W2S_OUT_ERRORS code on caller logits (tests only): logits fp32 [n, T, V] (CUDA) -> out [n, D], the
+    edit distance between each row's greedy transcript and every reference, through the head reduction kernel."""
+    lib = _lib.load()
+    n, T, V = logits.shape
+    _check_buffer("logits", logits, torch.float32, n * T * V)
+    labels, offsets = reference_arrays(refs, unit, blank, delimiter, V)
+    D = len(offsets) - 1
+    out = torch.empty((n, D), dtype=torch.float32, device=logits.device)
+    rc = lib.w2s_debug_errors(logits.data_ptr(), n, T, V, V, labels.ctypes.data_as(C.POINTER(C.c_int32)),
+                              offsets.ctypes.data_as(C.POINTER(C.c_int32)), D, int(blank), _lib.ERR_UNITS[unit],
+                              int(delimiter), out.data_ptr(), torch.cuda.current_stream().cuda_stream)
+    if rc != 0:
+        raise RuntimeError("w2s_debug_errors: " + lib.w2s_last_error(None).decode())
+    return out
 
 
 def relative_buckets(T: int, num_buckets: int = 320, max_distance: int = 800) -> np.ndarray:

@@ -21,7 +21,7 @@ from . import _lib
 from . import dist as wdist
 from .engine import background_arrays
 from .preprocess import band_components, check_band_edges
-from .targets import MAX_TRANSCRIPT, PAD_ID, char_targets, greedy_transcript
+from .targets import MAX_TRANSCRIPT, PAD_ID, SPACE_ID, char_targets, greedy_transcript, reference_length
 
 
 def unpack_coalitions(words: np.ndarray, M: int) -> np.ndarray:
@@ -180,11 +180,20 @@ class KernelShapExplainer:
         sampled = self._coalitions(num_features or M)
         return logits_dev.view(-1, eng.config.vocab_size).cpu().numpy(), sampled
 
+    def _greedy_target(self, M: int, num_features: int, blank: int, what: str):
+        """-> ([the greedy transcript of the unmasked clip], the sampled coalitions), from one _clip_logits pass"""
+        logits, sampled = self._clip_logits(M, num_features)
+        greedy = greedy_transcript(logits, blank)
+        if greedy.size > MAX_TRANSCRIPT:
+            raise ValueError(f"the greedy transcript of this clip has {greedy.size} labels, more than "
+                             f"W2S_MAX_TRANSCRIPT = {MAX_TRANSCRIPT}: pass the {what} as targets")
+        return [greedy], sampled
+
     def explain(self, clip, num_segments: int, mode: str = "logprob", targets=None, baseline: float = 0.0,
                 check: bool = True, background=None, background_weights=None, blank: int = PAD_ID, band_edges=None,
-                sr: int = 16000):
+                sr: int = 16000, unit: str = "words"):
         """-> dict(phi[M, D] fp64 device, fx, fnull, frames, tokens, Z, weights, y, status, info, background_weights,
-        transcripts, phi_cells, band_edges).
+        transcripts, phi_cells, band_edges, references, reference_lengths).
 
         ``mode="transcript"`` explains whole transcripts: output d is log p_CTC(y_d | clip), the log-likelihood the model
         was trained on (-WavXForCTC(x, labels=y_d).loss, reduction "sum"), with ``blank`` its pad_token_id.  ``targets``
@@ -193,6 +202,14 @@ class KernelShapExplainer:
         result lists them (None in the other modes).  A transcript holds at most W2S_MAX_TRANSCRIPT = 512 labels: when
         the greedy transcript of the clip is longer, explain raises ValueError (pass ``targets`` explicitly, e.g. the
         transcripts of shorter clips).
+
+        ``mode="errors"`` explains recognition errors: output d is the edit distance between the greedy transcript of the
+        (masked) clip and reference d, in ``unit`` "words" (split on the "|" label, targets.SPACE_ID; WER x N) or "labels".
+        ``targets`` is then a list of label-id sequences, e.g. ground-truth transcripts; by default the greedy transcript of
+        the unmasked clip, from the same one-row pass as in transcript mode, so the full coalition scores exactly 0 and phi
+        attributes the errors the masking introduces.  The result's ``references`` lists them and ``reference_lengths`` their
+        N in the unit (divide by N for rates).  Longer references than W2S_MAX_TRANSCRIPT labels are refused as transcripts
+        are.  The engine is left with the references set.
 
         ``check`` reads the solve's status word back (one 4-byte D2H after the solve) and raises if the regression
         did not produce a usable answer; a rank-deficient design (status 2: fewer distinct coalitions than segments)
@@ -239,21 +256,22 @@ class KernelShapExplainer:
         M = eng.num_segments
         Mf = M if edges is None else M * (edges.size - 1)     # features: segments, or time-frequency cells
         sampled = None
-        transcripts = None
+        transcripts = references = None
         if mode in ("max", "mean", "logits"):
             frames, tokens = (), ()
             eng.set_targets(mode)
         elif mode == "transcript":
             frames, tokens = (), ()
             if targets is None:
-                logits, sampled = self._clip_logits(M, Mf)
-                greedy = greedy_transcript(logits, blank)
-                if greedy.size > MAX_TRANSCRIPT:
-                    raise ValueError(f"the greedy transcript of this clip has {greedy.size} labels, more than "
-                                     f"W2S_MAX_TRANSCRIPT = {MAX_TRANSCRIPT}: pass the transcripts as targets")
-                targets = [greedy]
+                targets, sampled = self._greedy_target(M, Mf, blank, "transcripts")
             eng.set_transcripts(targets, blank)
             transcripts = eng.transcripts
+        elif mode == "errors":
+            frames, tokens = (), ()
+            if targets is None:
+                targets, sampled = self._greedy_target(M, Mf, blank, "references")
+            eng.set_references(targets, unit=unit, blank=blank, delimiter=SPACE_ID)
+            references = eng.references
         elif targets is None:
             logits, sampled = self._clip_logits(M, Mf)
             frames, tokens = char_targets(logits)
@@ -299,7 +317,9 @@ class KernelShapExplainer:
         phi_cells = None if edges is None else phi.view(M, edges.size - 1, phi.shape[1])
         return dict(phi=phi, fx=fx, fnull=fnull, frames=frames, tokens=tokens, Z=unpack_coalitions(words, Mf), weights=kw,
                     y=y_all[2:], status=status, info=info, words=words, background_weights=bg_w, transcripts=transcripts,
-                    phi_cells=phi_cells, band_edges=edges)
+                    phi_cells=phi_cells, band_edges=edges, references=references,
+                    reference_lengths=None if references is None else
+                    [reference_length(r, unit, SPACE_ID) for r in references])
 
 
 def kmeans_background(X, k: int, round_values: bool = True):

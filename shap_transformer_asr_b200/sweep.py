@@ -16,6 +16,7 @@ import numpy as np
 from .kernelshap import KernelShapExplainer, expand_to_samples
 from .metrics import greedy_ctc_decode
 from .preprocess import normalize_clip, synthetic_clip
+from .targets import greedy_transcript
 
 
 def add_noise(audio: np.ndarray, snr_db: float, rng: np.random.Generator) -> np.ndarray:
@@ -53,7 +54,12 @@ def explain_test_set(engine, test_set: List[Dict], out_dir: str = "data", num_se
     ``background``: passed to every ``KernelShapExplainer.explain`` call -- an array [B, L] or a ``(data, weights)`` pair,
     e.g. the reference's noise background ``make_background(L, 5, seed)`` (shap_calculation.py:125-127) -- so the
     KernelSHAP attributions are taken against the same background as the expected-gradients ones; None fills the dropped
-    segments with zeros."""
+    segments with zeros.
+
+    ``mode="errors"`` explains each item's word errors against its text, kept as label ids (the clean item's greedy
+    transcript): the attributions of a noisy item then locate the audio that caused its WER.  The result of an item adds
+    ``errors``, the device's word-error count of the unmasked item (``wer(text, hypothesis) * reference_words``), and
+    ``reference_words``.  Items must come without a text of their own in this mode."""
     os.makedirs(out_dir, exist_ok=True)
     explainer = KernelShapExplainer(engine, nsamples=nsamples, seed=seed, shard_coalitions=False)
     results, clean_text = [], None
@@ -65,12 +71,16 @@ def explain_test_set(engine, test_set: List[Dict], out_dir: str = "data", num_se
         logits = engine.eval_bits(ones).view(-1, engine.config.vocab_size).cpu().numpy()
         hyp = greedy_ctc_decode(logits.argmax(-1))
         if item["type"] == "clean":
-            clean_text = hyp
+            clean_text, clean_ids = hyp, greedy_transcript(logits)
         text = item["text"] if item["text"] is not None else clean_text
         T = logits.shape[0]
-        targets = None if mode == "max" else (np.arange(T, dtype=np.int32), logits.argmax(-1).astype(np.int32))
-        res = explainer.explain(x, num_segments=num_segments, mode=mode, targets=targets if mode != "max" else ((), ()),
-                                background=background)
+        if mode == "errors":
+            if item["text"] is not None:
+                raise ValueError("mode='errors' explains against the clean item's greedy transcript: items carry no text")
+            targets = [clean_ids]
+        else:
+            targets = ((), ()) if mode == "max" else (np.arange(T, dtype=np.int32), logits.argmax(-1).astype(np.int32))
+        res = explainer.explain(x, num_segments=num_segments, mode=mode, targets=targets, background=background)
         phi = res["phi"].cpu().numpy()
         tag = f"sample_{i + 1}_{item['type']}_{item['snr']}"
         saved = save_limit is None or i < save_limit
@@ -83,6 +93,8 @@ def explain_test_set(engine, test_set: List[Dict], out_dir: str = "data", num_se
             np.save(os.path.join(out_dir, f"text_{tag}.npy"), text)
         results.append(dict(tag=tag, hypothesis=hyp, text=text, shap_shape=shape, saved=saved,
                             status=int(res["status"].item())))
+        if mode == "errors":
+            results[-1].update(errors=float(res["fx"][0].item()), reference_words=res["reference_lengths"][0])
         if on_item is not None:
             on_item(i, item, phi, np.asarray(engine.bounds), results[-1])
     return results

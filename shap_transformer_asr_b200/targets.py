@@ -18,6 +18,16 @@ def greedy_transcript(logits, blank: int = PAD_ID) -> np.ndarray:
     return ids[keep].astype(np.int32)
 
 
+def reference_length(ref, unit: str = "words", delimiter: int = SPACE_ID) -> int:
+    """Units N of a reference of the recognition-error output: its labels, or its words -- the runs between
+    ``delimiter`` labels, empty ones dropped.  Error counts divided by N are the label or word error rates."""
+    y = np.asarray(ref).reshape(-1)
+    if unit == "labels":
+        return int(y.size)
+    word = y != delimiter
+    return int(np.count_nonzero(word[1:] & ~word[:-1]) + (word.size > 0 and word[0]))
+
+
 def frames_needed(transcript) -> int:
     """Frames a CTC alignment of ``transcript`` needs: one per label plus one blank between equal adjacent labels."""
     y = np.asarray(transcript).reshape(-1)
