@@ -124,7 +124,7 @@ struct w2s_handle {
   float baseline = 0.f;
   float* clip = nullptr;
   uint16_t* seg_id = nullptr;
-  long long clip_cap = 0;
+  long long clip_cap = 0, seg_id_cap = 0;   // elements
 
   // background (w2s_set_background): bg_B rows of bg_L samples replace the baseline; bg_B == 0: none
   int bg_B = 0;
@@ -144,14 +144,14 @@ struct w2s_handle {
 
   // targets
   int mode = W2S_OUT_MAX, D = 0, max_frame = 0;
-  int *frames = nullptr, *tokens = nullptr;
-  int targets_cap = 0;
+  int* targets = nullptr;              // [2 D]: the D target frames, then the D tokens
+  long long targets_cap = 0;           // ints
   std::vector<int32_t> targets_host;   // staging of the last w2s_set_targets arrays (source of the async upload)
 
   // transcripts (w2s_set_transcripts): kept across w2s_set_targets, so the gradient entry can use them in any mode
   int ctc_D = 0, ctc_blank = 0, ctc_smax = 1;   // count, blank id, largest 2U + 1
   int *ctc_labels = nullptr, *ctc_offsets = nullptr;
-  int ctc_labels_cap = 0, ctc_offsets_cap = 0;
+  long long ctc_labels_cap = 0, ctc_offsets_cap = 0;
   std::vector<int32_t> ctc_host;        // staging of the upload: offsets [D + 1], then the labels
   std::vector<int> ctc_need;            // frames each transcript needs
   float *ctc_alpha = nullptr, *ctc_lse = nullptr, *ctc_dz = nullptr;   // gradient-seed scratch, grown on demand
@@ -246,8 +246,7 @@ struct w2s_handle {
     if (bg_w) cudaFree(bg_w);
     if (bg_rows) cudaFree(bg_rows);
     if (bands) cudaFree(bands);
-    if (frames) cudaFree(frames);
-    if (tokens) cudaFree(tokens);
+    if (targets) cudaFree(targets);
     for (void* p : {(void*)ctc_labels, (void*)ctc_offsets, (void*)ctc_alpha, (void*)ctc_lse, (void*)ctc_dz, (void*)err_tab})
       if (p) cudaFree(p);
     if (wls_work) cudaFree(wls_work);
@@ -266,6 +265,25 @@ std::string dalloc(std::vector<void*>& pool, T** out, size_t count, bool zero = 
   if (zero) W2S_CUDA_OK(cudaMemset(p, 0, bytes));
   pool.push_back(p);
   *out = reinterpret_cast<T*>(p);
+  return "";
+}
+
+// Grow-on-demand device buffer: afterwards *p holds at least `need` elements, max(need, min_cap) when it had to grow.
+// Work queued on s may still read the old buffer, so s is synchronised before it is freed; a failed allocation leaves
+// *p == nullptr and *cap == 0, not a dangling pointer.  Errors: "stream error", "out of device memory".
+template <typename T>
+std::string grow(T** p, long long* cap, long long need, long long min_cap, cudaStream_t s) {
+  if (*cap >= need) return "";
+  if (cudaStreamSynchronize(s) != cudaSuccess) return "stream error";
+  if (*p) cudaFree(*p);
+  *p = nullptr;
+  *cap = 0;
+  const long long n = std::max(need, min_cap);
+  if (cudaMalloc((void**)p, sizeof(T) * n) != cudaSuccess) {
+    *p = nullptr;
+    return "out of device memory";
+  }
+  *cap = n;
   return "";
 }
 
@@ -1042,15 +1060,21 @@ std::string get_plan(w2s_handle* h, int n, int fill, Plan** out) {
   return "";
 }
 
+// D of the current mode: transcripts (CTC), references (ERRORS) or (frame, token) targets (LOGIT / LOGPROB; 0 otherwise)
+int out_count(const w2s_handle* h) {
+  return h->mode == W2S_OUT_CTC ? h->ctc_D : h->mode == W2S_OUT_ERRORS ? h->err_D : h->D;
+}
+
+// blank id of the current mode: that of the references (ERRORS), else that of the transcripts
+int out_blank(const w2s_handle* h) { return h->mode == W2S_OUT_ERRORS ? h->err_blank : h->ctc_blank; }
+
 int64_t out_width(const w2s_handle* h, int64_t L) {
   const int64_t T = num_frames(h->cfg, L, nullptr);
   switch (h->mode) {
     case W2S_OUT_MAX: return T;
     case W2S_OUT_MEAN: return 1;
     case W2S_OUT_LOGITS: return T * h->cfg.vocab_size;
-    case W2S_OUT_CTC: return h->ctc_D;
-    case W2S_OUT_ERRORS: return h->err_D;
-    default: return h->D;
+    default: return out_count(h);
   }
 }
 
@@ -1124,15 +1148,7 @@ std::string run_batches(w2s_handle* h, const uint32_t* zbits, const float* x, lo
                     (h->cfg.flags & (W2S_FLAG_DENSE_FRONTEND | W2S_FLAG_VALIDATE_GEMM)) == 0;
   float* dst = out;
   if (bg) {
-    const long long need = rows * width;
-    if (h->bg_rows_cap < need) {
-      W2S_CUDA_OK(cudaStreamSynchronize(s));   // evaluations in flight may still write the old scratch
-      if (h->bg_rows) cudaFree(h->bg_rows);
-      h->bg_rows = nullptr;
-      h->bg_rows_cap = 0;
-      W2S_CUDA_OK(cudaMalloc((void**)&h->bg_rows, sizeof(float) * need));
-      h->bg_rows_cap = need;
-    }
+    W2S_TRY(grow(&h->bg_rows, &h->bg_rows_cap, rows * width, 0, s));
     dst = h->bg_rows;
   }
   for (int64_t k0 = 0; k0 < rows; k0 += h->cfg.max_batch) {
@@ -1153,10 +1169,10 @@ std::string run_batches(w2s_handle* h, const uint32_t* zbits, const float* x, lo
       d.x = x + k0 * ld; d.ld = ld;
     }
     d.out = dst + k0 * width;
-    d.mode = h->mode; d.D = h->mode == W2S_OUT_CTC ? h->ctc_D : h->mode == W2S_OUT_ERRORS ? h->err_D : h->D;
-    d.frames = h->frames; d.tokens = h->tokens;
+    d.mode = h->mode; d.D = out_count(h);
+    d.frames = h->targets; d.tokens = h->targets ? h->targets + h->D : nullptr;
     d.ctc_labels = h->ctc_labels; d.ctc_offsets = h->ctc_offsets;
-    d.blank = h->mode == W2S_OUT_ERRORS ? h->err_blank : h->ctc_blank;
+    d.blank = out_blank(h);
     d.err_tab = h->err_tab; d.err_unit = h->err_unit; d.delim = h->err_delim;
     set_dyn_kernel<<<1, 1, 0, s>>>(h->dyn_dev, d);
     W2S_CUDA_OK(cudaGetLastError());
@@ -1204,7 +1220,7 @@ std::string check_bands(const w2s_handle* h) {
 std::string check_targets(const w2s_handle* h) {
   if (h->mode == W2S_OUT_CTC) return check_transcripts(h, h->T);
   if (h->mode == W2S_OUT_LOGIT || h->mode == W2S_OUT_LOGPROB) {
-    if (h->D <= 0 || !h->frames || !h->tokens) return "targets not set (w2s_set_targets)";
+    if (out_count(h) <= 0 || !h->targets) return "targets not set (w2s_set_targets)";
     if (h->max_frame >= h->T)
       return "target frame " + std::to_string(h->max_frame) + " beyond the clip's " + std::to_string(h->T) + " frames";
   }
@@ -1319,6 +1335,45 @@ AttnParams debug_attn_params(const void* qkv, const void* pos_proj, int B, int T
   return ap;
 }
 
+// Device buffers of one w2s_debug_* call.  release() waits for the work queued on s, frees them all and returns the
+// stream's error, or "".
+struct CallScratch {
+  cudaStream_t s;
+  std::vector<void*> ptrs;
+  template <typename T>
+  bool alloc(T** p, size_t count) {
+    if (cudaMalloc((void**)p, sizeof(T) * count) != cudaSuccess) {
+      *p = nullptr;
+      return false;
+    }
+    ptrs.push_back(*p);
+    return true;
+  }
+  std::string release() {
+    const cudaError_t se = cudaStreamSynchronize(s);
+    for (void* p : ptrs) cudaFree(p);
+    ptrs.clear();
+    return se == cudaSuccess ? "" : cudaGetErrorString(se);
+  }
+};
+
+// head_reduce_kernel on caller logits [n, T, ldl] for the w2s_debug_* entries: d, whose tables are already on the
+// device, travels in an argument block of the call's scratch
+std::string debug_head_reduce(const float* logits, int n, int T, int V, int ldl, const DynArgs& d, CallScratch& sc) {
+  DynArgs* dyn = nullptr;
+  if (!sc.alloc(&dyn, 1)) return "out of device memory";
+  if (cudaMemcpyAsync(dyn, &d, sizeof(DynArgs), cudaMemcpyHostToDevice, sc.s) != cudaSuccess) return "copy failed";
+  HeadParams hp{};
+  hp.n = n; hp.T = T; hp.V = V; hp.ldl = ldl; hp.dyn = dyn;
+  return launch_head_reduce(logits, hp, sc.s);
+}
+
+// result of a w2s_debug_* entry: its error goes where w2s_last_error(NULL) reads it
+int debug_result(const std::string& e) {
+  g_create_error = e;
+  return e.empty() ? 0 : 1;
+}
+
 }  // namespace
 
 // =================================================================================================
@@ -1421,14 +1476,9 @@ int w2s_set_clip(w2s_handle* h, const float* x_dev, int64_t L, const int32_t* se
   }
   std::string e = ensure_workspace(h, L);
   if (!e.empty()) return fail(h, e);
-  if (h->clip_cap < L) {
-    if (h->clip) cudaFree(h->clip);
-    if (h->seg_id) cudaFree(h->seg_id);
-    if (cudaMalloc((void**)&h->clip, sizeof(float) * (L + 16)) != cudaSuccess ||
-        cudaMalloc((void**)&h->seg_id, sizeof(uint16_t) * (L + 16)) != cudaSuccess)
-      return fail(h, "set_clip: out of device memory");
-    h->clip_cap = L;
-  }
+  e = grow(&h->clip, &h->clip_cap, L + 16, 0, s);
+  if (e.empty()) e = grow(&h->seg_id, &h->seg_id_cap, L + 16, 0, s);
+  if (!e.empty()) return fail(h, "set_clip: " + e);
   if (cudaMemcpyAsync(h->clip, x_dev, sizeof(float) * L, cudaMemcpyDeviceToDevice, s) != cudaSuccess ||
       cudaMemcpyAsync(h->seg_id, seg.data(), sizeof(uint16_t) * L, cudaMemcpyHostToDevice, s) != cudaSuccess ||
       cudaStreamSynchronize(s) != cudaSuccess)
@@ -1474,13 +1524,9 @@ int w2s_set_background(w2s_handle* h, const float* bg_dev, int64_t B, int64_t L,
   if (!(sum > 0.0) || !std::isfinite(sum)) return fail(h, "set_background: the weights sum to zero");
   // evaluations in flight on the stream still read the old rows and weights
   if (cudaStreamSynchronize(s) != cudaSuccess) return fail(h, "set_background: stream error");
-  if (h->bg_cap < B * L) {
-    if (h->bg) cudaFree(h->bg);
-    h->bg = nullptr;
-    h->bg_cap = 0;
-    if (cudaMalloc((void**)&h->bg, sizeof(float) * B * L) != cudaSuccess) return fail(h, "set_background: out of device memory");
-    h->bg_cap = B * L;
-  }
+  h->bg_B = 0;   // a failed allocation or copy below leaves no background set, not a dangling one
+  const std::string e = grow(&h->bg, &h->bg_cap, B * L, 0, s);
+  if (!e.empty()) return fail(h, "set_background: " + e);
   if (!h->bg_w && cudaMalloc((void**)&h->bg_w, sizeof(float) * W2S_MAX_BACKGROUND) != cudaSuccess)
     return fail(h, "set_background: out of device memory");
   h->bg_w_host.resize((size_t)B);
@@ -1518,14 +1564,9 @@ int w2s_set_bands(w2s_handle* h, const float* comp_dev, int64_t F, int64_t L, in
                        std::to_string((long long)h->M * F) + " cells; at most 2048 are supported");
   // evaluations in flight on the stream still read the old components
   if (cudaStreamSynchronize(s) != cudaSuccess) return fail(h, "set_bands: stream error");
-  if (h->bands_cap < F * L) {
-    h->bands_F = 0;   // the old buffer goes now: a failed allocation leaves no bands set, not dangling ones
-    if (h->bands) cudaFree(h->bands);
-    h->bands = nullptr;
-    h->bands_cap = 0;
-    if (cudaMalloc((void**)&h->bands, sizeof(float) * F * L) != cudaSuccess) return fail(h, "set_bands: out of device memory");
-    h->bands_cap = F * L;
-  }
+  h->bands_F = 0;   // a failed allocation or copy below leaves no bands set, not dangling ones
+  const std::string e = grow(&h->bands, &h->bands_cap, F * L, 0, s);
+  if (!e.empty()) return fail(h, "set_bands: " + e);
   if (cudaMemcpy2DAsync(h->bands, sizeof(float) * L, comp_dev, sizeof(float) * ld, sizeof(float) * L, (size_t)F,
                         cudaMemcpyDeviceToDevice, s) != cudaSuccess ||
       cudaStreamSynchronize(s) != cudaSuccess)
@@ -1544,25 +1585,13 @@ int w2s_set_targets(w2s_handle* h, const int32_t* frame_idx_host, const int32_t*
     for (int d = 0; d < D; ++d)
       if (token_idx_host[d] < 0 || token_idx_host[d] >= h->cfg.vocab_size || frame_idx_host[d] < 0)
         return fail(h, "set_targets: target out of range");
-    if (h->targets_cap < D) {
-      // evaluations in flight on the stream still read the old arrays
-      if (cudaStreamSynchronize(s) != cudaSuccess) return fail(h, "set_targets: stream error");
-      if (h->frames) cudaFree(h->frames);
-      if (h->tokens) cudaFree(h->tokens);
-      h->frames = h->tokens = nullptr;
-      h->targets_cap = 0;
-      const int cap = D < 1024 ? 1024 : D;
-      if (cudaMalloc((void**)&h->frames, sizeof(int) * cap) != cudaSuccess ||
-          cudaMalloc((void**)&h->tokens, sizeof(int) * cap) != cudaSuccess)
-        return fail(h, "set_targets: out of device memory");
-      h->targets_cap = cap;
-    }
+    const std::string e = grow(&h->targets, &h->targets_cap, 2LL * D, 2 * 1024, s);
+    if (!e.empty()) return fail(h, "set_targets: " + e);
     // ordered on the caller's stream behind any evaluation still running with the previous targets; the host arrays
     // are staged in the handle so the caller's buffers may be released when this returns
     h->targets_host.assign(frame_idx_host, frame_idx_host + D);
     h->targets_host.insert(h->targets_host.end(), token_idx_host, token_idx_host + D);
-    if (cudaMemcpyAsync(h->frames, h->targets_host.data(), sizeof(int) * D, cudaMemcpyHostToDevice, s) != cudaSuccess ||
-        cudaMemcpyAsync(h->tokens, h->targets_host.data() + D, sizeof(int) * D, cudaMemcpyHostToDevice, s) != cudaSuccess)
+    if (cudaMemcpyAsync(h->targets, h->targets_host.data(), sizeof(int) * 2 * D, cudaMemcpyHostToDevice, s) != cudaSuccess)
       return fail(h, "set_targets: copy failed");
     h->D = D;
     h->max_frame = 0;
@@ -1582,27 +1611,10 @@ int w2s_set_transcripts(w2s_handle* h, const int32_t* labels_host, const int32_t
   if (!e.empty()) return fail(h, "set_transcripts: " + e);
   const int total = offsets_host[D];
   const int label_slots = total > 0 ? total : 1;   // all transcripts empty: the kernels still take a valid pointer
-  if (h->ctc_offsets_cap < D + 1 || h->ctc_labels_cap < label_slots) {
-    // evaluations in flight on the stream still read the old arrays
-    if (cudaStreamSynchronize(s) != cudaSuccess) return fail(h, "set_transcripts: stream error");
-    h->ctc_D = 0;   // the old arrays go now: a failed allocation below leaves no transcripts set, not dangling ones
-    if (h->ctc_offsets_cap < D + 1) {
-      if (h->ctc_offsets) cudaFree(h->ctc_offsets);
-      h->ctc_offsets = nullptr;
-      h->ctc_offsets_cap = 0;
-      const int cap = D + 1 < 64 ? 64 : D + 1;
-      if (cudaMalloc((void**)&h->ctc_offsets, sizeof(int) * cap) != cudaSuccess) return fail(h, "set_transcripts: out of device memory");
-      h->ctc_offsets_cap = cap;
-    }
-    if (h->ctc_labels_cap < label_slots) {
-      if (h->ctc_labels) cudaFree(h->ctc_labels);
-      h->ctc_labels = nullptr;
-      h->ctc_labels_cap = 0;
-      const int cap = total < 1024 ? 1024 : total;
-      if (cudaMalloc((void**)&h->ctc_labels, sizeof(int) * cap) != cudaSuccess) return fail(h, "set_transcripts: out of device memory");
-      h->ctc_labels_cap = cap;
-    }
-  }
+  h->ctc_D = 0;   // a failed allocation or copy below leaves no transcripts set, not dangling ones
+  std::string ge = grow(&h->ctc_offsets, &h->ctc_offsets_cap, D + 1, 64, s);
+  if (ge.empty()) ge = grow(&h->ctc_labels, &h->ctc_labels_cap, label_slots, 1024, s);
+  if (!ge.empty()) return fail(h, "set_transcripts: " + ge);
   // ordered on the caller's stream, staged in the handle (as w2s_set_targets)
   h->ctc_host.assign(offsets_host, offsets_host + D + 1);
   h->ctc_host.insert(h->ctc_host.end(), labels_host, labels_host + total);
@@ -1628,17 +1640,9 @@ int w2s_set_references(w2s_handle* h, const int32_t* labels_host, const int32_t*
   std::vector<int32_t> tab;
   const std::string e = error_tables(labels_host, offsets_host, D, h->cfg.vocab_size, blank, unit, delimiter, &tab);
   if (!e.empty()) return fail(h, "set_references: " + e);
-  if (h->err_tab_cap < (long long)tab.size()) {
-    // evaluations in flight on the stream still read the old tables
-    if (cudaStreamSynchronize(s) != cudaSuccess) return fail(h, "set_references: stream error");
-    h->err_D = 0;   // a failed allocation below leaves no references set, not dangling ones
-    if (h->err_tab) cudaFree(h->err_tab);
-    h->err_tab = nullptr;
-    h->err_tab_cap = 0;
-    const long long cap = std::max<long long>((long long)tab.size(), 4096);
-    if (cudaMalloc((void**)&h->err_tab, sizeof(int) * cap) != cudaSuccess) return fail(h, "set_references: out of device memory");
-    h->err_tab_cap = cap;
-  }
+  h->err_D = 0;   // a failed allocation or copy below leaves no references set, not dangling ones
+  const std::string ge = grow(&h->err_tab, &h->err_tab_cap, (long long)tab.size(), 4096, s);
+  if (!ge.empty()) return fail(h, "set_references: " + ge);
   // ordered on the caller's stream, staged in the handle (as w2s_set_targets)
   h->err_host = std::move(tab);
   if (cudaMemcpyAsync(h->err_tab, h->err_host.data(), sizeof(int) * h->err_host.size(), cudaMemcpyHostToDevice, s) !=
@@ -1779,20 +1783,15 @@ int w2s_mask(w2s_handle* h, const uint32_t* z_bits_dev, int64_t K, float* out_de
 int w2s_wls(w2s_handle* h, const uint32_t* z_bits_dev, const double* w_dev, const float* y_dev, int64_t K, int M,
             int D, const double* fx_dev, const double* fnull_dev, double* phi_dev, int32_t* status_dev, void* stream) {
   const long long need = 2 * ((long long)(M - 1) * (M - 1) + (long long)(M - 1) * D);
-  if (h->wls_cap < need) {
-    cudaStreamSynchronize((cudaStream_t)stream);
-    if (h->wls_work) cudaFree(h->wls_work);
-    if (cudaMalloc((void**)&h->wls_work, sizeof(double) * need) != cudaSuccess) return fail(h, "wls: out of device memory");
-    h->wls_cap = need;
-  }
-  std::string e = launch_wls(z_bits_dev, (M + 31) / 32, w_dev, y_dev, K, M, D, fx_dev, fnull_dev, phi_dev, status_dev,
-                             h->wls_work, (cudaStream_t)stream);
+  std::string e = grow(&h->wls_work, &h->wls_cap, need, 0, (cudaStream_t)stream);
+  if (!e.empty()) return fail(h, "wls: " + e);
+  e = launch_wls(z_bits_dev, (M + 31) / 32, w_dev, y_dev, K, M, D, fx_dev, fnull_dev, phi_dev, status_dev, h->wls_work,
+                 (cudaStream_t)stream);
   return e.empty() ? 0 : fail(h, e);
 }
 
 int w2s_debug_gemm(int use_tcgen05, const void* a_bf16, const void* w_bf16, const float* bias, const void* residual,
                    int res_fp32, float alpha, void* out, int M, int N, int K, int act, int out_fp32, void* stream) {
-  g_create_error.clear();
   std::string e = gemm_init();
   if (e.empty()) {
     GemmProblem p = PlanBuilder::plain((const bf16*)a_bf16, M, K, (const bf16*)w_bf16, N);
@@ -1802,16 +1801,11 @@ int w2s_debug_gemm(int use_tcgen05, const void* a_bf16, const void* w_bf16, cons
     e = gemm_prepare(p, debug_num_sms(), &gl);
     if (e.empty()) e = use_tcgen05 ? gemm_launch_tc(gl, (cudaStream_t)stream) : gemm_launch_simt(gl, (cudaStream_t)stream);
   }
-  if (!e.empty()) {
-    g_create_error = e;
-    return 1;
-  }
-  return 0;
+  return debug_result(e);
 }
 
 int w2s_debug_attention(int use_tcgen05, const void* qkv, const void* pos_proj, int B, int T, int heads, float scale,
                         void* ctx, float* lse, void* stream) {
-  g_create_error.clear();
   const cudaStream_t s = (cudaStream_t)stream;
   AttnParams ap = debug_attn_params(qkv, pos_proj, B, T, heads, scale);
   ap.ctx = (bf16*)ctx;
@@ -1838,27 +1832,23 @@ int w2s_debug_attention(int use_tcgen05, const void* qkv, const void* pos_proj, 
     if (e.empty()) e = attention_fa_launch(fp, s);
     if (fp) attention_fa_free(fp);
   }
-  if (!e.empty()) {
-    g_create_error = e;
-    return 1;
-  }
-  return 0;
+  return debug_result(e);
 }
 
 int w2s_debug_attention_bias(int use_tcgen05, const void* qkv, const float* rel_bias, const float* gate, int B, int T,
                              int heads, float scale, void* ctx, float* lse, void* stream) {
-  g_create_error.clear();
   const cudaStream_t s = (cudaStream_t)stream;
   AttnParams ap = debug_attn_params(qkv, nullptr, B, T, heads, scale);
   ap.ctx = (bf16*)ctx;
   ap.gate = gate;
   std::string e;
+  CallScratch sc{s};
   float* table = nullptr;
   if (B <= 0 || T <= 0 || heads <= 0 || !qkv || !ctx || !rel_bias || !gate) {
     e = "debug_attention_bias: need B, T', heads >= 1 and qkv / rel_bias / gate / ctx buffers";
   } else if (lse) {
     e = "debug_attention_bias: the relative-position bias variant writes no log-sum-exp (lse must be NULL)";
-  } else if (cudaMalloc((void**)&table, sizeof(float) * heads * rel_bias_ld(T)) != cudaSuccess) {
+  } else if (!sc.alloc(&table, (size_t)heads * rel_bias_ld(T))) {
     e = "debug_attention_bias: out of device memory";
   } else if (!(e = launch_rel_bias_table(rel_bias, nullptr, T, heads, table, s)).empty()) {
   } else if (!(e = gemm_init()).empty()) {
@@ -1874,27 +1864,21 @@ int w2s_debug_attention_bias(int use_tcgen05, const void* qkv, const float* rel_
       if (fp) attention_fa_free(fp);
     }
   }
-  // the table lives for this call only
-  const cudaError_t se = cudaStreamSynchronize(s);
-  if (se != cudaSuccess && e.empty()) e = std::string("debug_attention_bias: ") + cudaGetErrorString(se);
-  if (table) cudaFree(table);
-  if (!e.empty()) {
-    g_create_error = e;
-    return 1;
-  }
-  return 0;
+  const std::string se = sc.release();
+  if (e.empty() && !se.empty()) e = "debug_attention_bias: " + se;
+  return debug_result(e);
 }
 
 int w2s_debug_attention_bwd(int use_tcgen05, const void* qkv, const void* ctx, const void* dctx, const float* lse, int B,
                             int T, int heads, float scale, void* dqkv, void* stream) {
-  g_create_error.clear();
   const cudaStream_t s = (cudaStream_t)stream;
   const AttnParams ap = debug_attn_params(qkv, nullptr, B, T, heads, scale);
   const long long rows = (long long)B * T;
   std::string e;
+  CallScratch sc{s};
   float *delta = nullptr, *dq = nullptr, *stats = nullptr;
   auto dalloc = [&](float** p, size_t n) {
-    if (e.empty() && cudaMalloc((void**)p, sizeof(float) * n) != cudaSuccess) e = "debug_attention_bwd: out of device memory";
+    if (e.empty() && !sc.alloc(p, n)) e = "debug_attention_bwd: out of device memory";
   };
   if (B <= 0 || T <= 0 || heads <= 0 || !qkv || !dctx || !dqkv) {
     e = "debug_attention_bwd: need B, T', heads >= 1 and qkv / dctx / dqkv buffers";
@@ -1912,21 +1896,13 @@ int w2s_debug_attention_bwd(int use_tcgen05, const void* qkv, const void* ctx, c
     dalloc(&stats, (size_t)rows * heads * 3);
     if (e.empty()) e = launch_attn_bwd(ap.qkv, (const bf16*)dctx, B, T, ap.H, heads, scale, (bf16*)dqkv, stats, s);
   }
-  // the workspace lives for this call only
-  const cudaError_t se = cudaStreamSynchronize(s);
-  if (se != cudaSuccess && e.empty()) e = std::string("debug_attention_bwd: ") + cudaGetErrorString(se);
-  for (float* p : {delta, dq, stats})
-    if (p) cudaFree(p);
-  if (!e.empty()) {
-    g_create_error = e;
-    return 1;
-  }
-  return 0;
+  const std::string se = sc.release();
+  if (e.empty() && !se.empty()) e = "debug_attention_bwd: " + se;
+  return debug_result(e);
 }
 
 int w2s_debug_ctc(const float* logits, int n, int T, int V, int ldl, const int32_t* labels_host, const int32_t* offsets_host,
                   int D, int blank, const int32_t* which_host, float* out_dev, float* dlogits_dev, void* stream) {
-  g_create_error.clear();
   const cudaStream_t s = (cudaStream_t)stream;
   std::vector<int> need;
   std::string e;
@@ -1942,53 +1918,37 @@ int w2s_debug_ctc(const float* logits, int n, int T, int V, int ldl, const int32
     const int total = offsets_host[D];
     int smax = 1;
     for (int d = 0; d < D; ++d) smax = std::max(smax, 2 * (offsets_host[d + 1] - offsets_host[d]) + 1);
+    CallScratch sc{s};
     int *lab = nullptr, *off = nullptr, *wh = nullptr;
-    DynArgs* dyn = nullptr;
     float *alpha = nullptr, *lse = nullptr, *val = nullptr;
-    auto al = [&](void** p, size_t bytes) {
-      if (e.empty() && cudaMalloc(p, bytes) != cudaSuccess) e = "debug_ctc: out of device memory";
-    };
-    al((void**)&lab, sizeof(int) * (total + 1));
-    al((void**)&off, sizeof(int) * (D + 1));
-    al((void**)&wh, sizeof(int) * n);
-    al((void**)&dyn, sizeof(DynArgs));
-    DynArgs d{};
-    d.out = out_dev; d.mode = W2S_OUT_CTC; d.D = D; d.ctc_labels = lab; d.ctc_offsets = off; d.blank = blank;
-    if (e.empty() && (cudaMemcpyAsync(off, offsets_host, sizeof(int) * (D + 1), cudaMemcpyHostToDevice, s) != cudaSuccess ||
-                      (total && cudaMemcpyAsync(lab, labels_host, sizeof(int) * total, cudaMemcpyHostToDevice, s) != cudaSuccess) ||
-                      cudaMemcpyAsync(dyn, &d, sizeof(DynArgs), cudaMemcpyHostToDevice, s) != cudaSuccess))
-      e = "debug_ctc: copy failed";
+    if (!sc.alloc(&lab, total + 1) || !sc.alloc(&off, D + 1) || !sc.alloc(&wh, n))
+      e = "out of device memory";
+    else if (cudaMemcpyAsync(off, offsets_host, sizeof(int) * (D + 1), cudaMemcpyHostToDevice, s) != cudaSuccess ||
+             (total && cudaMemcpyAsync(lab, labels_host, sizeof(int) * total, cudaMemcpyHostToDevice, s) != cudaSuccess))
+      e = "copy failed";
     if (e.empty()) {
-      HeadParams hp{};
-      hp.n = n; hp.T = T; hp.V = V; hp.ldl = ldl; hp.dyn = dyn;
-      e = launch_head_reduce(logits, hp, s);
+      DynArgs d{};
+      d.out = out_dev; d.mode = W2S_OUT_CTC; d.D = D; d.ctc_labels = lab; d.ctc_offsets = off; d.blank = blank;
+      e = debug_head_reduce(logits, n, T, V, ldl, d, sc);
     }
     if (e.empty() && dlogits_dev) {
-      al((void**)&alpha, sizeof(float) * (size_t)n * T * smax);
-      al((void**)&lse, sizeof(float) * (size_t)n * T);
-      al((void**)&val, sizeof(float) * (size_t)n);
-      if (e.empty() && cudaMemcpyAsync(wh, which_host, sizeof(int) * n, cudaMemcpyHostToDevice, s) != cudaSuccess)
-        e = "debug_ctc: copy failed";
+      if (!sc.alloc(&alpha, (size_t)n * T * smax) || !sc.alloc(&lse, (size_t)n * T) || !sc.alloc(&val, n))
+        e = "out of device memory";
+      else if (cudaMemcpyAsync(wh, which_host, sizeof(int) * n, cudaMemcpyHostToDevice, s) != cudaSuccess)
+        e = "copy failed";
       if (e.empty())
         e = launch_ctc_seed(logits, ldl, V, nullptr, n, T, 0, lab, off, wh, blank, smax, alpha, lse, dlogits_dev, V, nullptr,
                             val, s);
     }
-    // the buffers live for this call only
-    const cudaError_t se = cudaStreamSynchronize(s);
-    if (se != cudaSuccess && e.empty()) e = std::string("debug_ctc: ") + cudaGetErrorString(se);
-    for (void* p : {(void*)lab, (void*)off, (void*)wh, (void*)dyn, (void*)alpha, (void*)lse, (void*)val})
-      if (p) cudaFree(p);
+    const std::string se = sc.release();
+    if (e.empty()) e = se;
+    if (!e.empty()) e = "debug_ctc: " + e;
   }
-  if (!e.empty()) {
-    g_create_error = e;
-    return 1;
-  }
-  return 0;
+  return debug_result(e);
 }
 
 int w2s_debug_errors(const float* logits, int n, int T, int V, int ldl, const int32_t* labels_host,
                      const int32_t* offsets_host, int D, int blank, int unit, int delimiter, float* out_dev, void* stream) {
-  g_create_error.clear();
   const cudaStream_t s = (cudaStream_t)stream;
   std::vector<int32_t> tab;
   std::string e;
@@ -1996,32 +1956,21 @@ int w2s_debug_errors(const float* logits, int n, int T, int V, int ldl, const in
     e = "need n, T >= 1, 1 <= V <= 128, ldl >= V and logits / out buffers";
   if (e.empty()) e = error_tables(labels_host, offsets_host, D, V, blank, unit, delimiter, &tab);
   if (e.empty()) {
+    CallScratch sc{s};
     int* dtab = nullptr;
-    DynArgs* dyn = nullptr;
-    if (cudaMalloc((void**)&dtab, sizeof(int) * tab.size()) != cudaSuccess ||
-        cudaMalloc((void**)&dyn, sizeof(DynArgs)) != cudaSuccess)
+    if (!sc.alloc(&dtab, tab.size()))
       e = "out of device memory";
-    DynArgs d{};
-    d.out = out_dev; d.mode = W2S_OUT_ERRORS; d.D = D; d.blank = blank; d.err_tab = dtab; d.err_unit = unit; d.delim = delimiter;
-    if (e.empty() && (cudaMemcpyAsync(dtab, tab.data(), sizeof(int) * tab.size(), cudaMemcpyHostToDevice, s) != cudaSuccess ||
-                      cudaMemcpyAsync(dyn, &d, sizeof(DynArgs), cudaMemcpyHostToDevice, s) != cudaSuccess))
+    else if (cudaMemcpyAsync(dtab, tab.data(), sizeof(int) * tab.size(), cudaMemcpyHostToDevice, s) != cudaSuccess)
       e = "copy failed";
     if (e.empty()) {
-      HeadParams hp{};
-      hp.n = n; hp.T = T; hp.V = V; hp.ldl = ldl; hp.dyn = dyn;
-      e = launch_head_reduce(logits, hp, s);
+      DynArgs d{};
+      d.out = out_dev; d.mode = W2S_OUT_ERRORS; d.D = D; d.blank = blank; d.err_tab = dtab; d.err_unit = unit; d.delim = delimiter;
+      e = debug_head_reduce(logits, n, T, V, ldl, d, sc);
     }
-    // the buffers live for this call only
-    const cudaError_t se = cudaStreamSynchronize(s);
-    if (se != cudaSuccess && e.empty()) e = cudaGetErrorString(se);
-    for (void* p : {(void*)dtab, (void*)dyn})
-      if (p) cudaFree(p);
+    const std::string se = sc.release();
+    if (e.empty()) e = se;
   }
-  if (!e.empty()) {
-    g_create_error = "debug_errors: " + e;
-    return 1;
-  }
-  return 0;
+  return debug_result(e.empty() ? e : "debug_errors: " + e);
 }
 
 int w2s_profile_enable(w2s_handle* h, int on) {

@@ -50,6 +50,14 @@ __device__ __forceinline__ float ctc_frame_lse(const float (&logit)[J], int V, i
   return mx + logf(warp_sum(se));
 }
 
+// one frame one-per-lane (as ctc_frame_lse takes it) from its row of an fp32 logits buffer; returns the row
+template <int J>
+__device__ __forceinline__ const float* ctc_row_frame(const float* row, int V, int lane, float (&logit)[J]) {
+#pragma unroll
+  for (int j = 0; j < J; ++j) logit[j] = lane + 32 * j < V ? row[lane + 32 * j] : -INFINITY;
+  return row;
+}
+
 // log p_CTC(y | frames).  frame(t, logit) loads frame t one-per-lane (as ctc_frame_lse takes it) and returns a pointer
 // through which the frame's logits are indexed by vocabulary id.  alpha: this warp's shared scratch of S floats.  When
 // alpha_out is given, alpha_t(s) is also stored at alpha_out[t * S + s] and lse_t at lse_out[t] (the gradient seed).

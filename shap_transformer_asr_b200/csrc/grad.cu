@@ -357,14 +357,9 @@ __global__ void __launch_bounds__(32) ctc_grad_kernel(const float* __restrict__ 
   const float* rows = logits + (long long)b * T * ldl;
   float* alpha_row = alpha_all + (long long)b * T * s_max;
   float* lse = lse_all + (long long)b * T;
-  const float logp = ctc_forward_warp<4>(T, V, lab, U, blank, lane, alpha,
-                                         [&](int t, float(&lg)[4]) -> const float* {
-                                           const float* row = rows + (long long)t * ldl;
-#pragma unroll
-                                           for (int j = 0; j < 4; ++j) lg[j] = lane + 32 * j < V ? row[lane + 32 * j] : -INFINITY;
-                                           return row;
-                                         },
-                                         alpha_row, lse);
+  const float logp = ctc_forward_warp<4>(
+      T, V, lab, U, blank, lane, alpha,
+      [&](int t, float(&lg)[4]) { return ctc_row_frame(rows + (long long)t * ldl, V, lane, lg); }, alpha_row, lse);
   if (lane == 0) {
     if (out_val) out_val[b] = logp;
     for (int v = 0; v <= V; ++v) start[v] = 0;

@@ -979,19 +979,9 @@ std::string run_grad(w2s_handle* h, const float* x, long long ld, long long L, i
   if (T <= 0) return "clip shorter than the conv receptive field";
   if (h->grad_ctc) {   // transcript indices, checked by w2s_grad_transcripts; seed scratch for one tile
     const long long tile_rows = n < h->grad_tile ? n : h->grad_tile;
-    auto grow = [&](float** p, long long* cap, long long need) -> std::string {
-      if (*cap >= need) return "";
-      W2S_CUDA_OK(cudaStreamSynchronize(s));   // earlier calls may still use the old scratch
-      if (*p) cudaFree(*p);
-      *p = nullptr;
-      *cap = 0;
-      W2S_CUDA_OK(cudaMalloc((void**)p, sizeof(float) * need));
-      *cap = need;
-      return "";
-    };
-    W2S_TRY(grow(&h->ctc_alpha, &h->ctc_alpha_cap, tile_rows * T * h->ctc_smax));
-    W2S_TRY(grow(&h->ctc_lse, &h->ctc_lse_cap, tile_rows * T));
-    W2S_TRY(grow(&h->ctc_dz, &h->ctc_dz_cap, tile_rows * T * h->head_ldl));
+    W2S_TRY(grow(&h->ctc_alpha, &h->ctc_alpha_cap, tile_rows * T * h->ctc_smax, 0, s));
+    W2S_TRY(grow(&h->ctc_lse, &h->ctc_lse_cap, tile_rows * T, 0, s));
+    W2S_TRY(grow(&h->ctc_dz, &h->ctc_dz_cap, tile_rows * T * h->head_ldl, 0, s));
   }
   if (frames_host) {
     for (int64_t i = 0; i < n && !h->grad_ctc; ++i)

@@ -55,10 +55,66 @@ __device__ __forceinline__ long long head_items(const DynArgs& d, int n, int T) 
   return (long long)n * T;
 }
 
+// One work item it (see head_items): the single copy of every mode's reduction for both head kernels.
+// loader(b, t, logit) fills frame t of row b one per lane (logit[j] = entry lane + 32 j, -inf past V) and returns a pointer
+// through which that frame's logits are indexed by vocabulary id (the CTC recursion reads its labels' entries there).
+// scratch: this warp's shared row of CTC_MAX_S floats (CTC alpha, or the errors' hypothesis word).
+template <class Loader>
+__device__ __forceinline__ void head_item(const DynArgs& d, long long it, int T, int V, int lane, float* scratch,
+                                          Loader loader) {
+  if (d.mode == W2S_OUT_CTC) {
+    const int b = (int)(it / d.D), dd = (int)(it - (long long)b * d.D);
+    const float r = ctc_forward_warp<HEAD_MAXJ>(
+        T, V, d.ctc_labels + d.ctc_offsets[dd], d.ctc_offsets[dd + 1] - d.ctc_offsets[dd], d.blank, lane, scratch,
+        [&](int t, float(&lg)[HEAD_MAXJ]) -> const float* { return loader(b, t, lg); });
+    if (lane == 0) d.out[(long long)b * d.D + dd] = r;
+    return;
+  }
+  if (d.mode == W2S_OUT_ERRORS) {
+    const int b = (int)(it / d.D), dd = (int)(it - (long long)b * d.D);
+    const int r = errors_warp<HEAD_MAXJ>(T, V, d.err_tab, dd, d.err_unit, d.blank, d.delim, lane,
+                                         reinterpret_cast<int*>(scratch),
+                                         [&](int t, float(&lg)[HEAD_MAXJ]) { loader(b, t, lg); });
+    if (lane == 0) d.out[(long long)b * d.D + dd] = (float)r;
+    return;
+  }
+  float logit[HEAD_MAXJ];
+  if (d.mode == W2S_OUT_MEAN) {
+    float sm = 0.f;
+    for (int t = 0; t < T; ++t) {
+      loader((int)it, t, logit);
+#pragma unroll
+      for (int j = 0; j < HEAD_MAXJ; ++j)
+        if (lane + 32 * j < V) sm += logit[j];
+    }
+    sm = warp_sum(sm);
+    if (lane == 0) d.out[it] = sm / ((float)V * (float)T);
+    return;
+  }
+  const bool targeted = (d.mode == W2S_OUT_LOGIT || d.mode == W2S_OUT_LOGPROB);
+  const int per = targeted ? d.D : T;
+  const int b = (int)(it / per);
+  const int dd = (int)(it - (long long)b * per);
+  const int t = targeted ? d.frames[dd] : dd;
+  loader(b, t, logit);
+  if (d.mode == W2S_OUT_LOGITS) {
+#pragma unroll
+    for (int j = 0; j < HEAD_MAXJ; ++j) {
+      const int v = lane + 32 * j;
+      if (v < V) d.out[((long long)b * T + t) * V + v] = logit[j];
+    }
+    return;
+  }
+  head_reduce_frame(logit, V, d.mode, targeted ? d.tokens[dd] : 0, lane,
+                    d.out + (targeted ? (long long)b * d.D + dd : (long long)b * T + t));
+}
+
 // CUDA-core validation variant: lm_head (H -> V) + reduction in one kernel, weights staged in shared memory.
 __global__ void __launch_bounds__(256) head_kernel(const HeadParams p) {
   extern __shared__ uint8_t smem[];
-  const DynArgs d = *p.dyn;
+  // read through the pointer, not copied: a copy keeps every field in a register across the item loop, next to the
+  // GEMV's, and spills
+  const DynArgs& d = *p.dyn;
   // the pointers of the argument block are device allocations: keeps the stores and target loads global (LDG / STG)
   __builtin_assume(__isGlobal(d.out) && __isGlobal(d.frames) && __isGlobal(d.tokens));
   const int ldw = p.H + 2;  // bf16 elements; (H+2)/2 odd -> conflict-free row stride
@@ -72,90 +128,40 @@ __global__ void __launch_bounds__(256) head_kernel(const HeadParams p) {
   __syncthreads();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   __nv_bfloat16* hrow = hs + (size_t)warp * p.H;
-  const bool targeted = (d.mode == W2S_OUT_LOGIT || d.mode == W2S_OUT_LOGPROB);
   const long long items = head_items(d, p.n, p.T);
-  const int per = targeted ? d.D : p.T;
-  auto frame_logits = [&](int b, int t, float (&logit)[HEAD_MAXJ]) {
-    const __nv_bfloat16* src = p.h + ((long long)b * p.T + t) * p.H;
-    __syncwarp();
-    for (int k = lane * 2; k < p.H; k += 64)
-      *reinterpret_cast<uint32_t*>(hrow + k) = *reinterpret_cast<const uint32_t*>(src + k);
-    __syncwarp();
+  for (long long it = (long long)blockIdx.x * 8 + warp; it < items; it += (long long)gridDim.x * 8)
+    head_item(d, it, p.T, p.V, lane, ctc_alpha + warp * CTC_MAX_S,
+              [&](int b, int t, float(&logit)[HEAD_MAXJ]) -> const float* {
+                const __nv_bfloat16* src = p.h + ((long long)b * p.T + t) * p.H;
+                __syncwarp();
+                for (int k = lane * 2; k < p.H; k += 64)
+                  *reinterpret_cast<uint32_t*>(hrow + k) = *reinterpret_cast<const uint32_t*>(src + k);
+                __syncwarp();
 #pragma unroll
-    for (int j = 0; j < HEAD_MAXJ; ++j) {
-      const int v = lane + 32 * j;
-      float acc = 0.f;
-      if (v < p.V) {
-        const __nv_bfloat16* wr = ws + (size_t)v * ldw;
-        for (int k = 0; k < p.H; k += 2) {
-          const uint32_t hh = *reinterpret_cast<const uint32_t*>(hrow + k);
-          const uint32_t ww = *reinterpret_cast<const uint32_t*>(wr + k);
-          acc = fmaf(bf16_lo(hh), bf16_lo(ww), acc);
-          acc = fmaf(bf16_hi(hh), bf16_hi(ww), acc);
-        }
-        acc += p.bias[v];
-      }
-      logit[j] = acc;
-    }
-  };
-  for (long long it = (long long)blockIdx.x * 8 + warp; it < items; it += (long long)gridDim.x * 8) {
-    float logit[HEAD_MAXJ];
-    if (d.mode == W2S_OUT_CTC) {
-      const int b = (int)(it / d.D), dd = (int)(it - (long long)b * d.D);
-      float* zs = ctc_alpha + 8 * CTC_MAX_S + warp * 32 * HEAD_MAXJ;   // the frame's logits, indexed by vocabulary id
-      const float r = ctc_forward_warp<HEAD_MAXJ>(
-          p.T, p.V, d.ctc_labels + d.ctc_offsets[dd], d.ctc_offsets[dd + 1] - d.ctc_offsets[dd], d.blank, lane,
-          ctc_alpha + warp * CTC_MAX_S, [&](int t, float(&lg)[HEAD_MAXJ]) -> const float* {
-            frame_logits(b, t, lg);
+                for (int j = 0; j < HEAD_MAXJ; ++j) {
+                  const int v = lane + 32 * j;
+                  float acc = 0.f;
+                  if (v < p.V) {
+                    const __nv_bfloat16* wr = ws + (size_t)v * ldw;
+                    for (int k = 0; k < p.H; k += 2) {
+                      const uint32_t hh = *reinterpret_cast<const uint32_t*>(hrow + k);
+                      const uint32_t ww = *reinterpret_cast<const uint32_t*>(wr + k);
+                      acc = fmaf(bf16_lo(hh), bf16_lo(ww), acc);
+                      acc = fmaf(bf16_hi(hh), bf16_hi(ww), acc);
+                    }
+                    acc += p.bias[v];
+                  }
+                  logit[j] = acc;
+                }
+                float* zs = ctc_alpha + 8 * CTC_MAX_S + warp * 32 * HEAD_MAXJ;   // the frame's logits, indexed by vocabulary id
 #pragma unroll
-            for (int j = 0; j < HEAD_MAXJ; ++j)
-              if (lane + 32 * j < p.V) zs[lane + 32 * j] = lg[j];
-            __syncwarp();
-            return zs;
-          });
-      if (lane == 0) d.out[(long long)b * d.D + dd] = r;
-      continue;
-    }
-    if (d.mode == W2S_OUT_ERRORS) {
-      const int b = (int)(it / d.D), dd = (int)(it - (long long)b * d.D);
-      const int r = errors_warp<HEAD_MAXJ>(p.T, p.V, d.err_tab, dd, d.err_unit, d.blank, d.delim, lane,
-                                           reinterpret_cast<int*>(ctc_alpha + warp * CTC_MAX_S),
-                                           [&](int t, float(&lg)[HEAD_MAXJ]) {
-                                             frame_logits(b, t, lg);
-#pragma unroll
-                                             for (int j = 0; j < HEAD_MAXJ; ++j)
-                                               if (lane + 32 * j >= p.V) lg[j] = -INFINITY;
-                                           });
-      if (lane == 0) d.out[(long long)b * d.D + dd] = (float)r;
-      continue;
-    }
-    if (d.mode == W2S_OUT_MEAN) {
-      float sm = 0.f;
-      for (int t = 0; t < p.T; ++t) {
-        frame_logits((int)it, t, logit);
-#pragma unroll
-        for (int j = 0; j < HEAD_MAXJ; ++j)
-          if (lane + 32 * j < p.V) sm += logit[j];
-      }
-      sm = warp_sum(sm);
-      if (lane == 0) d.out[it] = sm / ((float)p.V * (float)p.T);
-      continue;
-    }
-    const int b = (int)(it / per);
-    const int dd = (int)(it - (long long)b * per);
-    const int t = targeted ? d.frames[dd] : dd;
-    frame_logits(b, t, logit);
-    if (d.mode == W2S_OUT_LOGITS) {
-#pragma unroll
-      for (int j = 0; j < HEAD_MAXJ; ++j) {
-        const int v = lane + 32 * j;
-        if (v < p.V) d.out[((long long)b * p.T + t) * p.V + v] = logit[j];
-      }
-      continue;
-    }
-    head_reduce_frame(logit, p.V, d.mode, targeted ? d.tokens[dd] : 0, lane,
-                      d.out + (targeted ? (long long)b * d.D + dd : (long long)b * p.T + t));
-  }
+                for (int j = 0; j < HEAD_MAXJ; ++j) {
+                  if (lane + 32 * j < p.V) zs[lane + 32 * j] = logit[j];
+                  else logit[j] = -INFINITY;
+                }
+                __syncwarp();
+                return zs;
+              });
 }
 
 // second stage of the tensor-core head: logits[rows, ldl] (fp32, bias included) -> reduction; one warp per work item.
@@ -166,70 +172,11 @@ __global__ void __launch_bounds__(256, 6) head_reduce_kernel(const float* __rest
   const DynArgs d = *p.dyn;
   __builtin_assume(__isGlobal(d.out) && __isGlobal(d.frames) && __isGlobal(d.tokens));   // as in head_kernel
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const bool targeted = (d.mode == W2S_OUT_LOGIT || d.mode == W2S_OUT_LOGPROB);
   const long long items = head_items(d, p.n, p.T);
-  const int per = targeted ? d.D : p.T;
-  for (long long it = (long long)blockIdx.x * 8 + warp; it < items; it += (long long)gridDim.x * 8) {
-    float logit[HEAD_MAXJ];
-    if (d.mode == W2S_OUT_CTC) {
-      const int b = (int)(it / d.D), dd = (int)(it - (long long)b * d.D);
-      const float* rows = logits + (long long)b * p.T * p.ldl;
-      const float r = ctc_forward_warp<HEAD_MAXJ>(
-          p.T, p.V, d.ctc_labels + d.ctc_offsets[dd], d.ctc_offsets[dd + 1] - d.ctc_offsets[dd], d.blank, lane,
-          ctc_alpha[warp], [&](int t, float(&lg)[HEAD_MAXJ]) -> const float* {
-            const float* row = rows + (long long)t * p.ldl;
-#pragma unroll
-            for (int j = 0; j < HEAD_MAXJ; ++j) lg[j] = lane + 32 * j < p.V ? row[lane + 32 * j] : -INFINITY;
-            return row;
-          });
-      if (lane == 0) d.out[(long long)b * d.D + dd] = r;
-      continue;
-    }
-    if (d.mode == W2S_OUT_ERRORS) {
-      const int b = (int)(it / d.D), dd = (int)(it - (long long)b * d.D);
-      const float* rows = logits + (long long)b * p.T * p.ldl;
-      const int r = errors_warp<HEAD_MAXJ>(p.T, p.V, d.err_tab, dd, d.err_unit, d.blank, d.delim, lane,
-                                           reinterpret_cast<int*>(ctc_alpha[warp]), [&](int t, float(&lg)[HEAD_MAXJ]) {
-                                             const float* row = rows + (long long)t * p.ldl;
-#pragma unroll
-                                             for (int j = 0; j < HEAD_MAXJ; ++j)
-                                               lg[j] = lane + 32 * j < p.V ? row[lane + 32 * j] : -INFINITY;
-                                           });
-      if (lane == 0) d.out[(long long)b * d.D + dd] = (float)r;
-      continue;
-    }
-    if (d.mode == W2S_OUT_MEAN) {
-      const float* row = logits + it * p.T * p.ldl;
-      float sm = 0.f;
-      for (int t = 0; t < p.T; ++t) {
-#pragma unroll
-        for (int j = 0; j < HEAD_MAXJ; ++j)
-          if (lane + 32 * j < p.V) sm += row[(long long)t * p.ldl + lane + 32 * j];
-      }
-      sm = warp_sum(sm);
-      if (lane == 0) d.out[it] = sm / ((float)p.V * (float)p.T);
-      continue;
-    }
-    const int b = (int)(it / per);
-    const int dd = (int)(it - (long long)b * per);
-    const int t = targeted ? d.frames[dd] : dd;
-    const float* row = logits + ((long long)b * p.T + t) * p.ldl;
-#pragma unroll
-    for (int j = 0; j < HEAD_MAXJ; ++j) {
-      const int v = lane + 32 * j;
-      logit[j] = v < p.V ? row[v] : -INFINITY;
-    }
-    if (d.mode == W2S_OUT_LOGITS) {
-#pragma unroll
-      for (int j = 0; j < HEAD_MAXJ; ++j) {
-        const int v = lane + 32 * j;
-        if (v < p.V) d.out[((long long)b * p.T + t) * p.V + v] = logit[j];
-      }
-      continue;
-    }
-    head_reduce_frame(logit, p.V, d.mode, targeted ? d.tokens[dd] : 0, lane,
-                      d.out + (targeted ? (long long)b * d.D + dd : (long long)b * p.T + t));
-  }
+  for (long long it = (long long)blockIdx.x * 8 + warp; it < items; it += (long long)gridDim.x * 8)
+    head_item(d, it, p.T, p.V, lane, ctc_alpha[warp], [&](int b, int t, float(&logit)[HEAD_MAXJ]) {
+      return ctc_row_frame(logits + ((long long)b * p.T + t) * p.ldl, p.V, lane, logit);
+    });
 }
 
 // The grid is sized for one item per (row, frame) -- the largest item count any mode has, unless more targets than

@@ -320,9 +320,7 @@ class Engine:
 
     def eval_waveforms(self, x: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """x: float32 device tensor [n, L] (last dim contiguous) -> float32 device tensor [n, width]."""
-        if x.dim() != 2 or x.stride(1) != 1 or x.dtype != torch.float32 or not x.is_cuda:
-            raise ValueError("expected a float32 CUDA tensor [n, L] with contiguous rows")
-        n, L = x.shape
+        n, L = _rows(x)
         width = self.out_width(L)
         if out is None:
             out = torch.empty((n, width), dtype=torch.float32, device=self.device)
@@ -335,9 +333,7 @@ class Engine:
         """x: float32 device tensor [n, L]; frames: one output frame per row -> (grad [n, L] float32 device tensor of
         d out[r] / d x[r], out [n]) with out[r] = max_v logits[r, frames[r], v] -- the scalar the reference's
         GradientExplainer differentiates through ModelWrapper (shap_calculation.py:50, :133, :162)."""
-        if x.dim() != 2 or x.stride(1) != 1 or x.dtype != torch.float32 or not x.is_cuda:
-            raise ValueError("expected a float32 CUDA tensor [n, L] with contiguous rows")
-        n, L = x.shape
+        n, L = _rows(x)
         f = np.ascontiguousarray(np.broadcast_to(np.asarray(frames, dtype=np.int32), (n,)))
         grad = torch.empty((n, L), dtype=torch.float32, device=self.device)
         out = torch.empty((n,), dtype=torch.float32, device=self.device)
@@ -349,9 +345,7 @@ class Engine:
     def grad_transcripts(self, x: torch.Tensor, which):
         """x: float32 device tensor [n, L]; which: one transcript index per row (of the last ``set_transcripts``) ->
         (grad [n, L], out [n]) with out[r] = log p_CTC(y_which[r] | x[r]) and grad[r] = d out[r] / d x[r]."""
-        if x.dim() != 2 or x.stride(1) != 1 or x.dtype != torch.float32 or not x.is_cuda:
-            raise ValueError("expected a float32 CUDA tensor [n, L] with contiguous rows")
-        n, L = x.shape
+        n, L = _rows(x)
         w = np.ascontiguousarray(np.broadcast_to(np.asarray(which, dtype=np.int32), (n,)))
         grad = torch.empty((n, L), dtype=torch.float32, device=self.device)
         out = torch.empty((n,), dtype=torch.float32, device=self.device)
@@ -363,9 +357,7 @@ class Engine:
     def vjp_waveforms(self, x: torch.Tensor, gout: torch.Tensor) -> torch.Tensor:
         """Vector-Jacobian product of ModelWrapper's output [n, T'] (max logit per frame) w.r.t. the waveforms:
         gout [n, T'] float32 device tensor -> grad [n, L]."""
-        if x.dim() != 2 or x.stride(1) != 1 or x.dtype != torch.float32 or not x.is_cuda:
-            raise ValueError("expected a float32 CUDA tensor [n, L] with contiguous rows")
-        n, L = x.shape
+        n, L = _rows(x)
         gout = gout.to(device=self.device, dtype=torch.float32).contiguous()
         if tuple(gout.shape) != (n, self.num_frames(L)):
             raise ValueError(f"upstream gradient must be [n, T'] = {(n, self.num_frames(L))}, got {tuple(gout.shape)}")
@@ -482,6 +474,13 @@ def debug_gemm(a: torch.Tensor, w: torch.Tensor, bias=None, act: int = 0, out_fp
     if rc != 0:
         raise RuntimeError("w2s_debug_gemm: " + lib.w2s_last_error(None).decode())
     return out
+
+
+def _rows(x: torch.Tensor):
+    """(n, L) of a float32 CUDA tensor [n, L] with contiguous rows (any row stride), the waveform input of the device paths."""
+    if x.dim() != 2 or x.stride(1) != 1 or x.dtype != torch.float32 or not x.is_cuda:
+        raise ValueError("expected a float32 CUDA tensor [n, L] with contiguous rows")
+    return x.shape
 
 
 def _check_buffer(name: str, t: torch.Tensor, dtype: torch.dtype, numel: int):
